@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N --steps K --warmup W]            the CUDA path (one process per GPU)
     python bench.py --impl reference [...]                     the CPU reference arm (oracle port, ALL rows)
+    python bench.py [...] --dump-outputs DIR                   also write the last timed step's (D, I) under DIR
 
 A "step" is ONE search call: a batch of `--nq` queries (default 1 -- what the app issues,
 oldapp.py:2005, and the case the north_star's roofline target names) scored against all rows, top-48
@@ -67,7 +68,14 @@ def parse_args():
     ap.add_argument("--tc-min-nq", type=int, default=None, help="override the library's tensor-core threshold (experiments)")
     ap.add_argument("--set", action="append", default=[], metavar="NAME=VALUE", help="evs.set_option before the run (experiments)")
     ap.add_argument("--extra", action="store_true", help="also time query batches 1/4/16/64 (reported under 'extra')")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the (D, I) the last timed step returned as DIR/D.npy and DIR/I.npy, to compare builds output for output")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs:
+        os.makedirs(a.dump_outputs, exist_ok=True)  # an unwritable DIR fails before the run, not after it
+    return a
 
 
 def workload_name(a) -> str:
@@ -191,6 +199,27 @@ def measured_peak_tflops():
         except Exception:  # noqa: BLE001
             pass
     return 1590.0, 1400.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, D, I) -> None:
+    """One search's answer as .npy files: D float32 [nq, k] and I as float64 (ids are exact below 2^53).  An answer larger
+    than 64 MB is cut to a fixed, seeded sample of its queries, whose row numbers go to rows.npy."""
+    D = np.asarray(D, dtype=np.float32)
+    I = np.asarray(I).astype(np.float64)
+    nq, k = D.shape
+    keep = (DUMP_LIMIT_BYTES - 4096) // (k * 12 + 8)  # 4 + 8 bytes per result, 8 per row number, room for three headers
+    rows_path = os.path.join(out_dir, "rows.npy")
+    if nq > keep:
+        rows = np.sort(np.random.default_rng(0).choice(nq, keep, replace=False))
+        D, I = D[rows], I[rows]
+        np.save(rows_path, rows.astype(np.float64))
+    elif os.path.exists(rows_path):
+        os.remove(rows_path)  # left by an earlier, sampled dump
+    np.save(os.path.join(out_dir, "D.npy"), D)
+    np.save(os.path.join(out_dir, "I.npy"), I)
 
 
 def scan_arithmetic(evs, storage: str, nq: int, rows_per_gpu: int, dim: int) -> str:
@@ -464,8 +493,10 @@ def run_reference(a) -> int:
         step(i)
     t0 = time.perf_counter()
     for i in range(a.steps):
-        step(a.warmup + i)
+        D_last, I_last = step(a.warmup + i)
     dt = time.perf_counter() - t0
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, D_last, I_last)
     qps = a.steps * a.nq / dt * scale
     # faiss's own threading for the same call, for the record (short)
     t1 = time.perf_counter()
@@ -585,6 +616,8 @@ def run_evs(a) -> int:
     if one_launch:
         n_prof, scan_ms_sum = a.steps, ms_total
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and a.dump_outputs:  # every rank holds the same merged (D, I)
+        dump_outputs(a.dump_outputs, D_last.cpu().numpy(), I_last.cpu().numpy())
     value = a.steps * a.nq / (ms_total * 1e-3)
     events_check = None
     if one_launch:  # cross-check: the same kernel with libevs' own event pair around every launch (a short extra pass)

@@ -670,6 +670,26 @@ def test_index_file_bytes_and_roundtrip(golden_dir, tmp_path):
         evs.read_index(str(tmp_path / "nope.faiss"))
 
 
+def test_bench_dump_is_the_last_timed_search(tmp_path):
+    """`bench.py --dump-outputs DIR`: --steps searches are timed (one launch each for a single query), and DIR holds the (D, I)
+    of the last one -- query (warmup + steps - 1) mod 64 of the seed-1 pool against the seed-0 database -- in the oracle's bits."""
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    n, steps, warmup = 70_000, 5, 2
+    cmd = [sys.executable, os.path.join(root, "bench.py"), "--rows", str(n), "--steps", str(steps), "--warmup", str(warmup),
+           "--no-configs", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)]
+    out = subprocess.run(cmd, capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-3000:]
+    line = json.loads([ln for ln in out.stdout.splitlines() if ln.startswith("{")][-1])
+    assert line["steps"] == steps and line["gpu_launches"] == steps
+    q = oracle.synth_fill(64, 512, seed=1)[(warmup + steps - 1) % 64][None]
+    Dr, Ir = oracle.canon_search(q, oracle.synth_fill(n, 512, seed=0), 48)
+    D, I = np.load(tmp_path / "D.npy"), np.load(tmp_path / "I.npy")
+    assert D.dtype == np.float32 and I.dtype == np.float64
+    assert np.array_equal(D, Dr) and np.array_equal(I, Ir)
+
+
 # ------------------------------------------------------------------------------------------------
 # full BASELINE sizes
 # ------------------------------------------------------------------------------------------------

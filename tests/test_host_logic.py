@@ -182,16 +182,17 @@ def test_resident_cache_is_an_lru_with_a_byte_budget(tmp_path, monkeypatch):
     assert lifecycle._want_sharded(False) is False and lifecycle._want_sharded(None) is False  # no process group here
 
 
-def test_bench_reference_arm_prints_the_contract_line():
+def test_bench_reference_arm_prints_the_contract_line(tmp_path):
     """`bench.py --impl reference` (the CPU arm the driver times beside the CUDA arm) on a small workload: ONE JSON line with the
     contract's keys, `impl: reference`, a cpu_baseline block describing the run and an e2e block equal to the line's value;
-    ranks other than 0 print nothing and exit 0."""
+    `--dump-outputs` holds the last timed step's answer; ranks other than 0 print nothing and exit 0."""
     import json
     import os
     import subprocess
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    cmd = [sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--rows", "20000", "--steps", "2", "--warmup", "1"]
+    cmd = [sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--rows", "20000", "--steps", "2", "--warmup", "1",
+           "--dump-outputs", str(tmp_path)]
     out = subprocess.run(cmd, capture_output=True, text=True, timeout=300, env={**os.environ, "RANK": "0"})
     assert out.returncode == 0, out.stderr[-2000:]
     lines = [ln for ln in out.stdout.splitlines() if ln.startswith("{")]
@@ -204,6 +205,12 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert d["value"] > 0 and d["e2e"]["value"] == d["value"] and d["e2e"]["h2d_bytes_per_step"] == 0
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1 and "20000" in d["cpu_baseline"]["sample"]
     assert d["config"]["workload"].startswith("20000x512 f32 flat-IP")
+    import oracle
+    q = np.roll(oracle.synth_fill(64, 512, seed=1), -2, axis=0)[:1]  # the last timed step is step 2 (after 1 warmup step): query 2
+    Dr, Ir = oracle.allcores_search(q, oracle.synth_fill(20000, 512, seed=0), 48, nthreads=d["cpu_baseline"]["cores"])
+    D, I = np.load(tmp_path / "D.npy"), np.load(tmp_path / "I.npy")
+    assert D.dtype == np.float32 and I.dtype == np.float64
+    assert np.array_equal(D, Dr) and np.array_equal(I, Ir)
     other = subprocess.run(cmd, capture_output=True, text=True, timeout=300, env={**os.environ, "RANK": "1"})
     assert other.returncode == 0 and other.stdout.strip() == ""
 
