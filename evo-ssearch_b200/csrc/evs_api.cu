@@ -66,13 +66,18 @@ static const int kTcQueryChunk = 4096;  // tensor-core path: queries per launch 
 
 // per-handle device words (idx->words): counters the kernels share across searches
 enum { W_TICKET = 0, W_NEXT_CHUNK = 1, W_GUARD_COUNT0 = 2, W_GUARD_COUNT1 = 3, W_UNCERT = 4 /* u64 */, W_RERUNS = 6 /* u64 */,
-       W_MAX_NORM = 8 /* float */, W_SPECIAL = 9, W_BAR = 10 /* 3 words: grid barrier of the in-launch pre-pass */, W_WORDS = 16 };
+       W_MAX_NORM = 8 /* float */, W_SPECIAL = 9, W_BAR = 10 /* 3 words: grid barrier of the in-launch pre-pass */,
+       W_EMAX = 13 /* float: largest |x - bf16(x)|_2 of a row of the bf16 copy */, W_WIDE = 14 /* single-query searches of the bf16
+       copy that re-scored more than POOL_KPMAX candidates */, W_LASTC = 15 /* candidates the last of them re-scored */, W_WORDS = 16 };
 
 struct evs_index {
     int d = 0, device = 0, storage = EVS_STORE_F32;
     int64_t ntotal = 0, capacity = 0, id_base = 0;
     float* xb32 = nullptr;            // fp32 rows (the master copy; what index.faiss holds)
-    void* xb16 = nullptr;             // derived bf16 rows (EVS_STORE_BF16_F32)
+    void* xb16 = nullptr;             // derived bf16 rows (EVS_STORE_BF16_F32, or the scan copy of an fp32 index: option
+                                      // "scan_shadow"); when present it always holds every row, and W_EMAX bounds its rounding
+    unsigned special_host = 0;        // host copies of W_SPECIAL / W_EMAX, read back by every add
+    float emax_host = 0.f;
     int sm_count = 0;
     cudaStream_t stream = nullptr;    // the handle's own stream
     cudaEvent_t ws_free = nullptr;    // recorded after each search: the workspace may be reused after it
@@ -232,6 +237,11 @@ extern "C" int evs_set_option(const char* name, int64_t value) {
     } else if (!strcmp(name, "small_fast_cap")) {
         if (value < 1 || value > 2048) return fail(EVS_EINVAL, "small_fast_cap must be in [1, 2048]");
         g_tune.small_fast_cap = (int)value;
+    } else if (!strcmp(name, "scan_shadow")) {
+        g_tune.scan_shadow = value ? 1 : 0;
+    } else if (!strcmp(name, "shadow_min_rows")) {
+        if (value < 0 || value > INT32_MAX) return fail(EVS_EINVAL, "shadow_min_rows must be in [0, 2^31 - 1]");
+        g_tune.shadow_min_rows = (int)value;
     } else if (!strcmp(name, "io_threads")) {
         if (value < 0 || value > 64) return fail(EVS_EINVAL, "io_threads must be in [0, 64]");
         g_io_threads.store((int)value);
@@ -272,6 +282,8 @@ extern "C" int evs_get_option(const char* name, int64_t* value) {
     else if (!strcmp(name, "io_threads")) *value = g_io_threads.load();
     else if (!strcmp(name, "small_max_rows")) *value = g_tune.small_max_rows;
     else if (!strcmp(name, "small_fast_cap")) *value = g_tune.small_fast_cap;
+    else if (!strcmp(name, "scan_shadow")) *value = g_tune.scan_shadow;
+    else if (!strcmp(name, "shadow_min_rows")) *value = g_tune.shadow_min_rows;
     else return fail(EVS_EINVAL, "unknown option '%s'", name);
     return EVS_OK;
 }
@@ -366,6 +378,11 @@ extern "C" int evs_index_set_id_base(evs_index* idx, int64_t base) {
 }
 
 // grow the row storage to hold at least `rows` rows (device-to-device copy of what is there)
+static bool shadow_wanted() {
+    std::lock_guard<std::mutex> lk(g_tune_mu);
+    return g_tune.scan_shadow != 0;
+}
+
 static int grow_locked(evs_index* idx, int64_t rows) {
     if (rows <= idx->capacity) return EVS_OK;
     if (rows >= (int64_t)0xFFFFFFFFll) return fail(EVS_ELIMIT, "a shard holds at most 2^32-2 rows");
@@ -373,7 +390,8 @@ static int grow_locked(evs_index* idx, int64_t rows) {
     float* n32 = nullptr;
     void* n16 = nullptr;
     CU(cudaMalloc(reinterpret_cast<void**>(&n32), (size_t)rows * d * sizeof(float)));
-    if (idx->storage == EVS_STORE_BF16_F32) {
+    // the bf16 copy grows with the rows; an fp32 index that has none yet but holds rows gets it built by its next add
+    if (idx->storage == EVS_STORE_BF16_F32 || idx->xb16 != nullptr || (idx->ntotal == 0 && shadow_wanted())) {
         cudaError_t e = cudaMalloc(&n16, (size_t)rows * d * 2);
         if (e != cudaSuccess) {
             cudaFree(n32);
@@ -382,7 +400,7 @@ static int grow_locked(evs_index* idx, int64_t rows) {
     }
     if (idx->ntotal > 0) {
         cudaError_t e = cudaMemcpyAsync(n32, idx->xb32, (size_t)idx->ntotal * d * sizeof(float), cudaMemcpyDeviceToDevice, idx->stream);
-        if (e == cudaSuccess && n16)
+        if (e == cudaSuccess && n16 && idx->xb16)
             e = cudaMemcpyAsync(n16, idx->xb16, (size_t)idx->ntotal * d * 2, cudaMemcpyDeviceToDevice, idx->stream);
         const cudaError_t es = cudaStreamSynchronize(idx->stream);  // also on the error path: nothing may still read the old rows
         if (e == cudaSuccess) e = es;
@@ -408,18 +426,37 @@ static int grow_for_add_locked(evs_index* idx, int64_t n) {
     return grow_locked(idx, cap);
 }
 
-// after new fp32 rows [ntotal, ntotal+n) are in place (enqueued on idx->stream): derive bf16, publish
-static int finish_add_locked(evs_index* idx, int64_t n) {
+// the rows [r0, r0 + n): largest row norm and special elements (the certification bound of the searches, finalize_query)
+// and -- when the index keeps a bf16 copy -- the copy and its rounding bound, in one pass; then the host copies of the flags
+static int derive_rows_locked(evs_index* idx, int64_t r0, int64_t n) {
     const size_t d = (size_t)idx->d;
-    if (idx->storage == EVS_STORE_BF16_F32) {
-        CU(launch_f32_to_bf16(idx->xb32 + (size_t)idx->ntotal * d,
-                              reinterpret_cast<unsigned char*>(idx->xb16) + (size_t)idx->ntotal * d * 2, (long long)n * idx->d,
-                              idx->sm_count, idx->stream));
-    }
-    // the largest row norm scales the certification bound of the searches (finalize_query)
-    CU(launch_row_norm_max(idx->xb32 + (size_t)idx->ntotal * d, (long long)n, idx->d, reinterpret_cast<float*>(idx->words + W_MAX_NORM),
-                           idx->words + W_SPECIAL, idx->sm_count, idx->stream));
+    void* dst16 = idx->xb16 ? reinterpret_cast<unsigned char*>(idx->xb16) + (size_t)r0 * d * 2 : nullptr;
+    CU(launch_row_norm_max(idx->xb32 + (size_t)r0 * d, (long long)n, idx->d, reinterpret_cast<float*>(idx->words + W_MAX_NORM),
+                           idx->words + W_SPECIAL, idx->sm_count, idx->stream, dst16, reinterpret_cast<float*>(idx->words + W_EMAX)));
     CU(cudaStreamSynchronize(idx->stream));
+    unsigned w[W_EMAX - W_SPECIAL + 1];
+    CU(cudaMemcpy(w, idx->words + W_SPECIAL, sizeof(w), cudaMemcpyDeviceToHost));
+    idx->special_host = w[0];
+    memcpy(&idx->emax_host, &w[W_EMAX - W_SPECIAL], sizeof(float));
+    return EVS_OK;
+}
+
+// after new fp32 rows [ntotal, ntotal+n) are in place (enqueued on idx->stream): derive bf16, publish.  An fp32 index keeps
+// its bf16 scan copy while the option "scan_shadow" is on at add time (built over every row if it has none yet) and drops
+// it otherwise.
+static int finish_add_locked(evs_index* idx, int64_t n) {
+    const bool want16 = idx->storage == EVS_STORE_BF16_F32 || shadow_wanted();
+    int64_t r0 = idx->ntotal;
+    if (!want16 && idx->xb16) {
+        CU(cudaStreamSynchronize(idx->stream));
+        cudaFree(idx->xb16);
+        idx->xb16 = nullptr;
+    } else if (want16 && !idx->xb16) {
+        CU(cudaMalloc(&idx->xb16, (size_t)idx->capacity * idx->d * 2));
+        r0 = 0;
+    }
+    int rc = derive_rows_locked(idx, r0, idx->ntotal + n - r0);
+    if (rc) return rc;
     idx->ntotal += n;
     return EVS_OK;
 }
@@ -560,6 +597,7 @@ struct PathInfo {
     float err_coef = 0.f;  // scan error bound relative to |q| * max|x| (0 = not certified: bf16 storage)
     float err_trunc = 0.f; // single tf32: the truncation part of the bound, relative to (|q| max|x| + |worst retained score|)
     bool fused = false;  // PATH_GEMV, one query: the scan's last CTA finalises (and, in exchange mode, merges): ONE launch
+    bool shadow = false; // ... with the pool kernel over the bf16 rows under the bound W_EMAX (exact: evs_scan.cuh)
 };
 
 // scan error models, relative to |q| * |x| (DESIGN.md section 2).  fp32 GEMV: 4 partial chains of d/128 FMAs per lane, 3 + 5
@@ -582,6 +620,22 @@ static bool takes_tc_path(const evs_index* idx, int64_t nq, const ScanTuning& tu
            tc_max_queries(idx->d, idx->storage == EVS_STORE_BF16_F32) > 0;
 }
 
+// A fused single-query search scans the bf16 rows with the pool kernel under the rounding bound (exact for any data) when
+// the copy exists (it always holds every row), the index has no subnormal / inf / NaN element and a finite bound, and the
+// shard is above the small-shard cut (those are L2-resident and latency-bound: scan_small_kernel over the fp32 rows) and
+// holds at least shadow_min_rows rows.
+// bf16-storage indexes take the same path; an fp32 index only while the option "scan_shadow" is on.
+static bool shadow_applies(const evs_index* idx, int64_t nq, int kp, const ScanTuning& tune) {
+    if (nq != 1 || !tune.fuse_finalize || !tune.pool_select || kp != 64 || idx->xb16 == nullptr) return false;
+    if (idx->storage != EVS_STORE_BF16_F32 && !tune.scan_shadow) return false;
+    if (idx->special_host != 0 || !(idx->emax_host <= FLT_MAX) || idx->ntotal <= tune.small_max_rows ||
+        idx->ntotal < tune.shadow_min_rows)
+        return false;
+    ScanPlan plan;
+    return plan_scan(idx->ntotal, idx->d, 1, kp, 1, idx->sm_count, tune, &plan) == cudaSuccess && plan.variant == 1 &&
+           plan.threads == 256;
+}
+
 static PathInfo plan_path(const evs_index* idx, int64_t nq, int64_t k, const ScanTuning& tune, bool allow_tc) {
     PathInfo pi;
     const bool bf16 = idx->storage == EVS_STORE_BF16_F32;
@@ -589,8 +643,11 @@ static PathInfo plan_path(const evs_index* idx, int64_t nq, int64_t k, const Sca
     pi.err_coef = bf16 ? 0.f : gemv_err_coef(idx->d);
     if (!allow_tc || !takes_tc_path(idx, nq, tune)) {
         if (nq == 1 && tune.fuse_finalize && idx->ntotal > 0) {
+            pi.shadow = shadow_applies(idx, nq, pi.kp, tune);
+            if (pi.shadow) pi.err_coef = 0.f;  // exact by construction: nothing to certify
             ScanPlan plan;
-            pi.fused = plan_scan(idx->ntotal, idx->d, bf16, pi.kp, 1, idx->sm_count, tune, &plan) == cudaSuccess && plan.variant == 1;
+            pi.fused = plan_scan(idx->ntotal, idx->d, bf16 || pi.shadow, pi.kp, 1, idx->sm_count, tune, &plan) == cudaSuccess &&
+                       plan.variant == 1;
         }
         return pi;
     }
@@ -1032,7 +1089,8 @@ static int search_enqueue_locked(evs_index* idx, int64_t nq, const float* q_dev,
     }
     const int kp = kp_override ? kp_override : pi.kp;
     const bool bf16 = idx->storage == EVS_STORE_BF16_F32;
-    const bool scan_bf16 = bf16 && kp_override == 0;  // an exact re-run always scans the fp32 rows
+    const bool shadow = pi.shadow && kp_override == 0;
+    const bool scan_bf16 = (bf16 || shadow) && kp_override == 0;  // an exact re-run always scans the fp32 rows
     const void* scan_rows = scan_bf16 ? idx->xb16 : (const void*)idx->xb32;
     const int qpp = max_queries_per_pass(idx->d, scan_bf16);
     ScanPlan plan;
@@ -1048,6 +1106,8 @@ static int search_enqueue_locked(evs_index* idx, int64_t nq, const float* q_dev,
     const bool fused = (kp_override ? (tune.fuse_finalize && nq == 1 && plan.variant == 1) : pi.fused) && !scan_only;
     if (out.x && out.x->merge_D && !fused) return fail(EVS_ECUDA, "internal: the exchange expected a fused single-query search");
     const float err_coef = scan_bf16 ? 0.f : gemv_err_coef(idx->d);
+    if (shadow && !(fused && tune.pool_select && kp == 64) && !scan_only)
+        return fail(EVS_ECUDA, "internal: the bf16 scan copy is searched by the fused pool kernel only");
 
     for (int64_t c0 = 0; c0 < nq; c0 += kQueryChunk) {
         const int64_t cn = (nq - c0) < kQueryChunk ? (nq - c0) : kQueryChunk;
@@ -1055,6 +1115,11 @@ static int search_enqueue_locked(evs_index* idx, int64_t nq, const float* q_dev,
         ProfileScope prof;
         if ((rc = prof.begin(idx, profile, st))) return rc;
         FinalizeParams f = make_finalize(idx, idx->lists, plan.grid, kp, qc, k, out, c0, nq, err_coef);
+        if (shadow) {
+            f.shadow_emax = reinterpret_cast<const float*>(idx->words + W_EMAX);
+            f.shadow_gamma = gemv_err_coef(idx->d);
+            f.wide = idx->words + W_WIDE;  // W_LASTC follows
+        }
         for (int64_t p0 = 0; p0 < cn; p0 += qpp) {
             ScanArgs a;
             a.xb = scan_rows;
@@ -1070,7 +1135,9 @@ static int search_enqueue_locked(evs_index* idx, int64_t nq, const float* q_dev,
                 a.fuse = &f;
                 a.ticket = idx->words + W_TICKET;
                 if (tune.pool_select && kp == 64) {
-                    const size_t need = scan_pool_words(plan);
+                    // under the lowered thresholds of the bf16 scan a near-tie burst may send any number of keys to the pool:
+                    // room for one per row (each row's key enters the pool at most once)
+                    const size_t need = scan_pool_words(plan) + (shadow ? (size_t)idx->ntotal : 0);
                     if (idx->pool_cap < need) {  // (re)allocated zeroed; every search's last CTA leaves it zeroed
                         if (idx->pool) CU(cudaFree(idx->pool));
                         idx->pool = nullptr;
@@ -1663,6 +1730,20 @@ extern "C" int evs_index_guard_stats(evs_index* idx, int64_t* reruns, int64_t* u
     return EVS_OK;
 }
 
+extern "C" int evs_index_shadow_stats(evs_index* idx, int64_t* wide_searches, float* emax, int64_t* last_candidates) {
+    if (!idx) return fail(EVS_EINVAL, "idx is NULL");
+    std::lock_guard<std::mutex> lk(idx->mu);
+    int rc = use_device(idx->device);
+    if (rc) return rc;
+    if (idx->have_last_stream) CU(cudaStreamSynchronize(idx->last_stream));
+    unsigned w[2] = {0, 0};
+    CU(cudaMemcpy(w, idx->words + W_WIDE, sizeof(w), cudaMemcpyDeviceToHost));  // W_WIDE, W_LASTC are adjacent
+    if (wide_searches) *wide_searches = (int64_t)w[0];
+    if (last_candidates) *last_candidates = (int64_t)w[1];
+    if (emax) *emax = idx->xb16 ? idx->emax_host : -1.f;
+    return EVS_OK;
+}
+
 extern "C" int evs_index_max_row_norm(evs_index* idx, float* max_norm) {
     if (!idx || !max_norm) return fail(EVS_EINVAL, "NULL argument");
     std::lock_guard<std::mutex> lk(idx->mu);
@@ -2115,24 +2196,23 @@ extern "C" int evs_index_set_storage(evs_index* idx, int storage) {
     if (storage == idx->storage) return EVS_OK;
     CU(cudaDeviceSynchronize());  // no search may be in flight while the scan rows change
     if (storage == EVS_STORE_F32) {
-        cudaFree(idx->xb16);
-        idx->xb16 = nullptr;
+        if (!shadow_wanted()) {  // otherwise the copy stays: it is the fp32 index's scan copy
+            cudaFree(idx->xb16);
+            idx->xb16 = nullptr;
+        }
         idx->storage = storage;
         return EVS_OK;
     }
-    if (idx->capacity > 0) {
-        void* n16 = nullptr;
-        cudaError_t e = cudaMalloc(&n16, (size_t)idx->capacity * idx->d * 2);
-        if (e != cudaSuccess) return fail(EVS_ENOMEM, "cudaMalloc of the bf16 copy failed: %s", cudaGetErrorString(e));
+    if (idx->capacity > 0 && idx->xb16 == nullptr) {
+        CU(cudaMalloc(&idx->xb16, (size_t)idx->capacity * idx->d * 2));
         if (idx->ntotal > 0) {
-            e = launch_f32_to_bf16(idx->xb32, n16, (long long)idx->ntotal * idx->d, idx->sm_count, idx->stream);
-            if (e == cudaSuccess) e = cudaStreamSynchronize(idx->stream);
-            if (e != cudaSuccess) {
-                cudaFree(n16);
-                return fail(EVS_ECUDA, "bf16 layout kernel failed: %s", cudaGetErrorString(e));
+            const int rc2 = derive_rows_locked(idx, 0, idx->ntotal);
+            if (rc2) {
+                cudaFree(idx->xb16);
+                idx->xb16 = nullptr;
+                return rc2;
             }
         }
-        idx->xb16 = n16;
     }
     idx->storage = storage;
     return EVS_OK;

@@ -290,9 +290,13 @@ __device__ __forceinline__ void exchange_merge(const Exchange& x, long long qi, 
 // has a smaller scan key.  Canonical re-score, ranking, output (final / shard partial / peer stores + fused merge), margin
 // and certification.  Called by every thread of the CTA; `scratch` holds at least max(world * k * 24 + 8, 0) bytes that
 // no longer hold anything needed (the exchange merge ranks the gathered partials there).
+// shadow_E > 0 (the pool kernel over bf16 rows, evs_scan.cuh): A holds EVERY row whose scan key is >= cut (1: every row),
+// unsorted, and every other row's scan score is below key_score(cut); the result is exact by construction and the margin is
+// the canonical score of rank k minus (that scan score + E).
 template <int MAXR = 4, int UW = 0>  // candidates a warp re-scores at a time at most (kernels held to 64 registers pass 2)
 __device__ __forceinline__ void finalize_rank_emit(const FinalizeParams& p, long long qi, const u64* A, FinalizeShared* sh, double* sc,
-                                                   long long* id, u64* ok, const double* qs, unsigned char* scratch, int kp_use = 0) {
+                                                   long long* id, u64* ok, const double* qs, unsigned char* scratch, int kp_use = 0,
+                                                   float shadow_E = 0.f, u64 cut = 0ull) {
     const int t = threadIdx.x, nt = blockDim.x;
     const int warp = t >> 5, lane = t & 31, nwarps = nt >> 5;
     const int kp = kp_use > 0 ? kp_use : p.kp;  // kp_use: only the best kp_use (<= p.kp) entries of A are candidates
@@ -367,7 +371,9 @@ __device__ __forceinline__ void finalize_rank_emit(const FinalizeParams& p, long
                 p.P_scores[(size_t)qi * p.k + rank] = st;
                 p.P_ids[(size_t)qi * p.k + rank] = it + p.id_base;
             }
-            if (rank == p.k - 1 && want_margin) {
+            if (rank == p.k - 1 && want_margin && shadow_E > 0.f) {
+                if (p.margins) p.margins[qi] = cut > 1ull ? (float)(st - widen_f32(key_score(cut))) - shadow_E : INFINITY;
+            } else if (rank == p.k - 1 && want_margin) {
                 // All kp slots taken -> every row outside the list has a scan score <= the worst retained one, so its
                 // true score is at most that plus the scan's error.  margin = canonical score of rank k minus (worst
                 // retained scan score + the largest under-estimate observed on the retained candidates); the result is

@@ -42,6 +42,11 @@ struct ScanTuning {
                                  // stored by row, threshold from 128 chunk maxima; 10k x 512: 27 -> ~20 us); 0 = never
     int small_fast_cap = 2048;   // ... whose last CTA takes the register fast path up to this many keys above the threshold (tests
                                  // lower it to drive the general path)
+    int scan_shadow = 1;         // fp32 indexes keep a bf16 scan copy (built at add); single-query searches with k <= 48 of shards
+                                 // of at least shadow_min_rows rows scan it -- half the bytes -- and stay exact (scan_pool_kernel)
+    int shadow_min_rows = 131072;  // below it the fp32 rows are scanned: in a shard whose warps see fewer than 128 rows each the
+                                   // pool receives nearly every key and the last CTA reads it twice (65 536 x 512: 50 us against
+                                   // 37 us; 250 000: 64 against 93 us; profiles/shadow_min_rows_sweep.jsonl)
 };
 
 struct ScanPlan {
@@ -119,6 +124,12 @@ struct FinalizeParams {
     unsigned long long* dbg = nullptr;          // diagnostics (option "scan_clock"): %globaltimer stamps of the finalise's phases
     unsigned* done_flag = nullptr;              // host-mapped word (scan_small_kernel with the query in its parameters): set to
     unsigned done_seq = 0;                      //   done_seq behind the results, polled by evs_index_search
+    // pool kernel scanning a bf16 copy of the fp32 master rows (scan_pool_kernel): the scan error is bounded by
+    // E = |q| (emax + gamma * max|x| (1 + 2^-7)) and the thresholds are lowered by 2E, which makes the result exact
+    const float* shadow_emax = nullptr;         // device: largest |x - bf16(x)|_2 of a row (null: the scan is not bounded this way)
+    float shadow_gamma = 0.f;                   // fp32 accumulation error of the scan relative to |q| |x|
+    unsigned* wide = nullptr;                   // device counter: searches that re-scored more than POOL_KPMAX candidates;
+                                                //   wide[1] = the number of candidates the last search re-scored
 };
 
 struct ScanArgs {
@@ -251,8 +262,10 @@ cudaError_t launch_gather_rows(const float* src, const long long* ids_dev, float
 cudaError_t launch_synth_fill(float* out, long long n, int d, unsigned long long seed, long long row_base, int sm_count,
                               cudaStream_t st);
 // max_norm[0] = max(max_norm[0], largest |row|) over rows [0, n): float bits compared as unsigned (norms are >= 0);
-// NaN rows are ignored.  *special |= 1 when a row holds a subnormal, infinite or NaN element.
-cudaError_t launch_row_norm_max(const float* rows, long long n, int d, float* max_norm, unsigned* special, int sm_count, cudaStream_t st);
+// NaN rows are ignored.  *special |= 1 when a row holds a subnormal, infinite or NaN element.  dst16 != null: the same pass
+// writes the rows rounded to bf16 there and raises *emax (float bits) to the largest |x - bf16(x)|_2 of a row.
+cudaError_t launch_row_norm_max(const float* rows, long long n, int d, float* max_norm, unsigned* special, int sm_count, cudaStream_t st,
+                                void* dst16 = nullptr, float* emax = nullptr);
 // small device fills used on the search path instead of memset nodes
 cudaError_t launch_fill_i32(int* p, long long count, int value, cudaStream_t st);
 

@@ -365,15 +365,29 @@ __device__ __forceinline__ unsigned is_special_f32(float x) {
     const unsigned t = __float_as_uint(x) & 0x7FFFFFFFu;
     return (t != 0u && (t - 0x00800000u) >= 0x7F000000u) ? 1u : 0u;
 }
+// With dst16 != null the same pass also writes the rows rounded to bf16 (RNE) and raises *emax to the largest
+// |x - bf16(x)|_2 of a row, summed in fp64 and rounded up: the bound the single-query scans of the bf16 copy are made exact
+// with (evs_scan.cuh: scan_pool_kernel).  An element that rounds to a bf16 infinity marks the index special.
 __global__ void __launch_bounds__(256) row_norm_max_kernel(const float* __restrict__ rows, long long n, int d, float* __restrict__ max_norm,
-                                                          unsigned* __restrict__ special) {
+                                                          unsigned* __restrict__ special, __nv_bfloat16* __restrict__ dst16,
+                                                          float* __restrict__ emax) {
     const int lane = threadIdx.x & 31;
     const long long warps = ((long long)gridDim.x * blockDim.x) >> 5;
     float best = 0.f;
+    double ebest = 0.0;
     unsigned spec = 0u;
+    auto to16 = [&](float v, double& e2) {
+        const __nv_bfloat16 h = __float2bfloat16_rn(v);
+        const float hf = __bfloat162float(h);
+        const double diff = (double)v - (double)hf;
+        e2 = fma(diff, diff, e2);
+        spec |= (isinf(hf) && !isinf(v)) ? 1u : 0u;
+        return h;
+    };
     for (long long r = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < n; r += warps) {
         const float* x = rows + (size_t)r * d;
         float s = 0.f;
+        double e2 = 0.0;
         if ((d & 3) == 0) {
             for (int i = lane; i < (d >> 2); i += 32) {
                 const float4 v = ldg_stream_f4(reinterpret_cast<const float4*>(x) + i);
@@ -382,19 +396,36 @@ __global__ void __launch_bounds__(256) row_norm_max_kernel(const float* __restri
                 s = fmaf(v.z, v.z, s);
                 s = fmaf(v.w, v.w, s);
                 spec |= is_special_f32(v.x) | is_special_f32(v.y) | is_special_f32(v.z) | is_special_f32(v.w);
+                if (dst16) {
+                    __nv_bfloat162 o0, o1;
+                    o0.x = to16(v.x, e2);
+                    o0.y = to16(v.y, e2);
+                    o1.x = to16(v.z, e2);
+                    o1.y = to16(v.w, e2);
+                    uint2 o;
+                    o.x = *reinterpret_cast<uint32_t*>(&o0);
+                    o.y = *reinterpret_cast<uint32_t*>(&o1);
+                    reinterpret_cast<uint2*>(dst16 + (size_t)r * d)[i] = o;
+                }
             }
         } else {
             for (int i = lane; i < d; i += 32) {
                 s = fmaf(x[i], x[i], s);
                 spec |= is_special_f32(x[i]);
+                if (dst16) dst16[(size_t)r * d + i] = to16(x[i], e2);
             }
         }
 #pragma unroll
-        for (int off = 16; off >= 1; off >>= 1) s += __shfl_xor_sync(0xffffffffu, s, off);
+        for (int off = 16; off >= 1; off >>= 1) {
+            s += __shfl_xor_sync(0xffffffffu, s, off);
+            e2 += __shfl_xor_sync(0xffffffffu, e2, off);
+        }
         if (s == s) best = fmaxf(best, s);
+        if (e2 > ebest) ebest = e2;  // (NaN rows mark the index special: its single-query searches scan the fp32 rows)
     }
     if (lane == 0 && best > 0.f) atomicMax(reinterpret_cast<unsigned*>(max_norm), __float_as_uint(sqrtf(best) * 1.000001f));
     if (spec && special) atomicOr(special, 1u);  // the index holds a subnormal / inf / NaN element: the finalise widens fp32 -> fp64 the slow exact way
+    if (lane == 0 && emax && ebest > 0.0) atomicMax(reinterpret_cast<unsigned*>(emax), __float_as_uint(__double2float_ru(__dsqrt_ru(ebest))));
 }
 
 __global__ void fill_i32_kernel(int* __restrict__ p, long long count, int value) {
@@ -583,10 +614,11 @@ cudaError_t launch_merge_exchange(const Exchange& x, long long nq, int k, float*
     return cudaGetLastError();
 }
 
-cudaError_t launch_row_norm_max(const float* rows, long long n, int d, float* max_norm, unsigned* special, int sm_count, cudaStream_t st) {
+cudaError_t launch_row_norm_max(const float* rows, long long n, int d, float* max_norm, unsigned* special, int sm_count, cudaStream_t st,
+                                void* dst16, float* emax) {
     if (n <= 0) return cudaSuccess;
     int grid = clamp_grid((n * 32 + 255) / 256, sm_count * 8);
-    row_norm_max_kernel<<<grid, 256, 0, st>>>(rows, n, d, max_norm, special);
+    row_norm_max_kernel<<<grid, 256, 0, st>>>(rows, n, d, max_norm, special, reinterpret_cast<__nv_bfloat16*>(dst16), emax);
     EVS_LAUNCH_CHECK();
     return cudaSuccess;
 }

@@ -368,6 +368,7 @@ constexpr int POOL_COUNT = POOL_SLOTS * POOL_GSTRIDE;   // word of the survivor 
 constexpr int POOL_TICKET = POOL_COUNT + 16;            // ... of the ticket counter
 constexpr int POOL_HDR = POOL_TICKET + 16;              // u64 words before S
 constexpr int POOL_SURV = 2048;         // survivors the last CTA holds in shared memory at a time
+constexpr int POOL_KPMAX = 256;         // candidates the last CTA re-scores in one round (bf16 scan: the 2E window around rank k)
 __host__ __device__ inline size_t pool_finalize_smem_bytes(int kp, int d, int world_k) {
     size_t surv = (size_t)(POOL_SURV + kp) * 8;
     const size_t merge = (size_t)world_k * 24 + 8;  // the fused exchange merge ranks world * k partials in the same place
@@ -378,6 +379,82 @@ __host__ __device__ inline size_t pool_finalize_smem_bytes(int kp, int d, int wo
 // byte offset of the fp32 query copy of scan_small_kernel<.., QP = true> (behind the finalise area), 16-byte aligned
 __host__ __device__ inline size_t small_query_smem_offset(int kp, int d, int world_k) {
     return (pool_finalize_smem_bytes(kp, d, world_k) + 15) & ~(size_t)15;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Exact single-query search from the bf16 rows (f.shadow_emax != null; DESIGN.md section 2).  For a row x with
+// x^ = bf16_rn(x) and s~ the fp32 scan score of x^:  |q.x - s~| <= |q| |x - x^| + gamma |q| |x^| <= E.
+//   rule 1: a key is dropped only below key_floor(score(t) - 2E), t the score of a key 64 rows are known to reach (a warp's
+//           own 64th best, tau_g): the dropped row's true score is < t - E <= that of each of those 64 rows;
+//   rule 2: the last CTA re-scores every survivor with s~ >= s~_(k) - 2E exactly (C): any row outside C has a true score
+//           < s~_(k) - E, below each of the k best-by-scan rows, so the top k of C is the exact answer.
+// With shadow_emax == null the lowered threshold IS the threshold (twoE = 0): the fp32 scan as before.
+// ---------------------------------------------------------------------------------------------
+__device__ __forceinline__ float shadow_bound(const FinalizeParams& f, double qn2) {
+    const double qn = sqrt(qn2) * (1.0 + 0x1p-20);
+    const double nh = (double)__ldg(f.max_norm) * (1.0 + 0x1p-7);  // |x^_i| <= |x_i| (1 + 2^-8); max_norm is an fp32 estimate
+    const double e = qn * ((double)__ldg(f.shadow_emax) + (double)f.shadow_gamma * nh) * (1.0 + 0x1p-20) + f.d * 0x1p-149;
+    return __double2float_ru(e);  // inf when it does not fit: every key is kept below
+}
+// the smallest key of score score(t) - 2E (rounded down); 1 (every key) without a finite bound
+__device__ __forceinline__ u64 key_lowered(u64 t, float twoE) {
+    if (twoE == 0.f || t == 0ull) return t;
+    if (!(twoE <= FLT_MAX)) return 1ull;
+    const uint32_t o = score_to_ordered(__fsub_rd(key_score(t), twoE));
+    return o == 0u ? 1ull : ((u64)o << 32);
+}
+
+// C has more than POOL_KPMAX keys (near-tie bursts): walk the pool in blocks of 128 keys and, whenever the next block may not
+// fit, re-score what was gathered and keep its exact top k (as scan keys: a row re-scores to the same canonical score) in
+// front of the buffer.  Returns the number of candidates left in cand[] for the final ranking.  Called by all threads.
+__device__ __forceinline__ int pool_wide_rounds(const FinalizeParams& f, const u64* S, unsigned m, u64 cut, u64* cand, u64* keep,
+                                             double* sc, long long* id, u64* ok, const double* qs, int* s_n) {
+    const int t = threadIdx.x, nt = blockDim.x, warp = t >> 5, lane = t & 31, nwarps = nt >> 5;
+    const float* xb32 = reinterpret_cast<const float*>(f.xb);
+    const bool fastw = f.special != nullptr && __ldg(f.special) == 0u;
+    int fill = 0;  // CTA-uniform
+    for (unsigned b0 = 0; b0 < m; b0 += 128) {
+        const u64 key = (t < 128 && b0 + t < m) ? __ldcg(S + b0 + t) : 0ull;
+        const bool mem = key != 0ull && key >= cut;
+        const int nb = __syncthreads_count(mem);
+        if (fill + nb > POOL_KPMAX) {
+            for (int c = 2 * warp; c < fill; c += 2 * nwarps) {
+                long long row[2];
+                const float* xr[2];
+                double sv[2];
+#pragma unroll
+                for (int r = 0; r < 2; r++) {
+                    row[r] = c + r < fill ? (long long)key_row(cand[c + r]) : -1;
+                    xr[r] = row[r] >= 0 ? xb32 + (size_t)row[r] * f.d : nullptr;
+                }
+                if (fastw) canon32_dot_multi<2, true>(xr, qs, f.d, lane, sv);
+                else canon32_dot_multi<2, false>(xr, qs, f.d, lane, sv);
+                if (lane == 0)
+#pragma unroll
+                    for (int r = 0; r < 2; r++)
+                        if (c + r < fill) {
+                            sc[c + r] = sv[r];
+                            id[c + r] = row[r];
+                            ok[c + r] = score_rank_key(sv[r]);
+                        }
+            }
+            __syncthreads();
+            for (int c = t; c < fill; c += nt) {
+                int rank = 0;
+                for (int j = 0; j < fill; j++) rank += better_i(ok[j], id[j], ok[c], id[c]);
+                if (rank < f.k) keep[rank] = cand[c];
+            }
+            __syncthreads();
+            fill = fill < f.k ? fill : f.k;
+            for (int c = t; c < fill; c += nt) cand[c] = keep[c];
+        }
+        if (t == 0) *s_n = fill;
+        __syncthreads();
+        if (mem) cand[atomicAdd(s_n, 1)] = key;
+        fill += nb;
+        __syncthreads();
+    }
+    return fill;
 }
 
 __device__ __forceinline__ u64 warp_min_u64(u64 v) {
@@ -408,7 +485,8 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ int s_last, s_ns, s_wcnt[9];
     __shared__ unsigned s_base;
-    __shared__ u64 s_tau;
+    __shared__ u64 s_tau, s_wtau[8];  // s_wtau: each warp's running threshold (read only when it compacts: registers stay for the loop)
+    __shared__ float s_twoE;
     typedef typename RawVec<T>::type raw_t;
     constexpr int QREGS = NV * Elem<T>::VEC;
     constexpr int RPG_RAW = (100 - QREGS) / (NV * 4);
@@ -435,8 +513,8 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
     QueryRegs<T, 1, NV> q;
     q.load(p.xq, p.q0, p.d, lane);
     int cnt = 0;
-    u64 tau = 0ull;
     bool early = false;
+    if (lane == 0) s_wtau[warp] = 0ull;
     // the last CTA's re-score wants the query in fp64: every CTA widens it now, off the critical path (the area lies behind
     // the warps' buffers and is not touched in between)
     double* qs;
@@ -444,10 +522,23 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
         size_t surv_bytes = (size_t)(POOL_SURV + KP) * 8;
         const size_t merge = (size_t)f.x.world * f.k * 24 + 8;
         if (merge > surv_bytes) surv_bytes = (merge + 7) & ~(size_t)7;
-        qs = reinterpret_cast<double*>(smem_raw + sizeof(FinalizeShared) + surv_bytes + 3 * (size_t)KP * 8);
+        qs = reinterpret_cast<double*>(smem_raw + sizeof(FinalizeShared) + surv_bytes + 3 * (size_t)POOL_KPMAX * 8);
         const float* qf = p.xq + (size_t)p.q0 * p.d;
         for (int i = threadIdx.x; i < p.d; i += blockDim.x) qs[i] = (double)qf[i];
     }
+    // bf16 rows under the rounding bound: thresholds are lowered by 2E (rules 1 and 2 above); every warp derives the same E
+    // (each warp stores the same bits to s_twoE; nothing reads it before the barrier ahead of the last CTA's work)
+    if (f.shadow_emax != nullptr) {
+        __syncthreads();  // qs complete
+        double s2 = 0.0;
+        for (int i = lane; i < p.d; i += 32) s2 = fma(qs[i], qs[i], s2);
+#pragma unroll
+        for (int off = 16; off >= 1; off >>= 1) s2 += __shfl_xor_sync(0xffffffffu, s2, off);
+        if (lane == 0) s_twoE = 2.f * shadow_bound(f, s2);
+    } else if (threadIdx.x == 0) {
+        s_twoE = 0.f;
+    }
+    u64 tcut = 0ull;  // = key_lowered(own threshold, 2E): what a key must beat to enter the buffer
 
     // buffer full: sort, keep the best 64, publish the best 8 where they raise their slot (a warp sees ~n / warps rows: whatever it holds of the shard's
     // best few hundred is among its own best 8), raise the threshold to max(own 64th best, tau_g)
@@ -458,9 +549,26 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
         u64 ga, gb;
         const u64 tg = pool_tau(G, lane, ga, gb);
         pool_publish(G, lane < 8 ? buf[lane] : 0ull, ga, gb);
-        tau = umax64(tau, umax64(buf[KP - 1], tg));
-        const u64 k0 = buf[lane], k1 = buf[lane + 32];  // sorted: the keys >= tau are a prefix
-        cnt = __popc(__ballot_sync(0xffffffffu, k0 != 0ull && k0 >= tau)) + __popc(__ballot_sync(0xffffffffu, k1 != 0ull && k1 >= tau));
+        const u64 tau = umax64(s_wtau[warp], umax64(buf[KP - 1], tg));
+        __syncwarp();
+        if (lane == 0) s_wtau[warp] = tau;
+        tcut = key_lowered(tau, f.shadow_emax ? s_twoE : 0.f);
+        cnt = 0;
+#pragma unroll
+        for (int h = 0; h < CAPW / 32; h++) {  // sorted: the keys >= tcut are a prefix (of at most KP when tcut = tau)
+            const u64 kh = buf[lane + 32 * h];
+            cnt += __popc(__ballot_sync(0xffffffffu, kh != 0ull && kh >= tcut));
+        }
+        if (cnt > CAPW - 32) {
+            // lowered threshold, near-tie burst: the best KP stay, the rest of the window goes to the pool (which has room for
+            // one key per row: a key is in the pool or in a buffer, never both)
+            unsigned b = 0;
+            if (lane == 0) b = atomicAdd(count, (unsigned)(cnt - KP));
+            b = __shfl_sync(0xffffffffu, b, 0);
+            for (int i = KP + lane; i < cnt; i += 32) S[b + i - KP] = buf[i];
+            cnt = KP;
+            __syncwarp();
+        }
     };
 
     auto do_group = [&](long long g) {
@@ -482,7 +590,7 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
             row_scores<T, 1, NV>(raw[r], q, s);
             if (r0 + r < p.n) {
                 const u64 key = make_key(s[0], (uint32_t)(r0 + r));  // warp-uniform
-                if (key > tau) {
+                if (key > tcut) {
                     if (lane == 0) buf[cnt] = key;
                     if (++cnt == CAPW) compact();
                     else if (cnt == 16 && !early) {
@@ -532,11 +640,12 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
     {
         __syncwarp();
         u64 ga, gb;
-        tau = umax64(tau, pool_tau(G, lane, ga, gb));
+        const u64 tg = pool_tau(G, lane, ga, gb);
+        tcut = key_lowered(umax64(s_wtau[warp], tg), f.shadow_emax ? s_twoE : 0.f);
         int kept = 0;
         for (int i0 = 0; i0 < cnt; i0 += 32) {  // warp-uniform
             const u64 key = (i0 + lane < cnt) ? buf[i0 + lane] : 0ull;
-            const bool keep = key != 0ull && key >= tau;
+            const bool keep = key != 0ull && key >= tcut;
             const unsigned m = __ballot_sync(0xffffffffu, keep);
             __syncwarp();
             if (keep) buf[kept + __popc(m & ((1u << lane) - 1u))] = key;  // kept <= i0: never ahead of the reads
@@ -585,8 +694,8 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
         if (merge > surv_bytes) surv_bytes = (merge + 7) & ~(size_t)7;
     }
     double* sc = reinterpret_cast<double*>(smem_raw + sizeof(FinalizeShared) + surv_bytes);
-    long long* id = reinterpret_cast<long long*>(sc + KP);
-    u64* ok = reinterpret_cast<u64*>(id + KP);  // qs (filled at kernel start) follows
+    long long* id = reinterpret_cast<long long*>(sc + POOL_KPMAX);
+    u64* ok = reinterpret_cast<u64*>(id + POOL_KPMAX);  // qs (filled at kernel start) follows
     if (p.cta_clock && t == 0) {
         unsigned long long* x = p.cta_clock + 2 * gridDim.x;
         x[0] = globaltimer_ns();  // this (the last) CTA holds its ticket
@@ -759,7 +868,42 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
         A = surv;
     }
     fin_stamp(f, 2);  // the KP best ranked
-    finalize_rank_emit<(ScanOcc<T, 1, NV>::value >= 4 ? 2 : 4)>(f, p.q0, A, sh, sc, id, ok, qs, reinterpret_cast<unsigned char*>(surv));
+    const float twoE = s_twoE;
+    if (f.shadow_emax == nullptr) {
+        finalize_rank_emit<(ScanOcc<T, 1, NV>::value >= 4 ? 2 : 4)>(f, p.q0, A, sh, sc, id, ok, qs, reinterpret_cast<unsigned char*>(surv));
+    } else {
+        // rule 2: C = every pool key >= key_lowered(s~_(k)), read again from the pool (the survivors above were cut at the
+        // plain KP-th best).  Every key C needs is in the pool: rule 1 never dropped one.
+        const u64 kth = A[f.k - 1];
+        __syncthreads();  // A lives in surv: read before C is gathered there
+        const u64 cut = kth ? key_lowered(kth, twoE) : 1ull;  // fewer than k keys: all of them
+        u64* cand = surv;
+        if (t == 0) s_ns = 0;
+        __syncthreads();
+        for (unsigned i = t; i < m; i += nt) {
+            const u64 key = __ldcg(S + i);
+            if (key != 0ull && key >= cut) {
+                const int pos = atomicAdd(&s_ns, 1);
+                if (pos < POOL_KPMAX) cand[pos] = key;
+            }
+        }
+        __syncthreads();
+        int nc = s_ns;
+        if (t == 0 && f.wide) {
+            f.wide[1] = (unsigned)nc;
+            if (nc > POOL_KPMAX) atomicAdd(f.wide, 1u);
+        }
+        if (nc > POOL_KPMAX) nc = pool_wide_rounds(f, S, m, cut, cand, surv + POOL_KPMAX, sc, id, ok, qs, &s_ns);
+        const int lines = (f.d * 4 + 127) / 128;  // the fp32 master rows of C on their way to L2
+        for (int i = t; i < nc * lines; i += nt) {
+            const char* row = reinterpret_cast<const char*>(f.xb) + (size_t)key_row(cand[i / lines]) * f.d * 4 + (size_t)(i % lines) * 128;
+            asm volatile("prefetch.global.L2 [%0];" ::"l"(row));
+        }
+        for (int i = nc + t; i < KP; i += nt) cand[i] = 0ull;  // at least KP slots, empty ones as padding
+        __syncthreads();
+        finalize_rank_emit<(ScanOcc<T, 1, NV>::value >= 4 ? 2 : 4)>(f, p.q0, cand, sh, sc, id, ok, qs, reinterpret_cast<unsigned char*>(surv),
+                                                                     nc > KP ? nc : KP, twoE * 0.5f, cut);
+    }
     if (p.cta_clock && t == 0) p.cta_clock[2 * gridDim.x + 1] = globaltimer_ns();
 }
 

@@ -69,7 +69,7 @@ static cudaError_t launch_scan_t(const ScanArgs& a, ScanPlan* plan, cudaStream_t
             }
             const size_t fs = pool_finalize_smem_bytes(64, f.d, f.x.world * f.k);
             smem = (size_t)(plan->threads / 32) * 128 * 8;
-            if (fs > smem) smem = fs;
+            if (fs + 3 * (size_t)(POOL_KPMAX - 64) * 8 > smem) smem = fs + 3 * (size_t)(POOL_KPMAX - 64) * 8;  // the pool kernel re-scores up to POOL_KPMAX
             if (a.small_fast_cap > 0) {  // small shard: keys by row, threshold from the chunk maxima (no buffers: only the finalise area)
                 const int cap = a.small_fast_cap < POOL_SURV ? a.small_fast_cap : POOL_SURV;
                 cudaError_t se;

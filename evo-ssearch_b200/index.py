@@ -131,6 +131,14 @@ class IndexFlatIP:
         check(lib().evs_index_guard_stats(self._h, ctypes.byref(r), ctypes.byref(u)))
         return r.value, u.value
 
+    def shadow_stats(self):
+        """``(wide_searches, emax, last_candidates)``: single-query searches of the bf16 scan copy that re-scored more
+        candidates than one round holds (near-tie bursts), the largest ``|x - bf16(x)|_2`` of a row (-1 without a copy),
+        and how many candidates the last such search re-scored exactly."""
+        w, e, c = ctypes.c_int64(0), ctypes.c_float(0), ctypes.c_int64(0)
+        check(lib().evs_index_shadow_stats(self._h, ctypes.byref(w), ctypes.byref(e), ctypes.byref(c)))
+        return w.value, e.value, c.value
+
     def scan_clocks(self) -> np.ndarray:
         """Diagnostics (option ``scan_clock``): ``uint64[nctas, 2]`` start / end-of-scan-loop times (ns) of the CTAs of
         the last fused single-query scan."""

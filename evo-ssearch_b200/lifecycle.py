@@ -44,9 +44,10 @@ load_stats = {"loads": 0, "bytes": 0, "seconds": 0.0, "evictions": 0}  # what th
 
 
 def _index_bytes(index) -> int:
-    per_row = index.d * (6 if getattr(index, "storage", "f32") == "bf16" else 4)
     local = getattr(index, "local", index)  # a sharded index holds only its block on this GPU
-    return int(local.ntotal) * per_row
+    # fp32 rows, plus the bf16 copy of bf16 storage or of an fp32 index built with the option "scan_shadow" on
+    copy = getattr(index, "storage", "f32") == "bf16" or (hasattr(local, "shadow_stats") and local.shadow_stats()[1] >= 0)
+    return int(local.ntotal) * index.d * (6 if copy else 4)
 
 
 def _signature(index_path: Path):

@@ -89,7 +89,8 @@ EVS_API int evs_index_storage(const evs_index* idx, int* storage);
 EVS_API int evs_index_set_id_base(evs_index* idx, int64_t base);
 EVS_API int evs_index_id_base(const evs_index* idx, int64_t* base);
 /* switch the scan precision in place: EVS_STORE_BF16_F32 derives the bf16 scan copy of an fp32-storage index (large query
- * batches otherwise scan in tf32 straight from the fp32 rows), EVS_STORE_F32 drops it.  Waits for searches in flight. */
+ * batches otherwise scan in tf32 straight from the fp32 rows), EVS_STORE_F32 drops it (keeps it as the scan copy of the
+ * fp32 index while the option "scan_shadow" is on).  Waits for searches in flight. */
 EVS_API int evs_index_set_storage(evs_index* idx, int storage);
 /* largest row norm of the index (maintained by add; it scales the certification bound of the searches) */
 EVS_API int evs_index_max_row_norm(evs_index* idx, float* max_norm);
@@ -199,6 +200,10 @@ EVS_API int evs_index_last_margins(evs_index* idx, int64_t nq, float* margins_ho
 /* counters of this handle: queries finalised again from the device-side exact re-run, and results that stayed
  * uncertified (more than k' - k rows within the scan error of rank k: ties at fp32 resolution) */
 EVS_API int evs_index_guard_stats(evs_index* idx, int64_t* reruns, int64_t* uncertified);
+/* the bf16 scan copy: single-query searches that re-scored more candidates than one round holds (bursts of near-ties
+ * around rank k: slower, never wrong), the largest |x - bf16(x)|_2 of a row (-1 when the index has no copy), and the number
+ * of candidates the last such search re-scored exactly */
+EVS_API int evs_index_shadow_stats(evs_index* idx, int64_t* wide_searches, float* emax, int64_t* last_candidates);
 
 /* ---- persistence: <folder>/.clip_index/index.faiss -------------------------------------------
  * evs_index_write       <- faiss.write_index(index, path)           oldapp.py:98
@@ -254,6 +259,12 @@ EVS_API int evs_f32_to_bf16_dev(int device, const float* src_dev, void* dst_dev,
  *                 "small_max_rows" (default 32768; 0 = never): single-query searches (k <= 48) of shards up to this many rows take
  *                 the small-shard kernel (keys stored by row, threshold from 128 chunk maxima: 10k x 512 in 16 us instead of 27);
  *                 "small_fast_cap" (default 2048, tests lower it): its register fast path up to this many keys above the threshold;
+ *                 "scan_shadow" (default 1): an fp32 index added to while it is on keeps a bf16 copy of its rows (+50 % device
+ *                 memory; added to while it is off, it drops the copy).  Single-query searches (k <= 48) of shards above
+ *                 small_max_rows and of at least "shadow_min_rows" rows (default 131072) scan that copy -- half the bytes --
+ *                 under a proven bound on its rounding, so their results
+ *                 are those of the fp32 scan (DESIGN.md section 2); bf16-storage indexes search the same way.  Indexes with
+ *                 subnormal, infinite or NaN elements scan their fp32 rows;
  *                 "io_threads" (default 0 = auto: one per hardware thread, at most 16): threads that pread each 64 MiB chunk of
  *                 index.faiss into the pinned staging buffers (evs_index_read[_rows]; 6.5 GB/s with 1, 35 GB/s with 16);
  *                 "exchange_fail_next" (tests): the next exchange-mode search of this process fails after taking its
