@@ -67,17 +67,19 @@ static const int kTcQueryChunk = 4096;  // tensor-core path: queries per launch 
 // per-handle device words (idx->words): counters the kernels share across searches
 enum { W_TICKET = 0, W_NEXT_CHUNK = 1, W_GUARD_COUNT0 = 2, W_GUARD_COUNT1 = 3, W_UNCERT = 4 /* u64 */, W_RERUNS = 6 /* u64 */,
        W_MAX_NORM = 8 /* float */, W_SPECIAL = 9, W_BAR = 10 /* 3 words: grid barrier of the in-launch pre-pass */,
-       W_EMAX = 13 /* float: largest |x - bf16(x)|_2 of a row of the bf16 copy */, W_WIDE = 14 /* single-query searches of the bf16
+       W_EMAX = 13 /* float: largest |x - s c|_2 of a row of the int8 copy */, W_WIDE = 14 /* single-query searches of the int8
        copy that re-scored more than POOL_KPMAX candidates */, W_LASTC = 15 /* candidates the last of them re-scored */, W_WORDS = 16 };
 
 struct evs_index {
     int d = 0, device = 0, storage = EVS_STORE_F32;
     int64_t ntotal = 0, capacity = 0, id_base = 0;
     float* xb32 = nullptr;            // fp32 rows (the master copy; what index.faiss holds)
-    void* xb16 = nullptr;             // derived bf16 rows (EVS_STORE_BF16_F32, or the scan copy of an fp32 index: option
-                                      // "scan_shadow"); when present it always holds every row, and W_EMAX bounds its rounding
-    unsigned special_host = 0;        // host copies of W_SPECIAL / W_EMAX, read back by every add
-    float emax_host = 0.f;
+    void* xb16 = nullptr;             // derived bf16 rows (EVS_STORE_BF16_F32 only)
+    signed char* xi8 = nullptr;       // the int8 scan copy of the single-query searches (bf16 storage, or an fp32 index while the
+    float* xs8 = nullptr;             //   option "scan_shadow" is on): codes [capacity][d] and one scale per row [capacity];
+                                      //   when present it always holds every row, and W_EMAX bounds its rounding
+    unsigned special_host = 0;        // host copies of W_MAX_NORM, W_SPECIAL and W_EMAX, read back by every add
+    float max_norm_host = 0.f, emax_host = 0.f;
     int sm_count = 0;
     cudaStream_t stream = nullptr;    // the handle's own stream
     cudaEvent_t ws_free = nullptr;    // recorded after each search: the workspace may be reused after it
@@ -332,6 +334,8 @@ extern "C" int evs_index_free(evs_index* idx) {
     cudaDeviceSynchronize();  // searches may still be in flight on the caller's streams
     cudaFree(idx->xb32);
     cudaFree(idx->xb16);
+    cudaFree(idx->xi8);
+    cudaFree(idx->xs8);
     cudaFree(idx->q_dev);
     cudaFree(idx->lists);
     cudaFree(idx->I_dev);  // D_dev points into the same allocation
@@ -377,11 +381,30 @@ extern "C" int evs_index_set_id_base(evs_index* idx, int64_t base) {
     return EVS_OK;
 }
 
-// grow the row storage to hold at least `rows` rows (device-to-device copy of what is there)
 static bool shadow_wanted() {
     std::lock_guard<std::mutex> lk(g_tune_mu);
     return g_tune.scan_shadow != 0;
 }
+// whether an add keeps the int8 scan copy: always for bf16 storage, for fp32 storage while the option "scan_shadow" is on
+static bool copy_wanted(const evs_index* idx) { return idx->storage == EVS_STORE_BF16_F32 || shadow_wanted(); }
+
+static void drop_i8_copy(evs_index* idx) {
+    cudaFree(idx->xi8);
+    cudaFree(idx->xs8);
+    idx->xi8 = nullptr;
+    idx->xs8 = nullptr;
+}
+static int alloc_i8_copy(evs_index* idx) {
+    cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&idx->xi8), (size_t)idx->capacity * idx->d);
+    if (e == cudaSuccess) e = cudaMalloc(reinterpret_cast<void**>(&idx->xs8), (size_t)idx->capacity * sizeof(float));
+    if (e != cudaSuccess) {
+        drop_i8_copy(idx);
+        return fail(EVS_ENOMEM, "cudaMalloc of the int8 copy failed: %s", cudaGetErrorString(e));
+    }
+    return EVS_OK;
+}
+
+// grow the row storage to hold at least `rows` rows (device-to-device copy of what is there)
 
 static int grow_locked(evs_index* idx, int64_t rows) {
     if (rows <= idx->capacity) return EVS_OK;
@@ -389,31 +412,50 @@ static int grow_locked(evs_index* idx, int64_t rows) {
     const size_t d = (size_t)idx->d;
     float* n32 = nullptr;
     void* n16 = nullptr;
+    signed char* n8 = nullptr;
+    float* ns8 = nullptr;
     CU(cudaMalloc(reinterpret_cast<void**>(&n32), (size_t)rows * d * sizeof(float)));
-    // the bf16 copy grows with the rows; an fp32 index that has none yet but holds rows gets it built by its next add
-    if (idx->storage == EVS_STORE_BF16_F32 || idx->xb16 != nullptr || (idx->ntotal == 0 && shadow_wanted())) {
-        cudaError_t e = cudaMalloc(&n16, (size_t)rows * d * 2);
-        if (e != cudaSuccess) {
-            cudaFree(n32);
-            return fail(EVS_ENOMEM, "cudaMalloc of the bf16 copy failed: %s", cudaGetErrorString(e));
-        }
+    // the derived copies grow with the rows; an index that has no int8 copy yet but holds rows gets it built by its next add
+    cudaError_t e = cudaSuccess;
+    if (idx->storage == EVS_STORE_BF16_F32) e = cudaMalloc(&n16, (size_t)rows * d * 2);
+    if (e == cudaSuccess && (idx->xi8 != nullptr || (idx->ntotal == 0 && copy_wanted(idx)))) {
+        e = cudaMalloc(reinterpret_cast<void**>(&n8), (size_t)rows * d);
+        if (e == cudaSuccess) e = cudaMalloc(reinterpret_cast<void**>(&ns8), (size_t)rows * sizeof(float));
+    }
+    if (e != cudaSuccess) {
+        cudaFree(n32);
+        cudaFree(n16);
+        cudaFree(n8);
+        cudaFree(ns8);
+        return fail(EVS_ENOMEM, "cudaMalloc of the derived row copies failed: %s", cudaGetErrorString(e));
     }
     if (idx->ntotal > 0) {
-        cudaError_t e = cudaMemcpyAsync(n32, idx->xb32, (size_t)idx->ntotal * d * sizeof(float), cudaMemcpyDeviceToDevice, idx->stream);
+        e = cudaMemcpyAsync(n32, idx->xb32, (size_t)idx->ntotal * d * sizeof(float), cudaMemcpyDeviceToDevice, idx->stream);
         if (e == cudaSuccess && n16 && idx->xb16)
             e = cudaMemcpyAsync(n16, idx->xb16, (size_t)idx->ntotal * d * 2, cudaMemcpyDeviceToDevice, idx->stream);
+        if (e == cudaSuccess && n8 && idx->xi8) {
+            e = cudaMemcpyAsync(n8, idx->xi8, (size_t)idx->ntotal * d, cudaMemcpyDeviceToDevice, idx->stream);
+            if (e == cudaSuccess)
+                e = cudaMemcpyAsync(ns8, idx->xs8, (size_t)idx->ntotal * sizeof(float), cudaMemcpyDeviceToDevice, idx->stream);
+        }
         const cudaError_t es = cudaStreamSynchronize(idx->stream);  // also on the error path: nothing may still read the old rows
         if (e == cudaSuccess) e = es;
         if (e != cudaSuccess) {
             cudaFree(n32);
             cudaFree(n16);
+            cudaFree(n8);
+            cudaFree(ns8);
             return fail(EVS_ECUDA, "copying the rows into the grown storage failed: %s", cudaGetErrorString(e));
         }
     }
     cudaFree(idx->xb32);
     cudaFree(idx->xb16);
+    cudaFree(idx->xi8);
+    cudaFree(idx->xs8);
     idx->xb32 = n32;
     idx->xb16 = n16;
+    idx->xi8 = n8;
+    idx->xs8 = ns8;
     idx->capacity = rows;
     return EVS_OK;
 }
@@ -427,32 +469,37 @@ static int grow_for_add_locked(evs_index* idx, int64_t n) {
 }
 
 // the rows [r0, r0 + n): largest row norm and special elements (the certification bound of the searches, finalize_query)
-// and -- when the index keeps a bf16 copy -- the copy and its rounding bound, in one pass; then the host copies of the flags
+// and -- when the index keeps them -- the bf16 rows and the int8 copy with its rounding bound, in one pass; then the host
+// copies of the flags
 static int derive_rows_locked(evs_index* idx, int64_t r0, int64_t n) {
     const size_t d = (size_t)idx->d;
     void* dst16 = idx->xb16 ? reinterpret_cast<unsigned char*>(idx->xb16) + (size_t)r0 * d * 2 : nullptr;
+    signed char* dst8 = idx->xi8 ? idx->xi8 + (size_t)r0 * d : nullptr;
+    float* scale8 = idx->xs8 ? idx->xs8 + r0 : nullptr;
     CU(launch_row_norm_max(idx->xb32 + (size_t)r0 * d, (long long)n, idx->d, reinterpret_cast<float*>(idx->words + W_MAX_NORM),
-                           idx->words + W_SPECIAL, idx->sm_count, idx->stream, dst16, reinterpret_cast<float*>(idx->words + W_EMAX)));
+                           idx->words + W_SPECIAL, idx->sm_count, idx->stream, dst16, dst8, scale8,
+                           reinterpret_cast<float*>(idx->words + W_EMAX)));
     CU(cudaStreamSynchronize(idx->stream));
-    unsigned w[W_EMAX - W_SPECIAL + 1];
-    CU(cudaMemcpy(w, idx->words + W_SPECIAL, sizeof(w), cudaMemcpyDeviceToHost));
-    idx->special_host = w[0];
-    memcpy(&idx->emax_host, &w[W_EMAX - W_SPECIAL], sizeof(float));
+    unsigned w[W_EMAX - W_MAX_NORM + 1];
+    CU(cudaMemcpy(w, idx->words + W_MAX_NORM, sizeof(w), cudaMemcpyDeviceToHost));
+    memcpy(&idx->max_norm_host, &w[0], sizeof(float));
+    idx->special_host = w[W_SPECIAL - W_MAX_NORM];
+    memcpy(&idx->emax_host, &w[W_EMAX - W_MAX_NORM], sizeof(float));
     return EVS_OK;
 }
 
-// after new fp32 rows [ntotal, ntotal+n) are in place (enqueued on idx->stream): derive bf16, publish.  An fp32 index keeps
-// its bf16 scan copy while the option "scan_shadow" is on at add time (built over every row if it has none yet) and drops
-// it otherwise.
+// after new fp32 rows [ntotal, ntotal+n) are in place (enqueued on idx->stream): derive the copies, publish.  An fp32 index
+// keeps its int8 scan copy while the option "scan_shadow" is on at add time (built over every row if it has none yet) and
+// drops it otherwise.
 static int finish_add_locked(evs_index* idx, int64_t n) {
-    const bool want16 = idx->storage == EVS_STORE_BF16_F32 || shadow_wanted();
+    const bool want8 = copy_wanted(idx);
     int64_t r0 = idx->ntotal;
-    if (!want16 && idx->xb16) {
+    if (!want8 && idx->xi8) {
         CU(cudaStreamSynchronize(idx->stream));
-        cudaFree(idx->xb16);
-        idx->xb16 = nullptr;
-    } else if (want16 && !idx->xb16) {
-        CU(cudaMalloc(&idx->xb16, (size_t)idx->capacity * idx->d * 2));
+        drop_i8_copy(idx);
+    } else if (want8 && !idx->xi8) {
+        const int rc = alloc_i8_copy(idx);
+        if (rc) return rc;
         r0 = 0;
     }
     int rc = derive_rows_locked(idx, r0, idx->ntotal + n - r0);
@@ -597,7 +644,7 @@ struct PathInfo {
     float err_coef = 0.f;  // scan error bound relative to |q| * max|x| (0 = not certified: bf16 storage)
     float err_trunc = 0.f; // single tf32: the truncation part of the bound, relative to (|q| max|x| + |worst retained score|)
     bool fused = false;  // PATH_GEMV, one query: the scan's last CTA finalises (and, in exchange mode, merges): ONE launch
-    bool shadow = false; // ... with the pool kernel over the bf16 rows under the bound W_EMAX (exact: evs_scan.cuh)
+    bool shadow = false; // ... with the pool kernel over the int8 copy under the bound W_EMAX (exact: evs_scan.cuh)
 };
 
 // scan error models, relative to |q| * |x| (DESIGN.md section 2).  fp32 GEMV: 4 partial chains of d/128 FMAs per lane, 3 + 5
@@ -620,19 +667,19 @@ static bool takes_tc_path(const evs_index* idx, int64_t nq, const ScanTuning& tu
            tc_max_queries(idx->d, idx->storage == EVS_STORE_BF16_F32) > 0;
 }
 
-// A fused single-query search scans the bf16 rows with the pool kernel under the rounding bound (exact for any data) when
-// the copy exists (it always holds every row), the index has no subnormal / inf / NaN element and a finite bound, and the
-// shard is above the small-shard cut (those are L2-resident and latency-bound: scan_small_kernel over the fp32 rows) and
-// holds at least shadow_min_rows rows.
+// A fused single-query search scans the int8 copy with the pool kernel under its bound (exact for any data) when the copy
+// exists (it always holds every row), the index has no subnormal / inf / NaN element, a finite largest norm and a finite
+// bound, d is a multiple of 256 up to 1024, and the shard is above the small-shard cut (those are L2-resident and
+// latency-bound: scan_small_kernel over the fp32 rows) and holds at least shadow_min_rows rows.
 // bf16-storage indexes take the same path; an fp32 index only while the option "scan_shadow" is on.
 static bool shadow_applies(const evs_index* idx, int64_t nq, int kp, const ScanTuning& tune) {
-    if (nq != 1 || !tune.fuse_finalize || !tune.pool_select || kp != 64 || idx->xb16 == nullptr) return false;
+    if (nq != 1 || !tune.fuse_finalize || !tune.pool_select || kp != 64 || idx->xi8 == nullptr) return false;
     if (idx->storage != EVS_STORE_BF16_F32 && !tune.scan_shadow) return false;
-    if (idx->special_host != 0 || !(idx->emax_host <= FLT_MAX) || idx->ntotal <= tune.small_max_rows ||
-        idx->ntotal < tune.shadow_min_rows)
+    if (idx->special_host != 0 || !(idx->emax_host <= FLT_MAX) || !(idx->max_norm_host <= FLT_MAX) ||
+        idx->ntotal <= tune.small_max_rows || idx->ntotal < tune.shadow_min_rows)
         return false;
     ScanPlan plan;
-    return plan_scan(idx->ntotal, idx->d, 1, kp, 1, idx->sm_count, tune, &plan) == cudaSuccess && plan.variant == 1 &&
+    return plan_scan(idx->ntotal, idx->d, SCAN_I8, kp, 1, idx->sm_count, tune, &plan) == cudaSuccess && plan.variant == 1 &&
            plan.threads == 256;
 }
 
@@ -646,7 +693,7 @@ static PathInfo plan_path(const evs_index* idx, int64_t nq, int64_t k, const Sca
             pi.shadow = shadow_applies(idx, nq, pi.kp, tune);
             if (pi.shadow) pi.err_coef = 0.f;  // exact by construction: nothing to certify
             ScanPlan plan;
-            pi.fused = plan_scan(idx->ntotal, idx->d, bf16 || pi.shadow, pi.kp, 1, idx->sm_count, tune, &plan) == cudaSuccess &&
+            pi.fused = plan_scan(idx->ntotal, idx->d, pi.shadow ? SCAN_I8 : bf16, pi.kp, 1, idx->sm_count, tune, &plan) == cudaSuccess &&
                        plan.variant == 1;
         }
         return pi;
@@ -1090,11 +1137,11 @@ static int search_enqueue_locked(evs_index* idx, int64_t nq, const float* q_dev,
     const int kp = kp_override ? kp_override : pi.kp;
     const bool bf16 = idx->storage == EVS_STORE_BF16_F32;
     const bool shadow = pi.shadow && kp_override == 0;
-    const bool scan_bf16 = (bf16 || shadow) && kp_override == 0;  // an exact re-run always scans the fp32 rows
-    const void* scan_rows = scan_bf16 ? idx->xb16 : (const void*)idx->xb32;
-    const int qpp = max_queries_per_pass(idx->d, scan_bf16);
+    const bool scan_bf16 = bf16 && !shadow && kp_override == 0;  // an exact re-run always scans the fp32 rows
+    const void* scan_rows = shadow ? (const void*)idx->xi8 : scan_bf16 ? idx->xb16 : (const void*)idx->xb32;
+    const int qpp = shadow ? 1 : max_queries_per_pass(idx->d, scan_bf16);
     ScanPlan plan;
-    CU(plan_scan(idx->ntotal, idx->d, scan_bf16, kp, qpp, idx->sm_count, tune, &plan));
+    CU(plan_scan(idx->ntotal, idx->d, shadow ? SCAN_I8 : scan_bf16, kp, qpp, idx->sm_count, tune, &plan));
     const int64_t chunk_cap = nq < kQueryChunk ? nq : kQueryChunk;
     int rc = ensure_dev(reinterpret_cast<unsigned long long**>(&idx->lists), &idx->lists_cap, (size_t)chunk_cap * plan.grid * kp);
     if (rc) return rc;
@@ -1105,9 +1152,9 @@ static int search_enqueue_locked(evs_index* idx, int64_t nq, const float* q_dev,
     // single-query searches (what the app issues, oldapp.py:2005): the scan's last CTA finalises -- one launch in all
     const bool fused = (kp_override ? (tune.fuse_finalize && nq == 1 && plan.variant == 1) : pi.fused) && !scan_only;
     if (out.x && out.x->merge_D && !fused) return fail(EVS_ECUDA, "internal: the exchange expected a fused single-query search");
-    const float err_coef = scan_bf16 ? 0.f : gemv_err_coef(idx->d);
-    if (shadow && !(fused && tune.pool_select && kp == 64) && !scan_only)
-        return fail(EVS_ECUDA, "internal: the bf16 scan copy is searched by the fused pool kernel only");
+    const float err_coef = (scan_bf16 || shadow) ? 0.f : gemv_err_coef(idx->d);
+    if (shadow && !(fused && tune.pool_select && kp == 64))
+        return fail(EVS_ECUDA, "internal: the int8 scan copy is searched by the fused pool kernel only");
 
     for (int64_t c0 = 0; c0 < nq; c0 += kQueryChunk) {
         const int64_t cn = (nq - c0) < kQueryChunk ? (nq - c0) : kQueryChunk;
@@ -1117,13 +1164,14 @@ static int search_enqueue_locked(evs_index* idx, int64_t nq, const float* q_dev,
         FinalizeParams f = make_finalize(idx, idx->lists, plan.grid, kp, qc, k, out, c0, nq, err_coef);
         if (shadow) {
             f.shadow_emax = reinterpret_cast<const float*>(idx->words + W_EMAX);
-            f.shadow_gamma = gemv_err_coef(idx->d);
             f.wide = idx->words + W_WIDE;  // W_LASTC follows
         }
         for (int64_t p0 = 0; p0 < cn; p0 += qpp) {
             ScanArgs a;
             a.xb = scan_rows;
+            a.xs = shadow ? idx->xs8 : nullptr;
             a.is_bf16 = scan_bf16;
+            a.is_i8 = shadow;
             a.n = idx->ntotal;
             a.d = idx->d;
             a.xq = qc;
@@ -1135,7 +1183,7 @@ static int search_enqueue_locked(evs_index* idx, int64_t nq, const float* q_dev,
                 a.fuse = &f;
                 a.ticket = idx->words + W_TICKET;
                 if (tune.pool_select && kp == 64) {
-                    // under the lowered thresholds of the bf16 scan a near-tie burst may send any number of keys to the pool:
+                    // under the lowered thresholds of the int8 scan a near-tie burst may send any number of keys to the pool:
                     // room for one per row (each row's key enters the pool at most once)
                     const size_t need = scan_pool_words(plan) + (shadow ? (size_t)idx->ntotal : 0);
                     if (idx->pool_cap < need) {  // (re)allocated zeroed; every search's last CTA leaves it zeroed
@@ -1682,10 +1730,16 @@ extern "C" int evs_index_time_scan(evs_index* idx, int64_t nq, const float* q_de
     SearchOut none;
     const ScanTuning tune = tune_snapshot();
     const PathInfo pi = plan_path(idx, nq, k, tune, true);
-    rc = search_enqueue_locked(idx, nq, q_dev, k, none, st, tune, pi, true);  // warm-up
+    // the int8 copy is scanned only by the fused search kernel: its scan is the whole search, results to the workspace
+    if (pi.shadow && !(rc = host_stage_locked(idx, nq, k))) {
+        none.D = idx->D_dev;
+        none.I = idx->I_dev;
+    }
+    const bool scan_only = !pi.shadow;
+    if (!rc) rc = search_enqueue_locked(idx, nq, q_dev, k, none, st, tune, pi, scan_only);  // warm-up
     if (!rc) {
         cudaEventRecord(e0, st);
-        for (int i = 0; i < iters && !rc; i++) rc = search_enqueue_locked(idx, nq, q_dev, k, none, st, tune, pi, true);
+        for (int i = 0; i < iters && !rc; i++) rc = search_enqueue_locked(idx, nq, q_dev, k, none, st, tune, pi, scan_only);
         cudaEventRecord(e1, st);
     }
     cudaError_t e = cudaStreamSynchronize(st);
@@ -1740,7 +1794,7 @@ extern "C" int evs_index_shadow_stats(evs_index* idx, int64_t* wide_searches, fl
     CU(cudaMemcpy(w, idx->words + W_WIDE, sizeof(w), cudaMemcpyDeviceToHost));  // W_WIDE, W_LASTC are adjacent
     if (wide_searches) *wide_searches = (int64_t)w[0];
     if (last_candidates) *last_candidates = (int64_t)w[1];
-    if (emax) *emax = idx->xb16 ? idx->emax_host : -1.f;
+    if (emax) *emax = idx->xi8 ? idx->emax_host : -1.f;
     return EVS_OK;
 }
 
@@ -2196,15 +2250,19 @@ extern "C" int evs_index_set_storage(evs_index* idx, int storage) {
     if (storage == idx->storage) return EVS_OK;
     CU(cudaDeviceSynchronize());  // no search may be in flight while the scan rows change
     if (storage == EVS_STORE_F32) {
-        if (!shadow_wanted()) {  // otherwise the copy stays: it is the fp32 index's scan copy
-            cudaFree(idx->xb16);
-            idx->xb16 = nullptr;
-        }
+        cudaFree(idx->xb16);
+        idx->xb16 = nullptr;
+        if (!shadow_wanted()) drop_i8_copy(idx);  // otherwise the int8 copy stays: it is the fp32 index's scan copy
         idx->storage = storage;
         return EVS_OK;
     }
-    if (idx->capacity > 0 && idx->xb16 == nullptr) {
+    if (idx->capacity > 0) {  // the bf16 rows, and the int8 copy bf16 storage always keeps, in one pass over the rows
         CU(cudaMalloc(&idx->xb16, (size_t)idx->capacity * idx->d * 2));
+        if (idx->xi8 == nullptr && (rc = alloc_i8_copy(idx))) {
+            cudaFree(idx->xb16);
+            idx->xb16 = nullptr;
+            return rc;
+        }
         if (idx->ntotal > 0) {
             const int rc2 = derive_rows_locked(idx, 0, idx->ntotal);
             if (rc2) {

@@ -162,5 +162,10 @@ __device__ __forceinline__ uint4 ldg_stream_u4(const uint4* p) {
                  : "l"(p));
     return r;
 }
+__device__ __forceinline__ uint2 ldg_stream_u2(const uint2* p) {
+    uint2 r;
+    asm volatile("ld.global.nc.L1::no_allocate.v2.u32 {%0, %1}, [%2];" : "=r"(r.x), "=r"(r.y) : "l"(p));
+    return r;
+}
 
 }  // namespace evs

@@ -42,11 +42,11 @@ struct ScanTuning {
                                  // stored by row, threshold from 128 chunk maxima; 10k x 512: 27 -> ~20 us); 0 = never
     int small_fast_cap = 2048;   // ... whose last CTA takes the register fast path up to this many keys above the threshold (tests
                                  // lower it to drive the general path)
-    int scan_shadow = 1;         // fp32 indexes keep a bf16 scan copy (built at add); single-query searches with k <= 48 of shards
-                                 // of at least shadow_min_rows rows scan it -- half the bytes -- and stay exact (scan_pool_kernel)
-    int shadow_min_rows = 131072;  // below it the fp32 rows are scanned: in a shard whose warps see fewer than 128 rows each the
-                                   // pool receives nearly every key and the last CTA reads it twice (65 536 x 512: 50 us against
-                                   // 37 us; 250 000: 64 against 93 us; profiles/shadow_min_rows_sweep.jsonl)
+    int scan_shadow = 1;         // fp32 indexes keep an int8 scan copy (built at add); single-query searches with k <= 48 of shards
+                                 // of at least shadow_min_rows rows scan it -- a quarter of the bytes -- and stay exact (scan_pool_kernel)
+    int shadow_min_rows = 262144;  // below it the fp32 rows are scanned: the int8 copy's search costs ~64 us however small the
+                                   // shard (the last CTA re-scores a window of ~200 rows in rounds); 131 072 x 512: 64 against
+                                   // 57 us; 262 144: 80 against 97 us (profiles/int8_min_rows_sweep.jsonl)
 };
 
 struct ScanPlan {
@@ -124,17 +124,23 @@ struct FinalizeParams {
     unsigned long long* dbg = nullptr;          // diagnostics (option "scan_clock"): %globaltimer stamps of the finalise's phases
     unsigned* done_flag = nullptr;              // host-mapped word (scan_small_kernel with the query in its parameters): set to
     unsigned done_seq = 0;                      //   done_seq behind the results, polled by evs_index_search
-    // pool kernel scanning a bf16 copy of the fp32 master rows (scan_pool_kernel): the scan error is bounded by
-    // E = |q| (emax + gamma * max|x| (1 + 2^-7)) and the thresholds are lowered by 2E, which makes the result exact
-    const float* shadow_emax = nullptr;         // device: largest |x - bf16(x)|_2 of a row (null: the scan is not bounded this way)
-    float shadow_gamma = 0.f;                   // fp32 accumulation error of the scan relative to |q| |x|
+    // pool kernel scanning the int8 copy of the fp32 master rows (scan_pool_kernel): the scan error is bounded by
+    // E = |q - q^| max|x| + |q^| emax + rounding (evs_scan.cuh: shadow_bound_i8) and the thresholds are lowered by 2E, which
+    // makes the result exact
+    const float* shadow_emax = nullptr;         // device: largest |x - s c|_2 of a row of the int8 copy (null: the scan is not
+                                                //   bounded this way)
     unsigned* wide = nullptr;                   // device counter: searches that re-scored more than POOL_KPMAX candidates;
                                                 //   wide[1] = the number of candidates the last search re-scored
 };
 
+// element type of the rows a scan reads
+enum { SCAN_F32 = 0, SCAN_BF16 = 1, SCAN_I8 = 2 /* the int8 copy: codes in xb, one fp32 scale per row in xs */ };
+
 struct ScanArgs {
     const void* xb = nullptr;
+    const float* xs = nullptr;
     int is_bf16 = 0;
+    int is_i8 = 0;
     long long n = 0;
     int d = 0;
     const float* xq = nullptr;
@@ -239,7 +245,7 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 
-cudaError_t plan_scan(long long n, int d, int is_bf16, int kp, int nq_pass, int sm_count, const ScanTuning& tune,
+cudaError_t plan_scan(long long n, int d, int elem /* SCAN_* */, int kp, int nq_pass, int sm_count, const ScanTuning& tune,
                       ScanPlan* plan);
 int max_queries_per_pass(int d, int is_bf16);
 cudaError_t launch_scan(const ScanArgs& a, ScanPlan* plan, cudaStream_t st);
@@ -263,9 +269,10 @@ cudaError_t launch_synth_fill(float* out, long long n, int d, unsigned long long
                               cudaStream_t st);
 // max_norm[0] = max(max_norm[0], largest |row|) over rows [0, n): float bits compared as unsigned (norms are >= 0);
 // NaN rows are ignored.  *special |= 1 when a row holds a subnormal, infinite or NaN element.  dst16 != null: the same pass
-// writes the rows rounded to bf16 there and raises *emax (float bits) to the largest |x - bf16(x)|_2 of a row.
+// writes the rows rounded to bf16 there.  dst8 != null: it writes the int8 copy (codes to dst8, one scale per row to
+// scale8) and raises *emax (float bits) to the largest |x - s c|_2 of a row.
 cudaError_t launch_row_norm_max(const float* rows, long long n, int d, float* max_norm, unsigned* special, int sm_count, cudaStream_t st,
-                                void* dst16 = nullptr, float* emax = nullptr);
+                                void* dst16 = nullptr, signed char* dst8 = nullptr, float* scale8 = nullptr, float* emax = nullptr);
 // small device fills used on the search path instead of memset nodes
 cudaError_t launch_fill_i32(int* p, long long count, int value, cudaStream_t st);
 

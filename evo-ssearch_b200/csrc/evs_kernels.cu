@@ -365,43 +365,51 @@ __device__ __forceinline__ unsigned is_special_f32(float x) {
     const unsigned t = __float_as_uint(x) & 0x7FFFFFFFu;
     return (t != 0u && (t - 0x00800000u) >= 0x7F000000u) ? 1u : 0u;
 }
-// With dst16 != null the same pass also writes the rows rounded to bf16 (RNE) and raises *emax to the largest
-// |x - bf16(x)|_2 of a row, summed in fp64 and rounded up: the bound the single-query scans of the bf16 copy are made exact
-// with (evs_scan.cuh: scan_pool_kernel).  An element that rounds to a bf16 infinity marks the index special.
+// With dst16 != null the same pass also writes the rows rounded to bf16 (RNE); an element that rounds to a bf16 infinity
+// marks the index special.  With dst8 != null it writes the int8 scan copy: per row the scale s = max|x_i| / 127 (fp32) to
+// scale8 and the codes c_i = rint(x_i / s) (|c_i| <= 127) to dst8, and raises *emax to the largest |x - s c|_2 of a row,
+// summed in fp64 and rounded up: the bound the single-query scans of the copy are made exact with (evs_scan.cuh:
+// scan_pool_kernel).  The codes take a second read of the row, which the first has just brought on chip.
 __global__ void __launch_bounds__(256) row_norm_max_kernel(const float* __restrict__ rows, long long n, int d, float* __restrict__ max_norm,
                                                           unsigned* __restrict__ special, __nv_bfloat16* __restrict__ dst16,
+                                                          signed char* __restrict__ dst8, float* __restrict__ scale8,
                                                           float* __restrict__ emax) {
     const int lane = threadIdx.x & 31;
     const long long warps = ((long long)gridDim.x * blockDim.x) >> 5;
     float best = 0.f;
     double ebest = 0.0;
     unsigned spec = 0u;
-    auto to16 = [&](float v, double& e2) {
+    auto to16 = [&](float v) {
         const __nv_bfloat16 h = __float2bfloat16_rn(v);
-        const float hf = __bfloat162float(h);
-        const double diff = (double)v - (double)hf;
-        e2 = fma(diff, diff, e2);
-        spec |= (isinf(hf) && !isinf(v)) ? 1u : 0u;
+        spec |= (isinf(__bfloat162float(h)) && !isinf(v)) ? 1u : 0u;
         return h;
     };
+    auto to8 = [&](float v, float sc, double& e2) {
+        const float c = sc > 0.f ? fminf(fmaxf(rintf(__fdiv_rn(v, sc)), -127.f), 127.f) : 0.f;
+        const double diff = (double)v - (double)sc * (double)c;  // s c exact in fp64
+        e2 = fma(diff, diff, e2);
+        return (int)c;
+    };
+    const bool vec = (d & 3) == 0;
     for (long long r = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < n; r += warps) {
         const float* x = rows + (size_t)r * d;
-        float s = 0.f;
+        float s = 0.f, amax = 0.f;
         double e2 = 0.0;
-        if ((d & 3) == 0) {
+        if (vec) {
             for (int i = lane; i < (d >> 2); i += 32) {
                 const float4 v = ldg_stream_f4(reinterpret_cast<const float4*>(x) + i);
                 s = fmaf(v.x, v.x, s);
                 s = fmaf(v.y, v.y, s);
                 s = fmaf(v.z, v.z, s);
                 s = fmaf(v.w, v.w, s);
+                amax = fmaxf(amax, fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w))));
                 spec |= is_special_f32(v.x) | is_special_f32(v.y) | is_special_f32(v.z) | is_special_f32(v.w);
                 if (dst16) {
                     __nv_bfloat162 o0, o1;
-                    o0.x = to16(v.x, e2);
-                    o0.y = to16(v.y, e2);
-                    o1.x = to16(v.z, e2);
-                    o1.y = to16(v.w, e2);
+                    o0.x = to16(v.x);
+                    o0.y = to16(v.y);
+                    o1.x = to16(v.z);
+                    o1.y = to16(v.w);
                     uint2 o;
                     o.x = *reinterpret_cast<uint32_t*>(&o0);
                     o.y = *reinterpret_cast<uint32_t*>(&o1);
@@ -411,14 +419,31 @@ __global__ void __launch_bounds__(256) row_norm_max_kernel(const float* __restri
         } else {
             for (int i = lane; i < d; i += 32) {
                 s = fmaf(x[i], x[i], s);
+                amax = fmaxf(amax, fabsf(x[i]));
                 spec |= is_special_f32(x[i]);
-                if (dst16) dst16[(size_t)r * d + i] = to16(x[i], e2);
+                if (dst16) dst16[(size_t)r * d + i] = to16(x[i]);
             }
         }
 #pragma unroll
         for (int off = 16; off >= 1; off >>= 1) {
             s += __shfl_xor_sync(0xffffffffu, s, off);
-            e2 += __shfl_xor_sync(0xffffffffu, e2, off);
+            amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, off));
+        }
+        if (dst8) {
+            const float sc = __fdiv_rn(amax, 127.f);  // (NaN rows: NaN scale; they mark the index special, whose searches scan fp32)
+            if (lane == 0) scale8[r] = sc;
+            if (vec) {
+                for (int i = lane; i < (d >> 2); i += 32) {
+                    const float4 v = reinterpret_cast<const float4*>(x)[i];
+                    const unsigned o = ((unsigned)to8(v.x, sc, e2) & 255u) | (((unsigned)to8(v.y, sc, e2) & 255u) << 8) |
+                                       (((unsigned)to8(v.z, sc, e2) & 255u) << 16) | (((unsigned)to8(v.w, sc, e2) & 255u) << 24);
+                    reinterpret_cast<unsigned*>(dst8 + (size_t)r * d)[i] = o;
+                }
+            } else {
+                for (int i = lane; i < d; i += 32) dst8[(size_t)r * d + i] = (signed char)to8(x[i], sc, e2);
+            }
+#pragma unroll
+            for (int off = 16; off >= 1; off >>= 1) e2 += __shfl_xor_sync(0xffffffffu, e2, off);
         }
         if (s == s) best = fmaxf(best, s);
         if (e2 > ebest) ebest = e2;  // (NaN rows mark the index special: its single-query searches scan the fp32 rows)
@@ -615,10 +640,10 @@ cudaError_t launch_merge_exchange(const Exchange& x, long long nq, int k, float*
 }
 
 cudaError_t launch_row_norm_max(const float* rows, long long n, int d, float* max_norm, unsigned* special, int sm_count, cudaStream_t st,
-                                void* dst16, float* emax) {
+                                void* dst16, signed char* dst8, float* scale8, float* emax) {
     if (n <= 0) return cudaSuccess;
     int grid = clamp_grid((n * 32 + 255) / 256, sm_count * 8);
-    row_norm_max_kernel<<<grid, 256, 0, st>>>(rows, n, d, max_norm, special, reinterpret_cast<__nv_bfloat16*>(dst16), emax);
+    row_norm_max_kernel<<<grid, 256, 0, st>>>(rows, n, d, max_norm, special, reinterpret_cast<__nv_bfloat16*>(dst16), dst8, scale8, emax);
     EVS_LAUNCH_CHECK();
     return cudaSuccess;
 }
@@ -649,21 +674,24 @@ cudaError_t launch_finalize(const FinalizeParams& p, long long nq, cudaStream_t 
     return cudaGetLastError();
 }
 
-// number of 16-byte vectors per lane per row for the vectorised kernels, 0 = use the generic kernel
-static int vectors_per_lane(int d, int is_bf16) {
-    int unit = is_bf16 ? 256 : 128;
+// number of vectors per lane per row for the vectorised kernels (16 bytes; 8 bytes of int8 codes), 0 = use the generic
+// kernel (int8: no scan)
+static int vectors_per_lane(int d, int elem) {
+    int unit = elem == SCAN_F32 ? 128 : 256;
     if (d % unit) return 0;
     int nv = d / unit;
-    if (is_bf16) return (nv >= 1 && nv <= 4) ? nv : 0;
+    if (elem != SCAN_F32) return (nv >= 1 && nv <= 4) ? nv : 0;
     return (nv == 1 || nv == 2 || nv == 3 || nv == 4 || nv == 6 || nv == 8) ? nv : 0;
 }
 
 // Decide variant, grid, block and shared memory for a scan over `n` rows (does not launch).
-cudaError_t plan_scan(long long n, int d, int is_bf16, int kp, int nq_pass, int sm_count, const ScanTuning& tune,
+cudaError_t plan_scan(long long n, int d, int elem, int kp, int nq_pass, int sm_count, const ScanTuning& tune,
                       ScanPlan* plan) {
-    const int nv = vectors_per_lane(d, is_bf16);
-    const size_t esz = is_bf16 ? 2 : 4;
+    const int nv = vectors_per_lane(d, elem);
+    const bool is_bf16 = elem != SCAN_F32;  // int8 rows: held to the occupancy of bf16 rows
+    const size_t esz = elem == SCAN_F32 ? 4 : (elem == SCAN_BF16 ? 2 : 1);
     plan->nv = nv;
+    if (nv == 0 && elem == SCAN_I8) return cudaErrorInvalidValue;
     if (nv == 0) {
         plan->variant = 0;
         plan->threads = 256;
@@ -673,7 +701,7 @@ cudaError_t plan_scan(long long n, int d, int is_bf16, int kp, int nq_pass, int 
         return cudaSuccess;
     }
     int variant = tune.scan_variant ? tune.scan_variant : 1;
-    if (variant == 2) {
+    if (variant == 2 && elem != SCAN_I8) {
         const int cw = 8;
         size_t row_bytes = (size_t)d * esz;
         int tr = tune.tile_rows > 0 ? tune.tile_rows : (int)(32768 / row_bytes);
@@ -701,7 +729,7 @@ cudaError_t plan_scan(long long n, int d, int is_bf16, int kp, int nq_pass, int 
     plan->tile_rows = plan->stages = 0;
     plan->smem_bytes = (size_t)(plan->threads / 32) * nq_pass * 2 * kp * 8;
     // measured on B200 at 10M x 512 (profiles/r01_tune_scan_*): fp32 rows peak at 2 CTAs/SM, bf16 rows
-    // (half the bytes in flight per row) need 4
+    // (half the bytes in flight per row) need 4; int8 rows (a quarter) keep 4 with twice the rows per group
     int per_sm = tune.ctas_per_sm > 0 ? tune.ctas_per_sm : (is_bf16 ? 4 : 2);
     long long groups = (n + 3) / 4;
     plan->grid = clamp_grid((groups + 7) / 8, sm_count * per_sm);
@@ -713,6 +741,7 @@ size_t scan_pool_words(const ScanPlan& plan) { return (size_t)POOL_HDR + (size_t
 
 cudaError_t launch_scan(const ScanArgs& a, ScanPlan* plan, cudaStream_t st) {
     if (a.n <= 0) return cudaErrorInvalidValue;
+    if (a.is_i8) return launch_scan_i8(a, plan, st);
     if (plan->nv == 0) return launch_scan_generic_any(a, plan, st);
     if (a.is_bf16) return plan->nv <= 2 ? launch_scan_bf16_narrow(a, plan, st) : launch_scan_bf16_wide(a, plan, st);
     if (plan->nv <= 3) return launch_scan_f32_narrow(a, plan, st);

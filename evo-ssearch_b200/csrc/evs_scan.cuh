@@ -22,7 +22,8 @@
 namespace evs {
 
 struct ScanParams {
-    const void* xb;    // database rows, row-major [n][d], fp32 or bf16
+    const void* xb;    // database rows, row-major [n][d], fp32, bf16 or int8 codes
+    const float* xs;   // int8 codes: the scale of each row [n] (row = scale * codes)
     long long n;       // rows in this shard
     int d;             // dimension
     const float* xq;   // queries fp32 [*, d] on the device
@@ -91,6 +92,85 @@ __device__ __forceinline__ void unpack(const uint4& raw, float (&x)[8]) {
 template <typename T> struct RawVec;
 template <> struct RawVec<float> { typedef float4 type; };
 template <> struct RawVec<__nv_bfloat16> { typedef uint4 type; };
+
+// ---------------------------------------------------------------------------------------------
+// int8 scan copy (scan_pool_kernel only): row x^ = s_r c_r with int8 codes c_r (8 per 8-byte vector), the query
+// q^ = s_q c_q with 16-bit codes |c_q| <= I8_QMAX split as c_q = 256 h + l into signed bytes, so that the dot product of
+// the codes is two IDP.4A chains, I = 256 sum(h c) + sum(l c), exact in int32, and the scan score is
+// s~ = fl(fl(I) * fl(s_q s_r)).
+// ---------------------------------------------------------------------------------------------
+template <> struct Elem<int8_t> { static constexpr int VEC = 8; };
+template <> struct RawVec<int8_t> { typedef uint2 type; };
+constexpr int I8_QMAX = 127 * 256 + 127;  // largest |c_q| whose high byte stays within [-127, 127]
+
+// the query code of one element: every CTA and the bound below derive the same codes from the same fp32 values
+__device__ __forceinline__ int i8_query_code(float v, float sq) {
+    if (!(sq > 0.f)) return 0;  // zero (or underflowing) query: q^ = 0, the bound then holds |q| max|x| in full
+    const float c = rintf(__fdiv_rn(v, sq));
+    return (int)fminf(fmaxf(c, (float)-I8_QMAX), (float)I8_QMAX);
+}
+// s_q = max|q_i| / I8_QMAX (fp32); warp-uniform
+__device__ __forceinline__ float i8_query_scale(const float* __restrict__ q, int d, int lane) {
+    float m = 0.f;
+    for (int i = lane; i < d; i += 32) m = fmaxf(m, fabsf(q[i]));
+#pragma unroll
+    for (int off = 16; off >= 1; off >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, off));
+    return __fdiv_rn(m, (float)I8_QMAX);
+}
+template <int NQ, int NV>
+struct QueryRegs<int8_t, NQ, NV> {
+    static_assert(NQ == 1, "the int8 copy is scanned for single queries only");
+    int h[NV][2], l[NV][2];  // packed signed bytes of the query codes that pair with the lane's 8-byte row vector j
+    float sq;
+    __device__ __forceinline__ void load(const float* __restrict__ xq, int q0, int d, int lane) {
+        const float* q = xq + (size_t)q0 * d;
+        sq = i8_query_scale(q, d, lane);
+#pragma unroll
+        for (int j = 0; j < NV; j++)
+#pragma unroll
+            for (int w = 0; w < 2; w++) {
+                unsigned hw = 0u, lw = 0u;
+#pragma unroll
+                for (int b = 0; b < 4; b++) {
+                    const int c = i8_query_code(q[8 * (lane + 32 * j) + 4 * w + b], sq);
+                    const int lo = ((c + 128) & 255) - 128;
+                    const int hi = (c - lo) >> 8;
+                    hw |= ((unsigned)hi & 255u) << (8 * b);
+                    lw |= ((unsigned)lo & 255u) << (8 * b);
+                }
+                h[j][w] = (int)hw;
+                l[j][w] = (int)lw;
+            }
+    }
+};
+// scan score of one int8 row with scale sr.  |I| <= d * I8_QMAX * 127 < 2^31 for d <= 512 (NV <= 2): the lane sums are
+// combined in int32 and butterflied; wider rows butterfly both chains (each < 2^31) and combine in fp64, exactly.
+template <int NV>
+__device__ __forceinline__ float row_score_i8(const uint2 (&raw)[NV], const QueryRegs<int8_t, 1, NV>& q, float sr) {
+    int ih = 0, il = 0;
+#pragma unroll
+    for (int j = 0; j < NV; j++) {
+        ih = __dp4a((int)raw[j].x, q.h[j][0], ih);
+        ih = __dp4a((int)raw[j].y, q.h[j][1], ih);
+        il = __dp4a((int)raw[j].x, q.l[j][0], il);
+        il = __dp4a((int)raw[j].y, q.l[j][1], il);
+    }
+    float fi;
+    if constexpr (NV <= 2) {
+        int I = ih * 256 + il;
+#pragma unroll
+        for (int off = 16; off >= 1; off >>= 1) I += __shfl_xor_sync(0xffffffffu, I, off);
+        fi = __int2float_rn(I);
+    } else {
+#pragma unroll
+        for (int off = 16; off >= 1; off >>= 1) {
+            ih += __shfl_xor_sync(0xffffffffu, ih, off);
+            il += __shfl_xor_sync(0xffffffffu, il, off);
+        }
+        fi = __double2float_rn(fma((double)ih, 256.0, (double)il));
+    }
+    return __fmul_rn(fi, __fmul_rn(q.sq, sr));
+}
 
 // Scan score of one row against NQ queries.  Fixed order: four partial sums per lane (vector
 // component mod 4) over j, combined as (p0+p1)+(p2+p3), then the xor butterfly 16,8,4,2,1.
@@ -204,8 +284,8 @@ __device__ __forceinline__ void cta_merge_and_store(u64* sel_base, int nwarps_se
 //   * nactive != null: guard re-run of the queries queued by the first finalise (evs_finalize.cuh), NQ at a time.
 // ---------------------------------------------------------------------------------------------
 template <typename T, int NQ, int NV>
-struct ScanOcc {  // CTAs per SM the register allocation is held to (the measured optimum: 2 for fp32 rows, 4 for bf16 rows)
-    static constexpr int value = NQ == 1 ? ((sizeof(T) == 2 && NV <= 2) ? 4 : 2) : 1;
+struct ScanOcc {  // CTAs per SM the register allocation is held to (the measured optimum: 2 for fp32 rows, 4 for bf16 and int8 rows)
+    static constexpr int value = NQ == 1 ? ((sizeof(T) == 1 || (sizeof(T) == 2 && NV <= 2)) ? 4 : 2) : 1;
 };
 
 __device__ __forceinline__ unsigned long long globaltimer_ns() {
@@ -382,18 +462,25 @@ __host__ __device__ inline size_t small_query_smem_offset(int kp, int d, int wor
 }
 
 // ---------------------------------------------------------------------------------------------
-// Exact single-query search from the bf16 rows (f.shadow_emax != null; DESIGN.md section 2).  For a row x with
-// x^ = bf16_rn(x) and s~ the fp32 scan score of x^:  |q.x - s~| <= |q| |x - x^| + gamma |q| |x^| <= E.
+// Exact single-query search from the int8 copy (T = int8_t, f.shadow_emax != null; DESIGN.md section 2).  Row x, its copy
+// x^ = s_r c_r, e_max >= max_r |x - x^| (fp64, rounded up at add time); query q, q^ = s_q c_q; N >= max_r |x|.  The codes'
+// dot product I is exact, so with P = fl(s_q s_r) and s~ = fl(fl(I) P) -- three roundings of relative 2^-24 each, plus an
+// absolute 2^-150 per product should one underflow, times |fl(I)| <= 2^31 for the first --
+//   |q.x - q^.x^| <= |q - q^| |x| + |q^| |x - x^| <= |q - q^| N + |q^| e_max
+//   |q^.x^ - s~|  <= ((1 + 2^-24)^3 - 1) |q^| |x^| + 2^-118 <= 2^-22 |q^| (N + e_max) + 2^-118
+// E = the sum of both, with |q - q^| and |q^| summed in fp64 (inflated by 2^-20 for their roundings), N = the fp32 norm
+// estimate max_norm inflated by 2^-7 (a d-term fp32 sum of squares is within d 2^-24 of the truth), rounded up.
 //   rule 1: a key is dropped only below key_floor(score(t) - 2E), t the score of a key 64 rows are known to reach (a warp's
 //           own 64th best, tau_g): the dropped row's true score is < t - E <= that of each of those 64 rows;
 //   rule 2: the last CTA re-scores every survivor with s~ >= s~_(k) - 2E exactly (C): any row outside C has a true score
 //           < s~_(k) - E, below each of the k best-by-scan rows, so the top k of C is the exact answer.
-// With shadow_emax == null the lowered threshold IS the threshold (twoE = 0): the fp32 scan as before.
+// With shadow_emax == null the lowered threshold IS the threshold (twoE = 0): the fp32 / bf16 scans as before.
 // ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ float shadow_bound(const FinalizeParams& f, double qn2) {
-    const double qn = sqrt(qn2) * (1.0 + 0x1p-20);
-    const double nh = (double)__ldg(f.max_norm) * (1.0 + 0x1p-7);  // |x^_i| <= |x_i| (1 + 2^-8); max_norm is an fp32 estimate
-    const double e = qn * ((double)__ldg(f.shadow_emax) + (double)f.shadow_gamma * nh) * (1.0 + 0x1p-20) + f.d * 0x1p-149;
+__device__ __forceinline__ float shadow_bound_i8(const FinalizeParams& f, double dq2, double qh2) {
+    const double dq = sqrt(dq2) * (1.0 + 0x1p-20), qh = sqrt(qh2) * (1.0 + 0x1p-20);  // |q - q^|, |q^|
+    const double nx = (double)__ldg(f.max_norm) * (1.0 + 0x1p-7);
+    const double em = (double)__ldg(f.shadow_emax);
+    const double e = (dq * nx + qh * em + 0x1p-22 * qh * (nx + em)) * (1.0 + 0x1p-20) + 0x1p-117;
     return __double2float_ru(e);  // inf when it does not fit: every key is kept below
 }
 // the smallest key of score score(t) - 2E (rounded down); 1 (every key) without a finite bound
@@ -404,18 +491,26 @@ __device__ __forceinline__ u64 key_lowered(u64 t, float twoE) {
     return o == 0u ? 1ull : ((u64)o << 32);
 }
 
-// C has more than POOL_KPMAX keys (near-tie bursts): walk the pool in blocks of 128 keys and, whenever the next block may not
-// fit, re-score what was gathered and keep its exact top k (as scan keys: a row re-scores to the same canonical score) in
-// front of the buffer.  Returns the number of candidates left in cand[] for the final ranking.  Called by all threads.
+// C has more than POOL_KPMAX keys (the int8 copy's window at 10M rows: every search; near-tie bursts): walk the pool in
+// blocks of 128 keys and, whenever the next block may not fit, re-score what was gathered and keep its exact top k (as scan
+// keys: a row re-scores to the same canonical score) in front of the buffer.  The next block's keys are in flight while a
+// block is filtered, and a member's fp32 row is sent to L2 as soon as it joins, so that the re-score rounds wait on L2, not
+// on HBM.  Returns the number of candidates left in cand[] for the final ranking.  Called by all threads.
 __device__ __forceinline__ int pool_wide_rounds(const FinalizeParams& f, const u64* S, unsigned m, u64 cut, u64* cand, u64* keep,
                                              double* sc, long long* id, u64* ok, const double* qs, int* s_n) {
     const int t = threadIdx.x, nt = blockDim.x, warp = t >> 5, lane = t & 31, nwarps = nt >> 5;
     const float* xb32 = reinterpret_cast<const float*>(f.xb);
     const bool fastw = f.special != nullptr && __ldg(f.special) == 0u;
+    const int lines = (f.d * 4 + 127) / 128;
     int fill = 0;  // CTA-uniform
+    u64 key = (t < 128 && t < m) ? __ldcg(S + t) : 0ull;
     for (unsigned b0 = 0; b0 < m; b0 += 128) {
-        const u64 key = (t < 128 && b0 + t < m) ? __ldcg(S + b0 + t) : 0ull;
+        const u64 nkey = (t < 128 && b0 + 128 + t < m) ? __ldcg(S + b0 + 128 + t) : 0ull;
         const bool mem = key != 0ull && key >= cut;
+        if (mem) {
+            const char* row = reinterpret_cast<const char*>(f.xb) + (size_t)key_row(key) * f.d * 4;
+            for (int i = 0; i < lines; i++) asm volatile("prefetch.global.L2 [%0];" ::"l"(row + (size_t)i * 128));
+        }
         const int nb = __syncthreads_count(mem);
         if (fill + nb > POOL_KPMAX) {
             for (int c = 2 * warp; c < fill; c += 2 * nwarps) {
@@ -452,6 +547,7 @@ __device__ __forceinline__ int pool_wide_rounds(const FinalizeParams& f, const u
         __syncthreads();
         if (mem) cand[atomicAdd(s_n, 1)] = key;
         fill += nb;
+        key = nkey;
         __syncthreads();
     }
     return fill;
@@ -488,9 +584,12 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
     __shared__ u64 s_tau, s_wtau[8];  // s_wtau: each warp's running threshold (read only when it compacts: registers stay for the loop)
     __shared__ float s_twoE;
     typedef typename RawVec<T>::type raw_t;
+    constexpr bool I8 = sizeof(T) == 1;
     constexpr int QREGS = NV * Elem<T>::VEC;
     constexpr int RPG_RAW = (100 - QREGS) / (NV * 4);
-    constexpr int RPG = RPG_RAW < 1 ? 1 : (RPG_RAW > 4 ? 4 : RPG_RAW);
+    // int8 rows: 8 bytes per lane and vector; 16 / NV rows per group (8 at d = 512) keep as many bytes in flight per warp as
+    // 4 bf16 rows
+    constexpr int RPG = I8 ? (NV >= 4 ? 4 : 16 / NV) : (RPG_RAW < 1 ? 1 : (RPG_RAW > 4 ? 4 : RPG_RAW));
     constexpr int KP = 64, CAPW = 128;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int nwarps = blockDim.x >> 5;
@@ -526,18 +625,29 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
         const float* qf = p.xq + (size_t)p.q0 * p.d;
         for (int i = threadIdx.x; i < p.d; i += blockDim.x) qs[i] = (double)qf[i];
     }
-    // bf16 rows under the rounding bound: thresholds are lowered by 2E (rules 1 and 2 above); every warp derives the same E
-    // (each warp stores the same bits to s_twoE; nothing reads it before the barrier ahead of the last CTA's work)
-    if (f.shadow_emax != nullptr) {
-        __syncthreads();  // qs complete
-        double s2 = 0.0;
-        for (int i = lane; i < p.d; i += 32) s2 = fma(qs[i], qs[i], s2);
+    // int8 rows under the bound: thresholds are lowered by 2E (rules 1 and 2 above); every warp derives the same E from the
+    // same query codes (each warp stores the same bits to s_twoE; nothing reads it before the barrier ahead of the last
+    // CTA's work)
+    bool bounded = false;  // CTA-uniform
+    if constexpr (I8) {
+        if (f.shadow_emax != nullptr) {
+            bounded = true;
+            __syncthreads();  // qs complete
+            double dq2 = 0.0, qh2 = 0.0;
+            for (int i = lane; i < p.d; i += 32) {
+                const double qh = (double)q.sq * (double)i8_query_code((float)qs[i], q.sq);  // exact: 24 x 16 bits
+                dq2 = fma(qs[i] - qh, qs[i] - qh, dq2);
+                qh2 = fma(qh, qh, qh2);
+            }
 #pragma unroll
-        for (int off = 16; off >= 1; off >>= 1) s2 += __shfl_xor_sync(0xffffffffu, s2, off);
-        if (lane == 0) s_twoE = 2.f * shadow_bound(f, s2);
-    } else if (threadIdx.x == 0) {
-        s_twoE = 0.f;
+            for (int off = 16; off >= 1; off >>= 1) {
+                dq2 += __shfl_xor_sync(0xffffffffu, dq2, off);
+                qh2 += __shfl_xor_sync(0xffffffffu, qh2, off);
+            }
+            if (lane == 0) s_twoE = 2.f * shadow_bound_i8(f, dq2, qh2);
+        }
     }
+    if (!bounded && threadIdx.x == 0) s_twoE = 0.f;
     u64 tcut = 0ull;  // = key_lowered(own threshold, 2E): what a key must beat to enter the buffer
 
     // buffer full: sort, keep the best 64, publish the best 8 where they raise their slot (a warp sees ~n / warps rows: whatever it holds of the shard's
@@ -574,6 +684,10 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
     auto do_group = [&](long long g) {
         const long long r0 = g * RPG;
         raw_t raw[RPG][NV];
+        float sr = 0.f;  // int8 rows: lane r < RPG holds the scale of row r0 + r
+        if constexpr (I8) {
+            if (lane < RPG) sr = __ldg(p.xs + (r0 + lane < p.n ? r0 + lane : p.n - 1));
+        }
 #pragma unroll
         for (int r = 0; r < RPG; r++) {
             long long row = r0 + r < p.n ? r0 + r : p.n - 1;  // clamp: tail rows are re-read, not offered
@@ -581,13 +695,15 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
 #pragma unroll
             for (int j = 0; j < NV; j++) {
                 if constexpr (sizeof(T) == 4) raw[r][j] = ldg_stream_f4(src + 32 * j);
+                else if constexpr (I8) raw[r][j] = ldg_stream_u2(src + 32 * j);
                 else raw[r][j] = ldg_stream_u4(src + 32 * j);
             }
         }
 #pragma unroll
         for (int r = 0; r < RPG; r++) {
             float s[1];
-            row_scores<T, 1, NV>(raw[r], q, s);
+            if constexpr (I8) s[0] = row_score_i8<NV>(raw[r], q, __shfl_sync(0xffffffffu, sr, r));
+            else row_scores<T, 1, NV>(raw[r], q, s);
             if (r0 + r < p.n) {
                 const u64 key = make_key(s[0], (uint32_t)(r0 + r));  // warp-uniform
                 if (key > tcut) {

@@ -29,10 +29,10 @@ static cudaError_t ensure_smem_optin(K kern, size_t smem, size_t (&table)[16]) {
     return e;
 }
 
-template <typename T, int NQ, int NV>
-static cudaError_t launch_scan_t(const ScanArgs& a, ScanPlan* plan, cudaStream_t st) {
+static ScanParams scan_params(const ScanArgs& a, const ScanPlan* plan) {
     ScanParams p;
     p.xb = a.xb;
+    p.xs = a.xs;
     p.n = a.n;
     p.d = a.d;
     p.xq = a.xq;
@@ -49,6 +49,20 @@ static cudaError_t launch_scan_t(const ScanArgs& a, ScanPlan* plan, cudaStream_t
     p.nactive = a.nactive;
     p.qcap = a.qcap;
     p.cta_clock = nullptr;
+    return p;
+}
+
+// dynamic shared memory of the pool kernel: the warps' buffers or the finalise area, whichever is larger (the pool kernel
+// re-scores up to POOL_KPMAX candidates at a time)
+static size_t pool_smem_bytes(const ScanPlan* plan, const FinalizeParams& f) {
+    const size_t fs = pool_finalize_smem_bytes(64, f.d, f.x.world * f.k) + 3 * (size_t)(POOL_KPMAX - 64) * 8;
+    const size_t bufs = (size_t)(plan->threads / 32) * 128 * 8;
+    return fs > bufs ? fs : bufs;
+}
+
+template <typename T, int NQ, int NV>
+static cudaError_t launch_scan_t(const ScanArgs& a, ScanPlan* plan, cudaStream_t st) {
+    ScanParams p = scan_params(a, plan);
     if (plan->variant == 2) {
         if (a.fuse || a.nactive) return cudaErrorInvalidValue;  // the ring variant neither fuses nor re-runs
         auto kern = scan_ring_kernel<T, NQ, NV>;
@@ -68,8 +82,7 @@ static cudaError_t launch_scan_t(const ScanArgs& a, ScanPlan* plan, cudaStream_t
                 p.chunk_groups = a.chunk_groups;
             }
             const size_t fs = pool_finalize_smem_bytes(64, f.d, f.x.world * f.k);
-            smem = (size_t)(plan->threads / 32) * 128 * 8;
-            if (fs + 3 * (size_t)(POOL_KPMAX - 64) * 8 > smem) smem = fs + 3 * (size_t)(POOL_KPMAX - 64) * 8;  // the pool kernel re-scores up to POOL_KPMAX
+            smem = pool_smem_bytes(plan, f);
             if (a.small_fast_cap > 0) {  // small shard: keys by row, threshold from the chunk maxima (no buffers: only the finalise area)
                 const int cap = a.small_fast_cap < POOL_SURV ? a.small_fast_cap : POOL_SURV;
                 cudaError_t se;
@@ -140,23 +153,7 @@ static cudaError_t launch_scan_nq(const ScanArgs& a, ScanPlan* plan, cudaStream_
 
 template <typename T>
 static cudaError_t launch_scan_generic(const ScanArgs& a, ScanPlan* plan, cudaStream_t st) {
-    ScanParams p;
-    p.xb = a.xb;
-    p.n = a.n;
-    p.d = a.d;
-    p.xq = a.xq;
-    p.lists = reinterpret_cast<u64*>(a.lists);
-    p.kp = a.kp;
-    p.tile_rows = 0;
-    p.stages = 0;
-    p.lists_stride_q = plan->grid * a.kp;
-    p.ticket = nullptr;
-    p.next_chunk = nullptr;
-    p.chunk_groups = 1;
-    p.qmap = nullptr;
-    p.nactive = nullptr;
-    p.qcap = 0;
-    p.cta_clock = nullptr;
+    ScanParams p = scan_params(a, plan);
     if (a.fuse || a.nactive) return cudaErrorInvalidValue;
     for (int qi = 0; qi < a.nq_pass; qi++) {
         p.q0 = a.q0 + qi;
@@ -173,6 +170,7 @@ cudaError_t launch_scan_f32_512(const ScanArgs& a, ScanPlan* plan, cudaStream_t 
 cudaError_t launch_scan_f32_wide(const ScanArgs& a, ScanPlan* plan, cudaStream_t st);    // nv = 6, 8
 cudaError_t launch_scan_bf16_narrow(const ScanArgs& a, ScanPlan* plan, cudaStream_t st); // nv = 1, 2
 cudaError_t launch_scan_bf16_wide(const ScanArgs& a, ScanPlan* plan, cudaStream_t st);   // nv = 3, 4
+cudaError_t launch_scan_i8(const ScanArgs& a, ScanPlan* plan, cudaStream_t st);          // nv = 1 .. 4, pool kernel only
 cudaError_t launch_scan_generic_any(const ScanArgs& a, ScanPlan* plan, cudaStream_t st); // any d
 
 }  // namespace evs

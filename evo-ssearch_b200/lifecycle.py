@@ -45,9 +45,12 @@ load_stats = {"loads": 0, "bytes": 0, "seconds": 0.0, "evictions": 0}  # what th
 
 def _index_bytes(index) -> int:
     local = getattr(index, "local", index)  # a sharded index holds only its block on this GPU
-    # fp32 rows, plus the bf16 copy of bf16 storage or of an fp32 index built with the option "scan_shadow" on
-    copy = getattr(index, "storage", "f32") == "bf16" or (hasattr(local, "shadow_stats") and local.shadow_stats()[1] >= 0)
-    return int(local.ntotal) * index.d * (6 if copy else 4)
+    # fp32 rows; the bf16 rows of bf16 storage; the int8 scan copy (one byte per element, one fp32 scale per row) that
+    # bf16 storage always keeps and an fp32 index built with the option "scan_shadow" on keeps
+    bf16 = getattr(index, "storage", "f32") == "bf16"
+    copy = bf16 or (hasattr(local, "shadow_stats") and local.shadow_stats()[1] >= 0)
+    n, d = int(local.ntotal), index.d
+    return n * d * (4 + (2 if bf16 else 0) + (1 if copy else 0)) + (4 * n if copy else 0)
 
 
 def _signature(index_path: Path):

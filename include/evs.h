@@ -259,12 +259,12 @@ EVS_API int evs_f32_to_bf16_dev(int device, const float* src_dev, void* dst_dev,
  *                 "small_max_rows" (default 32768; 0 = never): single-query searches (k <= 48) of shards up to this many rows take
  *                 the small-shard kernel (keys stored by row, threshold from 128 chunk maxima: 10k x 512 in 16 us instead of 27);
  *                 "small_fast_cap" (default 2048, tests lower it): its register fast path up to this many keys above the threshold;
- *                 "scan_shadow" (default 1): an fp32 index added to while it is on keeps a bf16 copy of its rows (+50 % device
- *                 memory; added to while it is off, it drops the copy).  Single-query searches (k <= 48) of shards above
- *                 small_max_rows and of at least "shadow_min_rows" rows (default 131072) scan that copy -- half the bytes --
- *                 under a proven bound on its rounding, so their results
- *                 are those of the fp32 scan (DESIGN.md section 2); bf16-storage indexes search the same way.  Indexes with
- *                 subnormal, infinite or NaN elements scan their fp32 rows;
+ *                 "scan_shadow" (default 1): an fp32 index added to while it is on keeps an int8 copy of its rows (one byte
+ *                 per element and one fp32 scale per row: +25 % device memory; added to while it is off, it drops the copy;
+ *                 bf16-storage indexes always keep it).  Single-query searches (k <= 48, d a multiple of 256 up to 1024) of
+ *                 shards above small_max_rows and of at least "shadow_min_rows" rows (default 262144) scan that copy -- a
+ *                 quarter of the fp32 bytes -- under a proven bound on its rounding, so their results are those of the fp32
+ *                 scan (DESIGN.md section 2).  Indexes with subnormal, infinite or NaN elements scan their own rows;
  *                 "io_threads" (default 0 = auto: one per hardware thread, at most 16): threads that pread each 64 MiB chunk of
  *                 index.faiss into the pinned staging buffers (evs_index_read[_rows]; 6.5 GB/s with 1, 35 GB/s with 16);
  *                 "exchange_fail_next" (tests): the next exchange-mode search of this process fails after taking its

@@ -1,8 +1,8 @@
-"""Single-query search of an fp32 index from its bf16 scan copy (option "scan_shadow") against the fp32 scan, one JSON line
+"""Single-query search of an fp32 index from its int8 scan copy (option "scan_shadow") against the fp32 scan, one JSON line
 per (rows, arm): time per search (CUDA events around `--iters` back-to-back searches of different queries), the bytes the
-search reads (bf16 rows plus the fp32 rows of the candidates it re-scored exactly) and their rate against 7.7 TB/s, the
-bound E of the first query, the distribution of the candidate count |C| over `--queries` queries and the searches that
-needed more than one re-score round.
+search reads (int8 codes and row scales plus the fp32 rows of the candidates it re-scored exactly) and their rate against
+7.7 TB/s, the bound E of the first query, the distribution of the candidate count |C| over `--queries` queries and the
+searches that needed more than one re-score round.
 
     python scripts/shadow_probe.py --rows 10000000 1250000 --out shadow_probe.jsonl
 """
@@ -55,10 +55,14 @@ def probe(n, d, k, shadow, queries, iters, seed=5):
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / iters
     wide, emax, _ = idx.shadow_stats()
-    qn = float(np.linalg.norm(q[0].astype(np.float64)))
-    E = qn * (emax + (d // 32 + 8) * 2.0**-24 * idx.max_row_norm * (1 + 2.0**-7))
+    # E of the first query (evs_scan.cuh: shadow_bound_i8)
+    q0 = q[0]
+    sq = np.float32(np.abs(q0).max() / np.float32(32639))
+    qh = float(sq) * np.clip(np.rint((q0 / sq).astype(np.float32)), -32639, 32639).astype(np.float64)
+    dq, qhn, nx = np.linalg.norm(q0.astype(np.float64) - qh), np.linalg.norm(qh), idx.max_row_norm * (1 + 2.0**-7)
+    E = dq * nx + qhn * emax + 2.0**-22 * qhn * (nx + emax)
     mean_c = float(np.mean(cands)) if shadow else 0.0
-    nbytes = n * d * (2 if shadow else 4) + mean_c * d * 4
+    nbytes = (n * d + n * 4 if shadow else n * d * 4) + mean_c * d * 4
     out = {"rows": n, "d": d, "k": k, "scan_shadow": shadow, "ms_per_search": ms, "bytes_per_search": nbytes,
            "tb_s": nbytes / ms / 1e9, "frac_hbm_peak": nbytes / (ms * 1e-3) / HBM_PEAK, "emax": emax,
            "E_first_query": E if shadow else None, "wide_searches": wide, "queries": queries}
