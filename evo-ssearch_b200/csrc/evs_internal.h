@@ -18,7 +18,7 @@ struct ScanTuning {
     int scan_variant = 0;  // 0 auto, 1 direct loads, 2 bulk-async ring
     int tile_rows = 0;     // ring: rows per stage (0 = ~32 KiB)
     int stages = 0;        // ring: depth (0 = 4)
-    int ctas_per_sm = 0;   // direct: CTAs per SM (0 = 2 fp32 / 4 bf16)
+    int ctas_per_sm = 0;   // direct: CTAs per SM (0 = 2 fp32 and int8 / 4 bf16)
     int tc_min_nq = 2;     // query batches of at least this many use the tensor-core scan (0 = never); measured
                            // (scripts/small_nq_sweep.py): from 2 queries on it beats the CUDA-core GEMV for fp32 and bf16 rows
     int tc_pair_min_nq = 129;  // ... and of at least this many the CTA-pair kernel (evs_tc2.cu); 0 = never

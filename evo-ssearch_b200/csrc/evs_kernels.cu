@@ -688,7 +688,6 @@ static int vectors_per_lane(int d, int elem) {
 cudaError_t plan_scan(long long n, int d, int elem, int kp, int nq_pass, int sm_count, const ScanTuning& tune,
                       ScanPlan* plan) {
     const int nv = vectors_per_lane(d, elem);
-    const bool is_bf16 = elem != SCAN_F32;  // int8 rows: held to the occupancy of bf16 rows
     const size_t esz = elem == SCAN_F32 ? 4 : (elem == SCAN_BF16 ? 2 : 1);
     plan->nv = nv;
     if (nv == 0 && elem == SCAN_I8) return cudaErrorInvalidValue;
@@ -729,8 +728,9 @@ cudaError_t plan_scan(long long n, int d, int elem, int kp, int nq_pass, int sm_
     plan->tile_rows = plan->stages = 0;
     plan->smem_bytes = (size_t)(plan->threads / 32) * nq_pass * 2 * kp * 8;
     // measured on B200 at 10M x 512 (profiles/r01_tune_scan_*): fp32 rows peak at 2 CTAs/SM, bf16 rows
-    // (half the bytes in flight per row) need 4; int8 rows (a quarter) keep 4 with twice the rows per group
-    int per_sm = tune.ctas_per_sm > 0 ? tune.ctas_per_sm : (is_bf16 ? 4 : 2);
+    // (half the bytes in flight per row) need 4; int8 rows hold two groups in registers (ScanOcc) and peak at 2
+    // (profiles/int8_group_occupancy_sweep.jsonl)
+    int per_sm = tune.ctas_per_sm > 0 ? tune.ctas_per_sm : (elem == SCAN_BF16 ? 4 : 2);
     long long groups = (n + 3) / 4;
     plan->grid = clamp_grid((groups + 7) / 8, sm_count * per_sm);
     return cudaSuccess;

@@ -94,14 +94,62 @@ template <> struct RawVec<float> { typedef float4 type; };
 template <> struct RawVec<__nv_bfloat16> { typedef uint4 type; };
 
 // ---------------------------------------------------------------------------------------------
-// int8 scan copy (scan_pool_kernel only): row x^ = s_r c_r with int8 codes c_r (8 per 8-byte vector), the query
-// q^ = s_q c_q with 16-bit codes |c_q| <= I8_QMAX split as c_q = 256 h + l into signed bytes, so that the dot product of
-// the codes is two IDP.4A chains, I = 256 sum(h c) + sum(l c), exact in int32, and the scan score is
-// s~ = fl(fl(I) * fl(s_q s_r)).
+// int8 scan copy (scan_pool_kernel only): row x^ = s_r c_r with int8 codes c_r, the query q^ = s_q c_q with 16-bit codes
+// |c_q| <= I8_QMAX split as c_q = 256 h + l into signed bytes, so that the dot product of the codes is two IDP.4A chains,
+// I = 256 sum(h c) + sum(l c), exact in int32, and the scan score is s~ = fl(fl(I) * fl(s_q s_r)).
+// NV = d / 256 counts 8 bytes of a row per lane.  Lane l reads NV / 2 16-byte vectors, at bytes [16 (l + 32 j), +16),
+// and for odd NV (d = 256, 768) one 8-byte vector at [512 (NV / 2) + 8 l, +8): at d = 512 one LDG.128 reads a whole row.
+// Word w (4 codes) of a lane's row data pairs with word w of its packed query bytes.
 // ---------------------------------------------------------------------------------------------
 template <> struct Elem<int8_t> { static constexpr int VEC = 8; };
-template <> struct RawVec<int8_t> { typedef uint2 type; };
 constexpr int I8_QMAX = 127 * 256 + 127;  // largest |c_q| whose high byte stays within [-127, 127]
+
+template <int NV>
+struct I8Lane {
+    static constexpr int V16 = NV / 2, WORDS = 2 * NV;
+    // rows per group: 128 bytes per lane, so that two groups in registers (one scored, one in flight) stay near 64
+    // registers; a power of two for the halving reduction (i8_warp_sum)
+    static constexpr int ROWS = NV == 1 ? 16 : (NV == 2 ? 8 : 4);
+    static constexpr int RSH = ROWS == 16 ? 1 : (ROWS == 8 ? 2 : 3);  // 32 / ROWS = 1 << RSH lanes end with each row's sum
+    // the column of byte 0 of word w
+    __device__ __forceinline__ static int col(int w, int lane) {
+        return w < 4 * V16 ? 16 * (lane + 32 * (w >> 2)) + 4 * (w & 3) : 512 * V16 + 8 * lane + 4 * (w - 4 * V16);
+    }
+    __device__ __forceinline__ static void load(const int8_t* __restrict__ row, int lane, unsigned (&w)[WORDS]) {
+#pragma unroll
+        for (int j = 0; j < V16; j++) {
+            const uint4 v = ldg_stream_u4(reinterpret_cast<const uint4*>(row) + lane + 32 * j);
+            w[4 * j + 0] = v.x; w[4 * j + 1] = v.y; w[4 * j + 2] = v.z; w[4 * j + 3] = v.w;
+        }
+        if constexpr (NV & 1) {
+            const uint2 v = ldg_stream_u2(reinterpret_cast<const uint2*>(row + 512 * V16) + lane);
+            w[4 * V16] = v.x; w[4 * V16 + 1] = v.y;
+        }
+    }
+};
+
+// Sums M per-lane values (M a power of two <= 32) over the warp with a halving exchange: at xor step `off` a lane keeps
+// the half of its values that the lane bit `off` selects and sends the other half; once one value is left the steps are a
+// plain butterfly.  M = 8: 4 + 2 + 1 + 1 + 1 shuffles.  Lane l ends with the sum of value l >> (5 - log2 M) in v[0].
+// Integer sums: exact in any order.
+template <int M>
+__device__ __forceinline__ void i8_warp_sum(int (&v)[M], int lane) {
+#pragma unroll
+    for (int s = 0; s < 5; s++) {
+        const int off = 16 >> s, m = M >> s;  // values left
+        if (m > 1) {
+            const bool up = lane & off;
+#pragma unroll
+            for (int i = 0; i < m / 2; i++) {
+                const int send = up ? v[i] : v[i + m / 2];
+                const int keep = up ? v[i + m / 2] : v[i];
+                v[i] = keep + __shfl_xor_sync(0xffffffffu, send, off);
+            }
+        } else {
+            v[0] += __shfl_xor_sync(0xffffffffu, v[0], off);
+        }
+    }
+}
 
 // the query code of one element: every CTA and the bound below derive the same codes from the same fp32 values
 __device__ __forceinline__ int i8_query_code(float v, float sq) {
@@ -120,57 +168,27 @@ __device__ __forceinline__ float i8_query_scale(const float* __restrict__ q, int
 template <int NQ, int NV>
 struct QueryRegs<int8_t, NQ, NV> {
     static_assert(NQ == 1, "the int8 copy is scanned for single queries only");
-    int h[NV][2], l[NV][2];  // packed signed bytes of the query codes that pair with the lane's 8-byte row vector j
+    int h[2 * NV], l[2 * NV];  // packed signed bytes of the query codes that pair with word w of the lane's row data
     float sq;
     __device__ __forceinline__ void load(const float* __restrict__ xq, int q0, int d, int lane) {
         const float* q = xq + (size_t)q0 * d;
         sq = i8_query_scale(q, d, lane);
 #pragma unroll
-        for (int j = 0; j < NV; j++)
+        for (int w = 0; w < 2 * NV; w++) {
+            unsigned hw = 0u, lw = 0u;
 #pragma unroll
-            for (int w = 0; w < 2; w++) {
-                unsigned hw = 0u, lw = 0u;
-#pragma unroll
-                for (int b = 0; b < 4; b++) {
-                    const int c = i8_query_code(q[8 * (lane + 32 * j) + 4 * w + b], sq);
-                    const int lo = ((c + 128) & 255) - 128;
-                    const int hi = (c - lo) >> 8;
-                    hw |= ((unsigned)hi & 255u) << (8 * b);
-                    lw |= ((unsigned)lo & 255u) << (8 * b);
-                }
-                h[j][w] = (int)hw;
-                l[j][w] = (int)lw;
+            for (int b = 0; b < 4; b++) {
+                const int c = i8_query_code(q[I8Lane<NV>::col(w, lane) + b], sq);
+                const int lo = ((c + 128) & 255) - 128;
+                const int hi = (c - lo) >> 8;
+                hw |= ((unsigned)hi & 255u) << (8 * b);
+                lw |= ((unsigned)lo & 255u) << (8 * b);
             }
+            h[w] = (int)hw;
+            l[w] = (int)lw;
+        }
     }
 };
-// scan score of one int8 row with scale sr.  |I| <= d * I8_QMAX * 127 < 2^31 for d <= 512 (NV <= 2): the lane sums are
-// combined in int32 and butterflied; wider rows butterfly both chains (each < 2^31) and combine in fp64, exactly.
-template <int NV>
-__device__ __forceinline__ float row_score_i8(const uint2 (&raw)[NV], const QueryRegs<int8_t, 1, NV>& q, float sr) {
-    int ih = 0, il = 0;
-#pragma unroll
-    for (int j = 0; j < NV; j++) {
-        ih = __dp4a((int)raw[j].x, q.h[j][0], ih);
-        ih = __dp4a((int)raw[j].y, q.h[j][1], ih);
-        il = __dp4a((int)raw[j].x, q.l[j][0], il);
-        il = __dp4a((int)raw[j].y, q.l[j][1], il);
-    }
-    float fi;
-    if constexpr (NV <= 2) {
-        int I = ih * 256 + il;
-#pragma unroll
-        for (int off = 16; off >= 1; off >>= 1) I += __shfl_xor_sync(0xffffffffu, I, off);
-        fi = __int2float_rn(I);
-    } else {
-#pragma unroll
-        for (int off = 16; off >= 1; off >>= 1) {
-            ih += __shfl_xor_sync(0xffffffffu, ih, off);
-            il += __shfl_xor_sync(0xffffffffu, il, off);
-        }
-        fi = __double2float_rn(fma((double)ih, 256.0, (double)il));
-    }
-    return __fmul_rn(fi, __fmul_rn(q.sq, sr));
-}
 
 // Scan score of one row against NQ queries.  Fixed order: four partial sums per lane (vector
 // component mod 4) over j, combined as (p0+p1)+(p2+p3), then the xor butterfly 16,8,4,2,1.
@@ -284,8 +302,9 @@ __device__ __forceinline__ void cta_merge_and_store(u64* sel_base, int nwarps_se
 //   * nactive != null: guard re-run of the queries queued by the first finalise (evs_finalize.cuh), NQ at a time.
 // ---------------------------------------------------------------------------------------------
 template <typename T, int NQ, int NV>
-struct ScanOcc {  // CTAs per SM the register allocation is held to (the measured optimum: 2 for fp32 rows, 4 for bf16 and int8 rows)
-    static constexpr int value = NQ == 1 ? ((sizeof(T) == 1 || (sizeof(T) == 2 && NV <= 2)) ? 4 : 2) : 1;
+struct ScanOcc {  // CTAs per SM the register allocation is held to (the measured optimum: 2 for fp32 and int8 rows, 4 for bf16 rows;
+                  // int8 rows hold two groups in registers)
+    static constexpr int value = NQ == 1 ? ((sizeof(T) == 2 && NV <= 2) ? 4 : 2) : 1;
 };
 
 __device__ __forceinline__ unsigned long long globaltimer_ns() {
@@ -583,13 +602,10 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
     __shared__ unsigned s_base;
     __shared__ u64 s_tau, s_wtau[8];  // s_wtau: each warp's running threshold (read only when it compacts: registers stay for the loop)
     __shared__ float s_twoE;
-    typedef typename RawVec<T>::type raw_t;
     constexpr bool I8 = sizeof(T) == 1;
     constexpr int QREGS = NV * Elem<T>::VEC;
     constexpr int RPG_RAW = (100 - QREGS) / (NV * 4);
-    // int8 rows: 8 bytes per lane and vector; 16 / NV rows per group (8 at d = 512) keep as many bytes in flight per warp as
-    // 4 bf16 rows
-    constexpr int RPG = I8 ? (NV >= 4 ? 4 : 16 / NV) : (RPG_RAW < 1 ? 1 : (RPG_RAW > 4 ? 4 : RPG_RAW));
+    constexpr int RPG = I8 ? I8Lane<NV>::ROWS : (RPG_RAW < 1 ? 1 : (RPG_RAW > 4 ? 4 : RPG_RAW));
     constexpr int KP = 64, CAPW = 128;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int nwarps = blockDim.x >> 5;
@@ -607,8 +623,6 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
     const long long total_warps = (long long)gridDim.x * nwarps;
     const long long gw = (long long)blockIdx.x * nwarps + warp;
     const long long ngroups = (p.n + RPG - 1) / RPG;
-    const size_t row_vecs = (size_t)p.d / Elem<T>::VEC;
-    const raw_t* base = reinterpret_cast<const raw_t*>(p.xb);
     QueryRegs<T, 1, NV> q;
     q.load(p.xq, p.q0, p.d, lane);
     int cnt = 0;
@@ -681,48 +695,16 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
         }
     };
 
-    auto do_group = [&](long long g) {
-        const long long r0 = g * RPG;
-        raw_t raw[RPG][NV];
-        float sr = 0.f;  // int8 rows: lane r < RPG holds the scale of row r0 + r
-        if constexpr (I8) {
-            if (lane < RPG) sr = __ldg(p.xs + (r0 + lane < p.n ? r0 + lane : p.n - 1));
-        }
+    // the best of the first 16 keys goes to its slot right away: on shards where a warp sees fewer than 128 rows (100k-row
+    // indexes) nobody ever compacts, and without this the slot maxima would stay empty and the pool would receive every key
+    // of the shard
+    auto publish_first16 = [&]() {
+        early = true;
+        __syncwarp();
+        u64 mx = lane < 16 ? buf[lane] : 0ull;
 #pragma unroll
-        for (int r = 0; r < RPG; r++) {
-            long long row = r0 + r < p.n ? r0 + r : p.n - 1;  // clamp: tail rows are re-read, not offered
-            const raw_t* src = base + (size_t)row * row_vecs + lane;
-#pragma unroll
-            for (int j = 0; j < NV; j++) {
-                if constexpr (sizeof(T) == 4) raw[r][j] = ldg_stream_f4(src + 32 * j);
-                else if constexpr (I8) raw[r][j] = ldg_stream_u2(src + 32 * j);
-                else raw[r][j] = ldg_stream_u4(src + 32 * j);
-            }
-        }
-#pragma unroll
-        for (int r = 0; r < RPG; r++) {
-            float s[1];
-            if constexpr (I8) s[0] = row_score_i8<NV>(raw[r], q, __shfl_sync(0xffffffffu, sr, r));
-            else row_scores<T, 1, NV>(raw[r], q, s);
-            if (r0 + r < p.n) {
-                const u64 key = make_key(s[0], (uint32_t)(r0 + r));  // warp-uniform
-                if (key > tcut) {
-                    if (lane == 0) buf[cnt] = key;
-                    if (++cnt == CAPW) compact();
-                    else if (cnt == 16 && !early) {
-                        // the best of the first 16 keys goes to its slot right away: on shards where a warp sees fewer than
-                        // 128 rows (100k-row indexes) nobody ever compacts, and without this the slot maxima would stay
-                        // empty and the pool would receive every key of the shard
-                        early = true;
-                        __syncwarp();
-                        u64 mx = lane < 16 ? buf[lane] : 0ull;
-#pragma unroll
-                        for (int off = 8; off >= 1; off >>= 1) mx = umax64(mx, __shfl_xor_sync(0xffffffffu, mx, off));
-                        if (lane == 0) atomicMax(reinterpret_cast<unsigned long long*>(G + (size_t)((~(uint32_t)mx) & (POOL_SLOTS - 1)) * POOL_GSTRIDE), (unsigned long long)mx);
-                    }
-                }
-            }
-        }
+        for (int off = 8; off >= 1; off >>= 1) mx = umax64(mx, __shfl_xor_sync(0xffffffffu, mx, off));
+        if (lane == 0) atomicMax(reinterpret_cast<unsigned long long*>(G + (size_t)((~(uint32_t)mx) & (POOL_SLOTS - 1)) * POOL_GSTRIDE), (unsigned long long)mx);
     };
     // Rows are dealt statically (group g to warp g mod W: the whole machine walks one window of the database, DRAM-friendly,
     // no counter traffic) for the first part of the shard and dynamically -- `chunk_groups` groups per grab from a global
@@ -734,17 +716,141 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
     const long long static_end = ngroups - dyn_groups;
     long long next = -1;
     if (dyn_groups > 0 && lane == 0) next = (long long)atomicAdd(p.next_chunk, 1u);  // the first grab: needed only after the static part
-    for (long long g = gw; g < static_end; g += total_warps) do_group(g);
-    if (dyn_groups > 0) {
+    if constexpr (I8) {
+        // int8 rows: a group of R rows is scored as a whole -- IDP.4A partial sums of every row, one halving reduction
+        // (i8_warp_sum), one admission ballot -- while the next group's loads are in flight in a second register buffer.
+        // Lanes rl * 2^RSH .. end with row rl's sum; the first of them offers its key.
+        typedef I8Lane<NV> L;
+        constexpr int R = L::ROWS, RSH = L::RSH;
+        const int8_t* codes = reinterpret_cast<const int8_t*>(p.xb);
+        const int rl = lane >> RSH;
+        const bool rep = (lane & ((1 << RSH) - 1)) == 0;
+        struct Group {
+            unsigned w[R][L::WORDS];
+            float sr;  // the scale of row rl
+        };
+        auto load = [&](Group& b, long long g) {
+            const long long r0 = g * R;
+            b.sr = __ldg(p.xs + (r0 + rl < p.n ? r0 + rl : p.n - 1));
+#pragma unroll
+            for (int r = 0; r < R; r++) {
+                const long long row = r0 + r < p.n ? r0 + r : p.n - 1;  // clamp: tail rows are re-read, not offered
+                L::load(codes + (size_t)row * p.d, lane, b.w[r]);
+            }
+        };
+        auto score = [&](const Group& b, long long g) {
+            // |I| <= d * I8_QMAX * 127 < 2^31 for d <= 512 (NV <= 2): the lane sums are combined in int32; wider rows reduce
+            // both chains (each < 2^31, interleaved) and combine them in fp64, exactly
+            constexpr int M = NV <= 2 ? R : 2 * R;
+            int v[M];
+#pragma unroll
+            for (int r = 0; r < R; r++) {
+                int ih = 0, il = 0;
+#pragma unroll
+                for (int w = 0; w < L::WORDS; w++) {
+                    ih = __dp4a((int)b.w[r][w], q.h[w], ih);
+                    il = __dp4a((int)b.w[r][w], q.l[w], il);
+                }
+                if constexpr (NV <= 2) v[r] = ih * 256 + il;
+                else {
+                    v[2 * r] = ih;
+                    v[2 * r + 1] = il;
+                }
+            }
+            i8_warp_sum<M>(v, lane);
+            float fi;
+            if constexpr (NV <= 2) fi = __int2float_rn(v[0]);
+            else {  // lanes with bit RSH - 1 clear hold the row's h sum, the others its l sum
+                const int o = __shfl_xor_sync(0xffffffffu, v[0], 1 << (RSH - 1));
+                const bool lo = lane & (1 << (RSH - 1));
+                fi = __double2float_rn(fma((double)(lo ? o : v[0]), 256.0, (double)(lo ? v[0] : o)));
+            }
+            const float s = __fmul_rn(fi, __fmul_rn(q.sq, b.sr));
+            const long long row = g * R + rl;
+            const u64 key = make_key(s, (uint32_t)row);
+            bool pass = rep && row < p.n && key > tcut;
+            unsigned m = __ballot_sync(0xffffffffu, pass);
+            if (m == 0u) return;
+            if (cnt + __popc(m) > CAPW) {  // after a compact cnt <= CAPW - 32: the group fits
+                compact();
+                pass = rep && row < p.n && key > tcut;
+                m = __ballot_sync(0xffffffffu, pass);
+            }
+            if (pass) buf[cnt + __popc(m & ((1u << lane) - 1u))] = key;
+            cnt += __popc(m);
+            if (cnt >= 16 && !early) publish_first16();
+        };
+        // the group after g in this warp's deal (-1: none); a grab consumes the one in flight and issues the next
         const long long C = p.chunk_groups;
-        const long long nchunks = (dyn_groups + C - 1) / C;
-        long long chunk = __shfl_sync(0xffffffffu, next, 0);
-        while (chunk < nchunks) {
-            if (lane == 0) next = (long long)atomicAdd(p.next_chunk, 1u);  // consumed after this chunk
+        const long long nchunks = dyn_groups > 0 ? (dyn_groups + C - 1) / C : 0;
+        long long cend = 0;  // end of the grabbed chunk being walked
+        auto grab = [&]() -> long long {
+            const long long chunk = dyn_groups > 0 ? __shfl_sync(0xffffffffu, next, 0) : nchunks;
+            if (chunk >= nchunks) return -1;
+            if (lane == 0) next = (long long)atomicAdd(p.next_chunk, 1u);
             const long long g0 = static_end + chunk * C;
-            const long long gend = g0 + C < ngroups ? g0 + C : ngroups;
-            for (long long g = g0; g < gend; g++) do_group(g);
-            chunk = __shfl_sync(0xffffffffu, next, 0);
+            cend = g0 + C < ngroups ? g0 + C : ngroups;
+            return g0;
+        };
+        auto advance = [&](long long g) -> long long {
+            if (g < static_end) return g + total_warps < static_end ? g + total_warps : grab();
+            return g + 1 < cend ? g + 1 : grab();
+        };
+        Group A, B;
+        long long g = gw < static_end ? gw : grab();
+        if (g >= 0) load(A, g);
+        while (g >= 0) {
+            const long long g1 = advance(g);
+            if (g1 >= 0) load(B, g1);
+            score(A, g);
+            if (g1 < 0) break;
+            g = advance(g1);
+            if (g >= 0) load(A, g);
+            score(B, g1);
+        }
+    } else {
+        typedef typename RawVec<T>::type raw_t;
+        const size_t row_vecs = (size_t)p.d / Elem<T>::VEC;
+        const raw_t* base = reinterpret_cast<const raw_t*>(p.xb);
+        auto do_group = [&](long long g) {
+            const long long r0 = g * RPG;
+            raw_t raw[RPG][NV];
+#pragma unroll
+            for (int r = 0; r < RPG; r++) {
+                long long row = r0 + r < p.n ? r0 + r : p.n - 1;  // clamp: tail rows are re-read, not offered
+                const raw_t* src = base + (size_t)row * row_vecs + lane;
+#pragma unroll
+                for (int j = 0; j < NV; j++) {
+                    if constexpr (sizeof(T) == 4) raw[r][j] = ldg_stream_f4(src + 32 * j);
+                    else raw[r][j] = ldg_stream_u4(src + 32 * j);
+                }
+            }
+#pragma unroll
+            for (int r = 0; r < RPG; r++) {
+                float s[1];
+                row_scores<T, 1, NV>(raw[r], q, s);
+                if (r0 + r < p.n) {
+                    const u64 key = make_key(s[0], (uint32_t)(r0 + r));  // warp-uniform
+                    if (key > tcut) {
+                        if (lane == 0) buf[cnt] = key;
+                        if (++cnt == CAPW) compact();
+                        else if (cnt == 16 && !early) publish_first16();
+                    }
+                }
+            }
+        };
+        for (long long g = gw; g < static_end; g += total_warps) do_group(g);
+        if (dyn_groups > 0) {
+            const long long C = p.chunk_groups;
+            const long long nchunks = (dyn_groups + C - 1) / C;
+            long long chunk = __shfl_sync(0xffffffffu, next, 0);
+            while (chunk < nchunks) {
+                if (lane == 0) next = (long long)atomicAdd(p.next_chunk, 1u);  // consumed after this chunk
+                const long long g0 = static_end + chunk * C;
+                const long long gend = g0 + C < ngroups ? g0 + C : ngroups;
+                for (long long g = g0; g < gend; g++) do_group(g);
+                chunk = __shfl_sync(0xffffffffu, next, 0);
+            }
         }
     }
     if (p.cta_clock && threadIdx.x == 0) t_loop = globaltimer_ns();

@@ -1,5 +1,5 @@
-// evs_scan_i8.cu -- the pool kernel (evs_scan.cuh: scan_pool_kernel) over the int8 scan copy of the rows, 1 .. 4 8-byte
-// vectors per lane (d = 256 .. 1024).  Only the fused single-query search scans this copy.
+// evs_scan_i8.cu -- the pool kernel (evs_scan.cuh: scan_pool_kernel) over the int8 scan copy of the rows, NV = d / 256
+// = 1 .. 4 (d = 256 .. 1024).  Only the fused single-query search scans this copy.
 #include "evs_scan_launch.cuh"
 
 namespace evs {

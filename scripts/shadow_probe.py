@@ -2,7 +2,9 @@
 per (rows, arm): time per search (CUDA events around `--iters` back-to-back searches of different queries), the bytes the
 search reads (int8 codes and row scales plus the fp32 rows of the candidates it re-scored exactly) and their rate against
 7.7 TB/s, the bound E of the first query, the distribution of the candidate count |C| over `--queries` queries and the
-searches that needed more than one re-score round.
+searches that needed more than one re-score round.  A separate pass with option "scan_clock" on (its searches are not
+timed) reads the per-CTA %globaltimer stamps: the scan loop's time (first CTA start to last loop end) and rate, and the
+phases of the last CTA's tail.
 
     python scripts/shadow_probe.py --rows 10000000 1250000 --out shadow_probe.jsonl
 """
@@ -55,6 +57,7 @@ def probe(n, d, k, shadow, queries, iters, seed=5):
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / iters
     wide, emax, _ = idx.shadow_stats()
+    clocks = scan_clock_pass(idx, qt, k, (n * d + n * 4) if shadow else n * d * 4)
     # E of the first query (evs_scan.cuh: shadow_bound_i8)
     q0 = q[0]
     sq = np.float32(np.abs(q0).max() / np.float32(32639))
@@ -66,6 +69,7 @@ def probe(n, d, k, shadow, queries, iters, seed=5):
     out = {"rows": n, "d": d, "k": k, "scan_shadow": shadow, "ms_per_search": ms, "bytes_per_search": nbytes,
            "tb_s": nbytes / ms / 1e9, "frac_hbm_peak": nbytes / (ms * 1e-3) / HBM_PEAK, "emax": emax,
            "E_first_query": E if shadow else None, "wide_searches": wide, "queries": queries}
+    out.update(clocks)
     if shadow:
         c = np.asarray(cands)
         out["candidates"] = {"min": int(c.min()), "p50": float(np.percentile(c, 50)), "p90": float(np.percentile(c, 90)),
@@ -73,6 +77,31 @@ def probe(n, d, k, shadow, queries, iters, seed=5):
     del idx
     torch.cuda.empty_cache()
     return out
+
+
+def scan_clock_pass(idx, qt, k, scan_bytes, searches=16):
+    """Medians over `searches` searches of the loop time (first CTA start to the last CTA's loop end), the loop's rate over
+    the bytes it streams, and the tail: last loop end -> the last CTA holds its ticket -> pool read -> the best KP ranked
+    -> re-scored -> results written (evs_scan.cuh: scan_pool_kernel)."""
+    evs.set_option("scan_clock", 1)
+    rec = {"loop_us": [], "end_spread_us": [], "loop_end_to_ticket_us": [], "ticket_to_pool_read_us": [],
+           "pool_read_to_ranked_us": [], "ranked_to_rescored_us": [], "rescored_to_written_us": [], "kernel_us": []}
+    try:
+        for i in range(searches):
+            idx.search(qt[i:i + 1], k)
+            c = idx.scan_clocks().astype(np.int64)
+            st, fs = idx.last_cta_stamps.astype(np.int64), idx.finalize_stamps.astype(np.int64)
+            t0, end = c[:, 0].min(), c[:, 1].max()
+            for name, v in (("loop_us", end - t0), ("end_spread_us", end - c[:, 1].min()), ("loop_end_to_ticket_us", st[0] - end),
+                            ("ticket_to_pool_read_us", fs[0] - st[0]), ("pool_read_to_ranked_us", fs[2] - fs[0]),
+                            ("ranked_to_rescored_us", fs[3] - fs[2]), ("rescored_to_written_us", fs[4] - fs[3]),
+                            ("kernel_us", fs[4] - t0)):
+                rec[name].append(v / 1e3)
+    finally:
+        evs.set_option("scan_clock", 0)
+    out = {name: round(float(np.median(v)), 2) for name, v in rec.items()}
+    out["loop_tb_s"] = round(scan_bytes / (out["loop_us"] * 1e-6) / 1e12, 3)
+    return {"scan_clock": out}
 
 
 def main():
@@ -84,14 +113,20 @@ def main():
     ap.add_argument("--iters", type=int, default=200)
     ap.add_argument("--out", default=None)
     ap.add_argument("--shadow-min-rows", type=int, default=0, help="routing cut of the copy's path (0: every size above small_max_rows)")
+    ap.add_argument("--ctas-per-sm", type=int, default=0, help="option ctas_per_sm (0: the planned default)")
+    ap.add_argument("--chunk-groups", type=int, default=0, help="option scan_chunk_groups (0: the default)")
+    ap.add_argument("--arms", type=int, nargs="+", default=[1, 0, 1, 0], help="scan_shadow of each pass, in order")
     a = ap.parse_args()
     evs.set_option("shadow_min_rows", a.shadow_min_rows)
+    evs.set_option("ctas_per_sm", a.ctas_per_sm)
+    if a.chunk_groups:
+        evs.set_option("scan_chunk_groups", a.chunk_groups)
     info = gpu_info()
     lines = []
     for n in a.rows:
-        for shadow in (1, 0, 1, 0):
+        for shadow in a.arms:
             r = probe(n, a.dim, a.k, shadow, a.queries if shadow else 0, a.iters)
-            r["gpu"] = info
+            r.update(gpu=info, ctas_per_sm=evs.get_option("ctas_per_sm"), scan_chunk_groups=evs.get_option("scan_chunk_groups"))
             lines.append(json.dumps(r))
             print(lines[-1], flush=True)
     if a.out:
