@@ -12,6 +12,7 @@ EVS_OK, EVS_EINVAL, EVS_ENODEV, EVS_ECUDA, EVS_ENOMEM, EVS_EIO, EVS_EFORMAT, EVS
 EVS_F32, EVS_F16, EVS_BF16 = 0, 1, 2
 EVS_STORE_F32, EVS_STORE_BF16_F32 = 0, 1
 EVS_MAX_K = 112
+EVS_MAX_K_LARGE = 2048
 EVS_IPC_HANDLE_BYTES = 64
 
 _c = ctypes
@@ -66,6 +67,7 @@ SIGNATURES = {
     "evs_index_max_row_norm": (_i, [_vp, _pf]),
     "evs_index_guard_stats": (_i, [_vp, _pi64, _pi64]),
     "evs_index_shadow_stats": (_i, [_vp, _pi64, _pf, _pi64]),
+    "evs_index_large_k_stats": (_i, [_vp, _pi64, _pi64]),
     "evs_index_read_rows": (_i, [_c.c_char_p, _i, _i, _i64, _i64, _c.POINTER(_vp), _pi64]),
     "evs_index_file_info": (_i, [_c.c_char_p, _pi, _pi64]),
     "evs_index_scan_clocks": (_i, [_vp, _vp, _i64, _pi64]),

@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libevs.so")
 SOURCES = ["evs_scan_f32_512.cu", "evs_scan_f32_narrow.cu", "evs_scan_f32_wide.cu", "evs_scan_bf16_narrow.cu", "evs_scan_bf16_wide.cu", "evs_scan_i8.cu",
-           "evs_scan_generic.cu", "evs_kernels.cu", "evs_api.cu", "evs_tc.cu", "evs_tc2.cu"]
+           "evs_scan_generic.cu", "evs_kernels.cu", "evs_api.cu", "evs_tc.cu", "evs_tc2.cu", "evs_large_k.cu"]
 HEADERS = ["evs_common.cuh", "evs_scan.cuh", "evs_scan_launch.cuh", "evs_finalize.cuh", "evs_tc_common.cuh", "evs_internal.h", os.path.join("..", "..", "include", "evs.h")]
 
 NVCC_FLAGS = [

@@ -116,6 +116,11 @@ struct evs_index {
     unsigned* done_pin = nullptr;     // host-mapped word the small-shard kernel raises behind its results (polled by evs_index_search)
     unsigned* done_pin_dev = nullptr;
     unsigned done_seq = 0;
+    // large-k searches (evs_large_k.cu): per query of a pass S, C [npad] u32 and R [npad] u64, then the pass state and one
+    // stats word; allocated by the first such search
+    unsigned char* lk_ws = nullptr; size_t lk_ws_cap = 0;
+    int64_t lk_searches = 0;
+    unsigned* lk_stats = nullptr;     // into lk_ws: largest |C| of the last large-k search
 };
 
 static int use_device(int device) {
@@ -247,6 +252,9 @@ extern "C" int evs_set_option(const char* name, int64_t value) {
     } else if (!strcmp(name, "io_threads")) {
         if (value < 0 || value > 64) return fail(EVS_EINVAL, "io_threads must be in [0, 64]");
         g_io_threads.store((int)value);
+    } else if (!strcmp(name, "max_k")) {
+        if (value < EVS_MAX_K || value > EVS_MAX_K_LARGE) return fail(EVS_EINVAL, "max_k must be in [%d, %d]", EVS_MAX_K, EVS_MAX_K_LARGE);
+        g_tune.max_k = (int)value;
     } else {
         return fail(EVS_EINVAL, "unknown option '%s'", name);
     }
@@ -286,6 +294,7 @@ extern "C" int evs_get_option(const char* name, int64_t* value) {
     else if (!strcmp(name, "small_fast_cap")) *value = g_tune.small_fast_cap;
     else if (!strcmp(name, "scan_shadow")) *value = g_tune.scan_shadow;
     else if (!strcmp(name, "shadow_min_rows")) *value = g_tune.shadow_min_rows;
+    else if (!strcmp(name, "max_k")) *value = g_tune.max_k;
     else return fail(EVS_EINVAL, "unknown option '%s'", name);
     return EVS_OK;
 }
@@ -347,6 +356,7 @@ extern "C" int evs_index_free(evs_index* idx) {
     cudaFree(idx->guard_lists);
     cudaFree(idx->cta_clock);
     cudaFree(idx->pool);
+    cudaFree(idx->lk_ws);
     cudaFreeHost(idx->tc_overflow_pin);
     cudaFreeHost(idx->q_pin);
     cudaFreeHost(idx->I_pin);  // D_pin points into the same allocation
@@ -634,7 +644,7 @@ struct SearchOut {
 
 // Which scan serves a batch.  Decided ONCE per search from one snapshot of the tuning options and passed down, so that the
 // exchange entry points and the search itself can never disagree (they used to read the options twice).
-enum { PATH_GEMV = 0, PATH_TC_HEAP = 1, PATH_TC_SYNC = 2 };
+enum { PATH_GEMV = 0, PATH_TC_HEAP = 1, PATH_TC_SYNC = 2, PATH_LARGE_K = 3 /* k > EVS_MAX_K: evs_large_k.cu */ };
 struct PathInfo {
     int kind = PATH_GEMV;
     int kp = 64;
@@ -685,6 +695,10 @@ static bool shadow_applies(const evs_index* idx, int64_t nq, int kp, const ScanT
 
 static PathInfo plan_path(const evs_index* idx, int64_t nq, int64_t k, const ScanTuning& tune, bool allow_tc) {
     PathInfo pi;
+    if (k > EVS_MAX_K) {  // whatever nq, storage or tensor-core routing say: the fp32 rows, exact by construction
+        pi.kind = PATH_LARGE_K;
+        return pi;
+    }
     const bool bf16 = idx->storage == EVS_STORE_BF16_F32;
     pi.kp = pick_kp(k);
     pi.err_coef = bf16 ? 0.f : gemv_err_coef(idx->d);
@@ -1117,6 +1131,67 @@ static int search_tc_sync_locked(evs_index* idx, int64_t nq, const float* q_dev,
     return EVS_OK;
 }
 
+// k > EVS_MAX_K (evs_large_k.cu): passes of max_queries_per_pass(d) queries over the fp32 rows, each a score scan that keeps
+// every row's scan key, a radix select of the k-th key, the window cut at 2E below it, a grid-wide canonical re-score of the
+// window and the ranking.  Exact by construction (DESIGN.md section 2): nothing is certified afterwards or re-run.
+static int search_large_k_locked(evs_index* idx, int64_t nq, const float* q_dev, int64_t k, const SearchOut& out, cudaStream_t st,
+                                 const ScanTuning& tune, bool scan_only, int profile) {
+    if (out.x) return fail(EVS_ECUDA, "internal: a large-k search writes its partial to staging, not to the exchange slots");
+    const int qpp = max_queries_per_pass(idx->d, 0);
+    ScanTuning gt = tune;
+    gt.scan_variant = 1;  // the direct-load grid (the ring variant keeps lists, not keys)
+    ScanPlan plan;
+    CU(plan_scan(idx->ntotal, idx->d, SCAN_F32, 64, qpp, idx->sm_count, gt, &plan));
+    const size_t npad = ((size_t)idx->ntotal + 31) & ~(size_t)31;
+    const size_t arrays = (size_t)qpp * npad * 16;  // S, C (u32) and R (u64)
+    const size_t state = large_k_state_bytes(qpp);
+    int rc = ensure_dev(&idx->lk_ws, &idx->lk_ws_cap, arrays + state + 16);
+    if (rc) return rc;
+    unsigned char* ws = idx->lk_ws;
+    idx->lk_stats = reinterpret_cast<unsigned*>(ws + arrays + state);
+    if (!scan_only) {
+        if ((rc = ensure_dev(&idx->margins_dev, &idx->margins_cap, (size_t)nq))) return rc;
+        idx->last_nq = nq;
+        idx->lk_searches++;
+        CU(cudaMemsetAsync(idx->lk_stats, 0, sizeof(unsigned), st));
+    }
+    LargeKArgs a;
+    a.xb = idx->xb32;
+    a.n = idx->ntotal;
+    a.npad = (long long)npad;
+    a.d = idx->d;
+    a.nv = plan.variant == 1 ? plan.nv : 0;
+    a.grid = plan.grid;
+    a.k = (int)k;
+    a.fast_widen = idx->special_host == 0u;
+    a.all_rows = idx->special_host != 0u;  // subnormal / inf / NaN elements: the fp32 scan has no bound, every row is a candidate
+    a.err_coef = gemv_err_coef(idx->d);
+    a.max_norm = reinterpret_cast<const float*>(idx->words + W_MAX_NORM);
+    a.S = reinterpret_cast<unsigned*>(ws);
+    a.C = a.S + (size_t)qpp * npad;
+    a.R = reinterpret_cast<unsigned long long*>(a.C + (size_t)qpp * npad);
+    a.hist = reinterpret_cast<unsigned*>(ws + arrays);
+    a.st = reinterpret_cast<LargeKQuery*>(a.hist + (size_t)3 * qpp * LK_BINS);
+    a.stats = idx->lk_stats;
+    a.id_base = idx->id_base;
+    for (int64_t p0 = 0; p0 < nq; p0 += qpp) {
+        a.nq_pass = (int)((nq - p0) < qpp ? (nq - p0) : qpp);
+        a.xq = q_dev + (size_t)p0 * idx->d;
+        a.D = out.D ? out.D + (size_t)p0 * k : nullptr;
+        a.I = out.I ? reinterpret_cast<long long*>(out.I + (size_t)p0 * k) : nullptr;
+        a.P_scores = out.P_scores ? out.P_scores + (size_t)p0 * k : nullptr;
+        a.P_ids = out.P_ids ? reinterpret_cast<long long*>(out.P_ids + (size_t)p0 * k) : nullptr;
+        a.margins = scan_only ? nullptr : idx->margins_dev + p0;
+        CU(cudaMemsetAsync(a.hist, 0, state, st));
+        ProfileScope prof;
+        if ((rc = prof.begin(idx, profile, st))) return rc;
+        CU(launch_large_k_scan(a, st));
+        if ((rc = prof.end(st))) return rc;
+        if (!scan_only) CU(launch_large_k_rest(a, idx->sm_count, st));
+    }
+    return EVS_OK;
+}
+
 static int search_enqueue_locked(evs_index* idx, int64_t nq, const float* q_dev, int64_t k, const SearchOut& out, cudaStream_t st,
                                  const ScanTuning& tune, const PathInfo& pi, bool scan_only, int kp_override) {
     int profile;
@@ -1124,6 +1199,7 @@ static int search_enqueue_locked(evs_index* idx, int64_t nq, const float* q_dev,
         std::lock_guard<std::mutex> lk(g_tune_mu);
         profile = g_profile_scans && !scan_only;
     }
+    if (pi.kind == PATH_LARGE_K) return search_large_k_locked(idx, nq, q_dev, k, out, st, tune, scan_only, profile);
     if (pi.kind == PATH_TC_HEAP || pi.kind == PATH_TC_SYNC) {
         idx->bar_used = false;
         int rc = pi.kind == PATH_TC_HEAP ? search_tc_heap_locked(idx, nq, q_dev, k, out, st, tune, pi, scan_only, profile)
@@ -1242,18 +1318,21 @@ __global__ void fill_partial_kernel(double* S, long long* I, long long count) {
     }
 }
 
-static int check_search_args(const evs_index* idx, int64_t nq, const void* q, int64_t k, const void* o1, const void* o2) {
-    if (!idx) return fail(EVS_EINVAL, "idx is NULL");
-    if (nq < 0) return fail(EVS_EINVAL, "nq must be >= 0");
-    if (k <= 0) return fail(EVS_EINVAL, "k must be > 0 (got %lld)", (long long)k);  // FAISS_THROW_IF_NOT(k > 0)
-    if (k > EVS_MAX_K) return fail(EVS_ELIMIT, "k = %lld exceeds EVS_MAX_K = %d", (long long)k, EVS_MAX_K);
-    if (nq > 0 && (!q || !o1 || !o2)) return fail(EVS_EINVAL, "NULL query or output buffer");
-    return EVS_OK;
-}
-
 static ScanTuning tune_snapshot() {
     std::lock_guard<std::mutex> lk(g_tune_mu);
     return g_tune;
+}
+
+// k is tested against the option "max_k" of the snapshot that then routes the search
+static int check_search_args(const evs_index* idx, int64_t nq, const void* q, int64_t k, const void* o1, const void* o2,
+                             const ScanTuning& tune) {
+    if (!idx) return fail(EVS_EINVAL, "idx is NULL");
+    if (nq < 0) return fail(EVS_EINVAL, "nq must be >= 0");
+    if (k <= 0) return fail(EVS_EINVAL, "k must be > 0 (got %lld)", (long long)k);  // FAISS_THROW_IF_NOT(k > 0)
+    if (k > tune.max_k) return fail(EVS_ELIMIT, "k = %lld exceeds the option max_k = %d (EVS_MAX_K = %d, EVS_MAX_K_LARGE = %d)",
+                                    (long long)k, tune.max_k, EVS_MAX_K, EVS_MAX_K_LARGE);
+    if (nq > 0 && (!q || !o1 || !o2)) return fail(EVS_EINVAL, "NULL query or output buffer");
+    return EVS_OK;
 }
 
 // order stream `st` after the previous user of the handle's workspace and enqueue the search
@@ -1276,27 +1355,27 @@ static int search_dev_common(evs_index* idx, int64_t nq, const float* q_dev, int
 
 extern "C" int evs_index_search_dev(evs_index* idx, int64_t nq, const float* q_dev, int64_t k, float* D_dev, int64_t* I_dev,
                                     void* stream) {
-    int rc = check_search_args(idx, nq, q_dev, k, D_dev, I_dev);
+    const ScanTuning tune = tune_snapshot();
+    int rc = check_search_args(idx, nq, q_dev, k, D_dev, I_dev, tune);
     if (rc || nq == 0) return rc;
     std::lock_guard<std::mutex> lk(idx->mu);
     if ((rc = use_device(idx->device))) return rc;
     SearchOut out;
     out.D = D_dev;
     out.I = I_dev;
-    const ScanTuning tune = tune_snapshot();
     return search_dev_common(idx, nq, q_dev, k, out, (cudaStream_t)stream, tune, plan_path(idx, nq, k, tune, true));
 }
 
 extern "C" int evs_index_search_partial_dev(evs_index* idx, int64_t nq, const float* q_dev, int64_t k, double* out_scores_dev,
                                             int64_t* out_ids_dev, void* stream) {
-    int rc = check_search_args(idx, nq, q_dev, k, out_scores_dev, out_ids_dev);
+    const ScanTuning tune = tune_snapshot();
+    int rc = check_search_args(idx, nq, q_dev, k, out_scores_dev, out_ids_dev, tune);
     if (rc || nq == 0) return rc;
     std::lock_guard<std::mutex> lk(idx->mu);
     if ((rc = use_device(idx->device))) return rc;
     SearchOut out;
     out.P_scores = out_scores_dev;
     out.P_ids = out_ids_dev;
-    const ScanTuning tune = tune_snapshot();
     return search_dev_common(idx, nq, q_dev, k, out, (cudaStream_t)stream, tune, plan_path(idx, nq, k, tune, true));
 }
 
@@ -1305,6 +1384,18 @@ extern "C" int evs_merge_partials_dev(int device, int nparts, int64_t nq, int64_
     if (nparts <= 0 || nq < 0 || k <= 0) return fail(EVS_EINVAL, "bad nparts/nq/k");
     if (nq == 0) return EVS_OK;
     if (!scores_dev || !ids_dev || !D_dev || !I_dev) return fail(EVS_EINVAL, "NULL buffer");
+    if (k > EVS_MAX_K) {  // large k: up to 8 parts, merged without a shared-memory copy
+        const ScanTuning tune = tune_snapshot();
+        if (k > tune.max_k) return fail(EVS_ELIMIT, "k = %lld exceeds the option max_k = %d", (long long)k, tune.max_k);
+        if (nparts > 8) return fail(EVS_ELIMIT, "a merge for k > %d takes at most 8 parts (got %d)", EVS_MAX_K, nparts);
+        int rc = use_device(device);
+        if (rc) return rc;
+        if (part_stride == 0) part_stride = nq * k;
+        if (part_stride < nq * k) return fail(EVS_EINVAL, "part_stride smaller than nq*k");
+        CU(launch_merge_partials_large(nparts, nq, (int)k, scores_dev, reinterpret_cast<const long long*>(ids_dev), part_stride,
+                                       D_dev, reinterpret_cast<long long*>(I_dev), (cudaStream_t)stream));
+        return EVS_OK;
+    }
     if ((size_t)nparts * k * 24 > 200 * 1024) return fail(EVS_ELIMIT, "nparts*k too large for one merge");
     int rc = use_device(device);
     if (rc) return rc;
@@ -1372,7 +1463,8 @@ static int host_fetch_locked(evs_index* idx, int64_t nq, int64_t k, float* D_hos
 }
 
 extern "C" int evs_index_search(evs_index* idx, int64_t nq, const float* q_host, int64_t k, float* D_host, int64_t* I_host) {
-    int rc = check_search_args(idx, nq, q_host, k, D_host, I_host);
+    const ScanTuning tune = tune_snapshot();
+    int rc = check_search_args(idx, nq, q_host, k, D_host, I_host, tune);
     if (rc || nq == 0) return rc;
     std::lock_guard<std::mutex> lk(idx->mu);
     if ((rc = use_device(idx->device))) return rc;
@@ -1382,7 +1474,6 @@ extern "C" int evs_index_search(evs_index* idx, int64_t nq, const float* q_host,
     SearchOut out;
     out.D = idx->D_dev;
     out.I = idx->I_dev;
-    const ScanTuning tune = tune_snapshot();
     const PathInfo pi = plan_path(idx, nq, k, tune, true);
     // one query, one launch: the kernel's last CTA writes the k results (k * 12 bytes) straight into the mapped pinned
     // buffer; the host only waits for the stream (what the application issues, oldapp.py:2005: ~6 us less per search)
@@ -1481,7 +1572,7 @@ extern "C" int evs_exchange_create(int device, int rank, int world, int64_t max_
     *out = nullptr;
     if (world < 1 || world > 8) return fail(EVS_ELIMIT, "world must be in [1, 8] (one NVSwitch box), got %d", world);
     if (rank < 0 || rank >= world) return fail(EVS_EINVAL, "rank %d out of range for world %d", rank, world);
-    if (max_nq <= 0 || max_k <= 0 || max_k > EVS_MAX_K) return fail(EVS_EINVAL, "bad max_nq/max_k");
+    if (max_nq <= 0 || max_k <= 0 || max_k > tune_snapshot().max_k) return fail(EVS_EINVAL, "bad max_nq/max_k");
     int ndev = 0;
     evs_device_count(&ndev);
     if (ndev <= 0) return fail(EVS_ENODEV, "no CUDA device: libevs has no CPU fallback");
@@ -1590,7 +1681,7 @@ static int exchange_take_failure(evs_exchange* ex) {
 
 // enqueue scan -> finalise (-> publish) -> merge for one exchange-mode search; idx->mu and ex->mu are held
 static int search_exchange_enqueue_locked(evs_index* idx, evs_exchange* ex, int64_t nq, const float* q_dev, int64_t k, float* D_dev,
-                                          int64_t* I_dev, cudaStream_t st) {
+                                          int64_t* I_dev, cudaStream_t st, const ScanTuning& tune) {
     Exchange x;
     for (int g = 0; g < ex->world; g++) x.peer[g] = ex->peer[g];
     x.rank = ex->rank;
@@ -1601,12 +1692,11 @@ static int search_exchange_enqueue_locked(evs_index* idx, evs_exchange* ex, int6
     x.nq_total = nq;
     x.k = (int)k;
     x.status = ex->status_dev;
-    const ScanTuning tune = tune_snapshot();  // ONE snapshot decides the path here and inside the search
-    const PathInfo pi = plan_path(idx, nq, k, tune, true);
+    const PathInfo pi = plan_path(idx, nq, k, tune, true);  // ONE snapshot decides the path here and inside the search
     // empty shard / scans that need the host (overflow repair) / device-guarded batches (their second finalise may still
     // overwrite results): the partial goes to local staging and a publish kernel stores it into the peers' slots;
     // otherwise the finalise kernel stores this shard's k best straight into every rank's slot
-    const bool staged = idx->ntotal == 0 || pi.kind == PATH_TC_SYNC || (pi.kind == PATH_TC_HEAP && pi.guard);
+    const bool staged = idx->ntotal == 0 || pi.kind == PATH_TC_SYNC || (pi.kind == PATH_TC_HEAP && pi.guard) || pi.kind == PATH_LARGE_K;
     const bool one_launch = !staged && pi.kind == PATH_GEMV && pi.fused;  // scan + finalise + peer stores + wait + merge
     SearchOut out;
     if (staged) {
@@ -1623,7 +1713,9 @@ static int search_exchange_enqueue_locked(evs_index* idx, evs_exchange* ex, int6
                                               : search_dev_common(idx, nq, q_dev, k, out, st, tune, pi);
     cudaError_t e = cudaSuccess;
     if (!rc && staged) e = launch_publish_partials(x, nq, (int)k, ex->stage_scores, reinterpret_cast<const long long*>(ex->stage_ids), st);
-    if (!rc && e == cudaSuccess && !one_launch) e = launch_merge_exchange(x, nq, (int)k, D_dev, reinterpret_cast<long long*>(I_dev), st);
+    if (!rc && e == cudaSuccess && !one_launch)
+        e = k > EVS_MAX_K ? launch_merge_exchange_large(x, nq, (int)k, D_dev, reinterpret_cast<long long*>(I_dev), st)
+                          : launch_merge_exchange(x, nq, (int)k, D_dev, reinterpret_cast<long long*>(I_dev), st);
     if (!rc && e != cudaSuccess) rc = fail(EVS_ECUDA, "exchange launch failed: %s", cudaGetErrorString(e));
     ex->seq = x.seq;  // stay in step with the peers whatever happened
     if (rc) {
@@ -1650,7 +1742,8 @@ static int check_exchange_args(const evs_index* idx, const evs_exchange* ex, int
 
 extern "C" int evs_index_search_exchange_dev(evs_index* idx, evs_exchange* ex, int64_t nq, const float* q_dev, int64_t k,
                                              float* D_dev, int64_t* I_dev, void* stream) {
-    int rc = check_search_args(idx, nq, q_dev, k, D_dev, I_dev);
+    const ScanTuning tune = tune_snapshot();
+    int rc = check_search_args(idx, nq, q_dev, k, D_dev, I_dev, tune);
     if (rc || nq == 0) return rc;
     if ((rc = check_exchange_args(idx, ex, nq, k))) return rc;
     std::lock_guard<std::mutex> lk(idx->mu);
@@ -1659,13 +1752,14 @@ extern "C" int evs_index_search_exchange_dev(evs_index* idx, evs_exchange* ex, i
     // asynchronous entry point: a failure seen by an EARLIER search's merge kernel is reported here (once), before this
     // search is enqueued -- every rank still enqueues its searches in step
     const int late = exchange_take_failure(ex);
-    rc = search_exchange_enqueue_locked(idx, ex, nq, q_dev, k, D_dev, I_dev, (cudaStream_t)stream);
+    rc = search_exchange_enqueue_locked(idx, ex, nq, q_dev, k, D_dev, I_dev, (cudaStream_t)stream, tune);
     return rc ? rc : late;
 }
 
 extern "C" int evs_index_search_exchange(evs_index* idx, evs_exchange* ex, int64_t nq, const float* q_host, int64_t k, float* D_host,
                                          int64_t* I_host) {
-    int rc = check_search_args(idx, nq, q_host, k, D_host, I_host);
+    const ScanTuning tune = tune_snapshot();
+    int rc = check_search_args(idx, nq, q_host, k, D_host, I_host, tune);
     if (rc || nq == 0) return rc;
     if ((rc = check_exchange_args(idx, ex, nq, k))) return rc;
     std::lock_guard<std::mutex> lk(idx->mu);
@@ -1680,13 +1774,12 @@ extern "C" int evs_index_search_exchange(evs_index* idx, evs_exchange* ex, int64
     // mapped pinned buffer (decided like search_exchange_enqueue_locked decides the path: same options snapshot rules)
     bool direct = false;
     {
-        const ScanTuning tune = tune_snapshot();
         const PathInfo pi = plan_path(idx, nq, k, tune, true);
         direct = nq == 1 && idx->ntotal > 0 && pi.kind == PATH_GEMV && pi.fused && idx->I_pin_dev != nullptr;
     }
     float* Dd = direct ? reinterpret_cast<float*>(idx->I_pin_dev + (size_t)nq * k) : idx->D_dev;
     int64_t* Id = direct ? idx->I_pin_dev : idx->I_dev;
-    rc = search_exchange_enqueue_locked(idx, ex, nq, idx->q_dev, k, Dd, Id, st);
+    rc = search_exchange_enqueue_locked(idx, ex, nq, idx->q_dev, k, Dd, Id, st, tune);
     if (!rc && direct) {
         cudaError_t se = cudaStreamSynchronize(st);
         if (se != cudaSuccess) rc = fail(EVS_ECUDA, "search failed: %s", cudaGetErrorString(se));
@@ -1717,7 +1810,8 @@ extern "C" int evs_index_last_margins(evs_index* idx, int64_t nq, float* margins
 }
 
 extern "C" int evs_index_time_scan(evs_index* idx, int64_t nq, const float* q_dev, int64_t k, int iters, float* mean_ms) {
-    int rc = check_search_args(idx, nq, q_dev, k, mean_ms, mean_ms);
+    const ScanTuning tune = tune_snapshot();
+    int rc = check_search_args(idx, nq, q_dev, k, mean_ms, mean_ms, tune);
     if (rc) return rc;
     if (nq == 0 || iters <= 0 || idx->ntotal == 0) return fail(EVS_EINVAL, "nothing to time");
     std::lock_guard<std::mutex> lk(idx->mu);
@@ -1728,7 +1822,6 @@ extern "C" int evs_index_time_scan(evs_index* idx, int64_t nq, const float* q_de
     CU(cudaEventCreate(&e1));
     if ((rc = ws_acquire(idx, st))) return rc;
     SearchOut none;
-    const ScanTuning tune = tune_snapshot();
     const PathInfo pi = plan_path(idx, nq, k, tune, true);
     // the int8 copy is scanned only by the fused search kernel: its scan is the whole search, results to the workspace
     if (pi.shadow && !(rc = host_stage_locked(idx, nq, k))) {
@@ -1795,6 +1888,19 @@ extern "C" int evs_index_shadow_stats(evs_index* idx, int64_t* wide_searches, fl
     if (wide_searches) *wide_searches = (int64_t)w[0];
     if (last_candidates) *last_candidates = (int64_t)w[1];
     if (emax) *emax = idx->xi8 ? idx->emax_host : -1.f;
+    return EVS_OK;
+}
+
+extern "C" int evs_index_large_k_stats(evs_index* idx, int64_t* searches, int64_t* last_candidates) {
+    if (!idx) return fail(EVS_EINVAL, "idx is NULL");
+    std::lock_guard<std::mutex> lk(idx->mu);
+    int rc = use_device(idx->device);
+    if (rc) return rc;
+    if (idx->have_last_stream) CU(cudaStreamSynchronize(idx->last_stream));
+    unsigned c = 0;
+    if (idx->lk_stats) CU(cudaMemcpy(&c, idx->lk_stats, sizeof(c), cudaMemcpyDeviceToHost));
+    if (searches) *searches = idx->lk_searches;
+    if (last_candidates) *last_candidates = (int64_t)c;
     return EVS_OK;
 }
 

@@ -47,6 +47,8 @@ struct ScanTuning {
     int shadow_min_rows = 262144;  // below it the fp32 rows are scanned: the int8 copy's search costs ~64 us however small the
                                    // shard (the last CTA re-scores a window of ~200 rows in rounds); 131 072 x 512: 64 against
                                    // 57 us; 262 144: 80 against 97 us (profiles/int8_min_rows_sweep.jsonl)
+    int max_k = EVS_MAX_K;         // largest k a search accepts, in [EVS_MAX_K, EVS_MAX_K_LARGE]; k > EVS_MAX_K takes the
+                                   // large-k path (evs_large_k.cu)
 };
 
 struct ScanPlan {
@@ -275,5 +277,51 @@ cudaError_t launch_row_norm_max(const float* rows, long long n, int d, float* ma
                                 void* dst16 = nullptr, signed char* dst8 = nullptr, float* scale8 = nullptr, float* emax = nullptr);
 // small device fills used on the search path instead of memset nodes
 cudaError_t launch_fill_i32(int* p, long long count, int value, cudaStream_t st);
+
+// ---- large-k search (EVS_MAX_K < k <= EVS_MAX_K_LARGE; evs_large_k.cu, DESIGN.md section 2) ----
+constexpr int LK_BINS = 2048;  // radix digits of 11 bits
+struct LargeKQuery {           // per query of a pass, device; written by the threshold select at level 0
+    unsigned prefix;           // digits of the k-th largest scan key found so far
+    unsigned krem;             // rank of that key among the keys that share the prefix
+    unsigned cut;              // candidates: scan key >= cut (0: every row)
+    unsigned ncand;            // |C|
+    unsigned best_excl;        // largest scan key below the cut (0: none)
+    unsigned done;             // the cut is known (every row is a candidate): the later digit passes have nothing to do
+    float E;                   // bound of |scan score - exact score| of every row for this query
+    unsigned pad;
+};
+struct LargeKArgs {
+    const float* xb = nullptr;  // the fp32 rows
+    long long n = 0;
+    long long npad = 0;         // row stride of the per-query workspace arrays (n rounded up to 32)
+    int d = 0;
+    int nv = 0;                 // 16-byte vectors per lane per row (0: generic-d kernel)
+    int grid = 0;               // score scan: CTAs of 256 threads
+    const float* xq = nullptr;  // the queries of this pass [nq_pass][d]
+    int nq_pass = 0;
+    int k = 0;
+    int fast_widen = 0;         // the index holds no subnormal / inf / NaN element
+    int all_rows = 0;           // ... it does: every row is a candidate
+    float err_coef = 0.f;       // scan error relative to |q| max|x| (gemv_err_coef)
+    const float* max_norm = nullptr;
+    unsigned* S = nullptr;      // [nq_pass][npad] order-preserving scan keys
+    unsigned* C = nullptr;      // [nq_pass][npad] candidate rows
+    unsigned long long* R = nullptr;  // [nq_pass][npad] canonical rank keys of the candidates (0: NaN)
+    unsigned* hist = nullptr;   // [3][nq_pass][LK_BINS] digit histograms (zeroed before the pass)
+    LargeKQuery* st = nullptr;  // [nq_pass]
+    unsigned* stats = nullptr;  // largest |C| of this search
+    long long id_base = 0;
+    float* D = nullptr;         // final results of the pass's first query, row stride k (or null)
+    long long* I = nullptr;
+    double* P_scores = nullptr;  // shard partial (when D is null)
+    long long* P_ids = nullptr;
+    float* margins = nullptr;   // [nq_pass]
+};
+size_t large_k_state_bytes(int qpp);  // hist + st of a pass (zeroed before it)
+cudaError_t launch_large_k_scan(const LargeKArgs& a, cudaStream_t st);
+cudaError_t launch_large_k_rest(const LargeKArgs& a, int sm_count, cudaStream_t st);
+cudaError_t launch_merge_partials_large(int nparts, long long nq, int k, const double* scores, const long long* ids,
+                                        long long part_stride, float* D, long long* I, cudaStream_t st);
+cudaError_t launch_merge_exchange_large(const Exchange& x, long long nq, int k, float* D, long long* I, cudaStream_t st);
 
 }  // namespace evs

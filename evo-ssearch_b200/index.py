@@ -139,6 +139,13 @@ class IndexFlatIP:
         check(lib().evs_index_shadow_stats(self._h, ctypes.byref(w), ctypes.byref(e), ctypes.byref(c)))
         return w.value, e.value, c.value
 
+    def large_k_stats(self):
+        """``(searches, last_candidates)``: searches with k > 112 (option ``max_k``) on this index, and how many rows the
+        last one re-scored exactly (its largest candidate set over the queries)."""
+        s, c = ctypes.c_int64(0), ctypes.c_int64(0)
+        check(lib().evs_index_large_k_stats(self._h, ctypes.byref(s), ctypes.byref(c)))
+        return s.value, c.value
+
     def scan_clocks(self) -> np.ndarray:
         """Diagnostics (option ``scan_clock``): ``uint64[nctas, 2]`` start / end-of-scan-loop times (ns) of the CTAs of
         the last fused single-query scan."""

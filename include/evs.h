@@ -51,7 +51,7 @@ extern "C" {
 #define EVS_ENOMEM (-4)   /* host or device allocation failed                           */
 #define EVS_EIO (-5)      /* file could not be opened / read / written                  */
 #define EVS_EFORMAT (-6)  /* not a flat index.faiss file, or corrupt                    */
-#define EVS_ELIMIT (-7)   /* outside the limits of this build (k > EVS_MAX_K, ...)      */
+#define EVS_ELIMIT (-7)   /* outside the limits of this build (k > option max_k, ...)   */
 #define EVS_ETIMEOUT (-8) /* a collective (row-sharded) search lost a rank: it never arrived, or reported failure */
 
 /* element types of device buffers */
@@ -64,6 +64,7 @@ extern "C" {
 #define EVS_STORE_BF16_F32 1   /* fp32 master + derived bf16 copy; bf16 scan, fp32 canonical rerank */
 
 #define EVS_MAX_K 112          /* app limit is 48 (config.py:29); candidates kept per list: 64 or 128 */
+#define EVS_MAX_K_LARGE 2048   /* ceiling of the option "max_k": searches with EVS_MAX_K < k <= max_k take the large-k path */
 
 typedef struct evs_index evs_index; /* opaque */
 
@@ -204,6 +205,9 @@ EVS_API int evs_index_guard_stats(evs_index* idx, int64_t* reruns, int64_t* unce
  * around rank k: slower, never wrong), the largest |x - bf16(x)|_2 of a row (-1 when the index has no copy), and the number
  * of candidates the last such search re-scored exactly */
 EVS_API int evs_index_shadow_stats(evs_index* idx, int64_t* wide_searches, float* emax, int64_t* last_candidates);
+/* large-k searches (k > EVS_MAX_K) on this handle, and the number of candidates the last one re-scored exactly (the largest
+ * over its queries): rows whose fp32 scan score lies within twice the scan's error bound of the k-th best scan score */
+EVS_API int evs_index_large_k_stats(evs_index* idx, int64_t* searches, int64_t* last_candidates);
 
 /* ---- persistence: <folder>/.clip_index/index.faiss -------------------------------------------
  * evs_index_write       <- faiss.write_index(index, path)           oldapp.py:98
@@ -272,6 +276,10 @@ EVS_API int evs_f32_to_bf16_dev(int device, const float* src_dev, void* dst_dev,
  *                 evs_get_option also reads "tc_fallbacks": queries the HOST re-ran through the GEMV scan because a
  *                 tensor-core candidate buffer overflowed (batches beyond 256 queries; smaller batches repair on the device
  *                 and count in evs_index_guard_stats; should stay 0 on ordinary data).
+ *                 "max_k" (default EVS_MAX_K = 112, range [112, EVS_MAX_K_LARGE = 2048]): the largest k a search, a merge and
+ *                 an exchange accept; searches with k > 112 scan the fp32 rows once per pass of up to 4 queries, keep every
+ *                 row's scan key, select the k-th and re-score exactly every row within twice the scan's error bound of it
+ *                 (exact by construction, DESIGN.md section 2); k <= 112 routes as before whatever the value.
  *                 Unknown names -> EVS_EINVAL.
  * evs_kernel_launches: number of kernels this library has launched in this process.
  * evs_index_time_scan: runs the scan stage alone `iters` times on the index's stream for queries
