@@ -68,7 +68,7 @@ static const int kTcQueryChunk = 4096;  // tensor-core path: queries per launch 
 enum { W_TICKET = 0, W_NEXT_CHUNK = 1, W_GUARD_COUNT0 = 2, W_GUARD_COUNT1 = 3, W_UNCERT = 4 /* u64 */, W_RERUNS = 6 /* u64 */,
        W_MAX_NORM = 8 /* float */, W_SPECIAL = 9, W_BAR = 10 /* 3 words: grid barrier of the in-launch pre-pass */,
        W_EMAX = 13 /* float: largest |x - s c|_2 of a row of the int8 copy */, W_WIDE = 14 /* single-query searches of the int8
-       copy that re-scored more than POOL_KPMAX candidates */, W_LASTC = 15 /* candidates the last of them re-scored */, W_WORDS = 16 };
+       copy whose window held more than 256 candidates */, W_LASTC = 15 /* candidates the last of them re-scored */, W_WORDS = 16 };
 
 struct evs_index {
     int d = 0, device = 0, storage = EVS_STORE_F32;

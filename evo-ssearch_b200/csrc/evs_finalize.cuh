@@ -102,6 +102,49 @@ __device__ __forceinline__ void canon32_dot_multi(const float* const (&x)[R], co
     for (int r = 0; r < R; r++) res[r] = x[r] ? acc[r] : -DBL_MAX;
 }
 
+// Canonical re-score of the candidates keys[0..n) (0 = empty slot): slot c gets its canonical score sc[c], row id[c] (-1 when
+// empty) and rank key ok[c] (0 when empty).  A warp takes R candidates at a time with U values per row and lane in flight
+// (canon32_dot_multi: the order of a lane's additions, hence every score's bits, depend on neither).  Called by every
+// thread of the CTA; the slots are visible after the next barrier.
+template <int R, int UW = 0>
+__device__ __forceinline__ void canon_rescore(const FinalizeParams& p, const u64* keys, int n, double* sc, long long* id, u64* ok,
+                                              const double* qs) {
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
+    const float* xb32 = reinterpret_cast<const float*>(p.xb);
+    auto run = [&](auto ftag) {
+        constexpr bool FAST = decltype(ftag)::value;
+        for (int c = R * warp; c < n; c += R * nwarps) {
+            u64 key[R];
+            long long row[R];
+            const float* xr[R];
+            double sv[R];
+#pragma unroll
+            for (int r = 0; r < R; r++) {
+                key[r] = (c + r < n) ? keys[c + r] : 0ull;
+                row[r] = key[r] ? (long long)key_row(key[r]) : -1;
+                xr[r] = (key[r] && !p.xb_is_bf16) ? xb32 + (size_t)row[r] * p.d : nullptr;
+            }
+            canon32_dot_multi<R, FAST, UW>(xr, qs, p.d, lane, sv);
+            if (p.xb_is_bf16) {
+                const __nv_bfloat16* xb16 = reinterpret_cast<const __nv_bfloat16*>(p.xb);
+#pragma unroll
+                for (int r = 0; r < R; r++) sv[r] = key[r] ? canon32_dot_bf16(xb16 + (size_t)row[r] * p.d, qs, p.d, lane) : -DBL_MAX;
+            }
+            if (lane == 0) {
+#pragma unroll
+                for (int r = 0; r < R; r++)
+                    if (c + r < n) {
+                        sc[c + r] = sv[r];
+                        id[c + r] = row[r];
+                        ok[c + r] = row[r] >= 0 ? score_rank_key(sv[r]) : 0ull;
+                    }
+            }
+        }
+    };
+    if (p.special != nullptr && __ldg(p.special) == 0u) run(std::true_type{});  // CTA-uniform
+    else run(std::false_type{});
+}
+
 // The L per-CTA lists are sorted, so the global top-kp is found without merging them all:
 //   T0 = kp-th largest list HEAD is a lower bound of the kp-th best key (kp heads are >= it), only the
 //   <= kp lists whose head is >= T0 can hold survivors, and only their prefix >= T0 does.  The
@@ -292,55 +335,20 @@ __device__ __forceinline__ void exchange_merge(const Exchange& x, long long qi, 
 // no longer hold anything needed (the exchange merge ranks the gathered partials there).
 // shadow_E > 0 (the pool kernel over bf16 rows, evs_scan.cuh): A holds EVERY row whose scan key is >= cut (1: every row),
 // unsorted, and every other row's scan score is below key_score(cut); the result is exact by construction and the margin is
-// the canonical score of rank k minus (that scan score + E).
+// the canonical score of rank k minus (that scan score + E).  scored: sc / id / ok already hold the canonical re-score of
+// A[0..kp_use) (canon_rescore), which is not repeated.
 template <int MAXR = 4, int UW = 0>  // candidates a warp re-scores at a time at most (kernels held to 64 registers pass 2)
 __device__ __forceinline__ void finalize_rank_emit(const FinalizeParams& p, long long qi, const u64* A, FinalizeShared* sh, double* sc,
                                                    long long* id, u64* ok, const double* qs, unsigned char* scratch, int kp_use = 0,
-                                                   float shadow_E = 0.f, u64 cut = 0ull) {
+                                                   float shadow_E = 0.f, u64 cut = 0ull, bool scored = false) {
     const int t = threadIdx.x, nt = blockDim.x;
-    const int warp = t >> 5, lane = t & 31, nwarps = nt >> 5;
+    const int nwarps = nt >> 5;
     const int kp = kp_use > 0 ? kp_use : p.kp;  // kp_use: only the best kp_use (<= p.kp) entries of A are candidates
     // 4. canonical re-score of the kp candidates: a warp takes two candidates at a time, or four when the CTA has fewer than
     //    kp / 2 warps (the 256-thread CTA of the single-query scan: two rounds instead of four)
-    const float* xb32 = reinterpret_cast<const float*>(p.xb);
-    const bool fastw = p.special != nullptr && __ldg(p.special) == 0u;  // CTA-uniform
-    auto rescore = [&](auto rtag, auto ftag) {
-        constexpr int R = decltype(rtag)::value;
-        constexpr bool FAST = decltype(ftag)::value;
-        for (int c = R * warp; c < kp; c += R * nwarps) {
-            u64 key[R];
-            long long row[R];
-            const float* xr[R];
-            double sv[R];
-#pragma unroll
-            for (int r = 0; r < R; r++) {
-                key[r] = (c + r < kp) ? A[c + r] : 0ull;
-                row[r] = key[r] ? (long long)key_row(key[r]) : -1;
-                xr[r] = (key[r] && !p.xb_is_bf16) ? xb32 + (size_t)row[r] * p.d : nullptr;
-            }
-            canon32_dot_multi<R, FAST, UW>(xr, qs, p.d, lane, sv);
-            if (p.xb_is_bf16) {
-                const __nv_bfloat16* xb16 = reinterpret_cast<const __nv_bfloat16*>(p.xb);
-#pragma unroll
-                for (int r = 0; r < R; r++) sv[r] = key[r] ? canon32_dot_bf16(xb16 + (size_t)row[r] * p.d, qs, p.d, lane) : -DBL_MAX;
-            }
-            if (lane == 0) {
-#pragma unroll
-                for (int r = 0; r < R; r++)
-                    if (c + r < kp) {
-                        sc[c + r] = sv[r];
-                        id[c + r] = row[r];
-                        ok[c + r] = row[r] >= 0 ? score_rank_key(sv[r]) : 0ull;
-                    }
-            }
-        }
-    };
-    if (MAXR < 4 || 2 * nwarps >= kp) {
-        if (fastw) rescore(std::integral_constant<int, 2>{}, std::true_type{});
-        else rescore(std::integral_constant<int, 2>{}, std::false_type{});
-    } else {
-        if (fastw) rescore(std::integral_constant<int, MAXR < 4 ? 2 : 4>{}, std::true_type{});
-        else rescore(std::integral_constant<int, MAXR < 4 ? 2 : 4>{}, std::false_type{});
+    if (!scored) {
+        if (MAXR < 4 || 2 * nwarps >= kp) canon_rescore<2, UW>(p, A, kp, sc, id, ok, qs);
+        else canon_rescore<MAXR < 4 ? 2 : 4, UW>(p, A, kp, sc, id, ok, qs);
     }
     __syncthreads();
     fin_stamp(p, 3);  // re-scored
@@ -399,6 +407,7 @@ __device__ __forceinline__ void finalize_rank_emit(const FinalizeParams& p, long
         }
     }
     __syncthreads();
+    fin_stamp(p, 7);  // ranked
     // 6. padding (-FLT_MAX,-1) / (-DBL_MAX,-1) for the slots no candidate ranked into
     const int nvalid = sh->nvalid;
     for (int r = nvalid + t; r < p.k; r += nt) {

@@ -131,7 +131,7 @@ struct FinalizeParams {
     // makes the result exact
     const float* shadow_emax = nullptr;         // device: largest |x - s c|_2 of a row of the int8 copy (null: the scan is not
                                                 //   bounded this way)
-    unsigned* wide = nullptr;                   // device counter: searches that re-scored more than POOL_KPMAX candidates;
+    unsigned* wide = nullptr;                   // device counter: searches whose window held more than 256 candidates;
                                                 //   wide[1] = the number of candidates the last search re-scored
 };
 

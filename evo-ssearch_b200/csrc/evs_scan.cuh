@@ -467,7 +467,11 @@ constexpr int POOL_COUNT = POOL_SLOTS * POOL_GSTRIDE;   // word of the survivor 
 constexpr int POOL_TICKET = POOL_COUNT + 16;            // ... of the ticket counter
 constexpr int POOL_HDR = POOL_TICKET + 16;              // u64 words before S
 constexpr int POOL_SURV = 2048;         // survivors the last CTA holds in shared memory at a time
-constexpr int POOL_KPMAX = 256;         // candidates the last CTA re-scores in one round (bf16 scan: the 2E window around rank k)
+constexpr int POOL_KPMAX = 256;         // re-score slots of the fp32 / bf16 scans' finalise area; an int8 window of more candidates
+                                        // is counted as wide (evs_index_shadow_stats)
+constexpr int POOL_CMAX = 1024;         // candidates of the int8 copy's window the last CTA re-scores in one pass
+// re-score slots (sc / id / ok) of the pool kernel's finalise area
+__host__ __device__ inline int pool_rescore_slots(const FinalizeParams& f) { return f.shadow_emax != nullptr ? POOL_CMAX : POOL_KPMAX; }
 __host__ __device__ inline size_t pool_finalize_smem_bytes(int kp, int d, int world_k) {
     size_t surv = (size_t)(POOL_SURV + kp) * 8;
     const size_t merge = (size_t)world_k * 24 + 8;  // the fused exchange merge ranks world * k partials in the same place
@@ -510,48 +514,35 @@ __device__ __forceinline__ u64 key_lowered(u64 t, float twoE) {
     return o == 0u ? 1ull : ((u64)o << 32);
 }
 
-// C has more than POOL_KPMAX keys (the int8 copy's window at 10M rows: every search; near-tie bursts): walk the pool in
-// blocks of 128 keys and, whenever the next block may not fit, re-score what was gathered and keep its exact top k (as scan
-// keys: a row re-scores to the same canonical score) in front of the buffer.  The next block's keys are in flight while a
-// block is filtered, and a member's fp32 row is sent to L2 as soon as it joins, so that the re-score rounds wait on L2, not
-// on HBM.  Returns the number of candidates left in cand[] for the final ranking.  Called by all threads.
+// The int8 copy's window C (rule 2) is re-scored by warps of four rows with all 16 values per lane and row in flight (64
+// loads per lane; the row's lines were sent to L2 when it joined C).
+__device__ __forceinline__ void pool_rescore(const FinalizeParams& f, const u64* keys, int n, double* sc, long long* id, u64* ok,
+                                             const double* qs) {
+    canon_rescore<4, 16>(f, keys, n, sc, id, ok, qs);
+}
+__device__ __forceinline__ void prefetch_row_l2(const FinalizeParams& f, u64 key) {
+    const char* row = reinterpret_cast<const char*>(f.xb) + (size_t)key_row(key) * f.d * 4;
+    const int lines = (f.d * 4 + 127) / 128;
+    for (int i = 0; i < lines; i++) asm volatile("prefetch.global.L2 [%0];" ::"l"(row + (size_t)i * 128));
+}
+
+// C has more than POOL_CMAX keys (near-tie bursts): walk the pool in blocks of 128 keys and, whenever the next block may not
+// fit, re-score what was gathered and keep its exact top k (as scan keys: a row re-scores to the same canonical score) in
+// front of the buffer.  The next block's keys are in flight while a block is filtered, and a member's fp32 row is sent to L2
+// as soon as it joins.  Returns the number of candidates left in cand[] (<= POOL_CMAX) for the final re-score and ranking.
+// Called by all threads.
 __device__ __forceinline__ int pool_wide_rounds(const FinalizeParams& f, const u64* S, unsigned m, u64 cut, u64* cand, u64* keep,
                                              double* sc, long long* id, u64* ok, const double* qs, int* s_n) {
-    const int t = threadIdx.x, nt = blockDim.x, warp = t >> 5, lane = t & 31, nwarps = nt >> 5;
-    const float* xb32 = reinterpret_cast<const float*>(f.xb);
-    const bool fastw = f.special != nullptr && __ldg(f.special) == 0u;
-    const int lines = (f.d * 4 + 127) / 128;
+    const int t = threadIdx.x, nt = blockDim.x;
     int fill = 0;  // CTA-uniform
     u64 key = (t < 128 && t < m) ? __ldcg(S + t) : 0ull;
     for (unsigned b0 = 0; b0 < m; b0 += 128) {
         const u64 nkey = (t < 128 && b0 + 128 + t < m) ? __ldcg(S + b0 + 128 + t) : 0ull;
         const bool mem = key != 0ull && key >= cut;
-        if (mem) {
-            const char* row = reinterpret_cast<const char*>(f.xb) + (size_t)key_row(key) * f.d * 4;
-            for (int i = 0; i < lines; i++) asm volatile("prefetch.global.L2 [%0];" ::"l"(row + (size_t)i * 128));
-        }
+        if (mem) prefetch_row_l2(f, key);
         const int nb = __syncthreads_count(mem);
-        if (fill + nb > POOL_KPMAX) {
-            for (int c = 2 * warp; c < fill; c += 2 * nwarps) {
-                long long row[2];
-                const float* xr[2];
-                double sv[2];
-#pragma unroll
-                for (int r = 0; r < 2; r++) {
-                    row[r] = c + r < fill ? (long long)key_row(cand[c + r]) : -1;
-                    xr[r] = row[r] >= 0 ? xb32 + (size_t)row[r] * f.d : nullptr;
-                }
-                if (fastw) canon32_dot_multi<2, true>(xr, qs, f.d, lane, sv);
-                else canon32_dot_multi<2, false>(xr, qs, f.d, lane, sv);
-                if (lane == 0)
-#pragma unroll
-                    for (int r = 0; r < 2; r++)
-                        if (c + r < fill) {
-                            sc[c + r] = sv[r];
-                            id[c + r] = row[r];
-                            ok[c + r] = score_rank_key(sv[r]);
-                        }
-            }
+        if (fill + nb > POOL_CMAX) {
+            pool_rescore(f, cand, fill, sc, id, ok, qs);
             __syncthreads();
             for (int c = t; c < fill; c += nt) {
                 int rank = 0;
@@ -635,7 +626,7 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
         size_t surv_bytes = (size_t)(POOL_SURV + KP) * 8;
         const size_t merge = (size_t)f.x.world * f.k * 24 + 8;
         if (merge > surv_bytes) surv_bytes = (merge + 7) & ~(size_t)7;
-        qs = reinterpret_cast<double*>(smem_raw + sizeof(FinalizeShared) + surv_bytes + 3 * (size_t)POOL_KPMAX * 8);
+        qs = reinterpret_cast<double*>(smem_raw + sizeof(FinalizeShared) + surv_bytes + 3 * (size_t)pool_rescore_slots(f) * 8);
         const float* qf = p.xq + (size_t)p.q0 * p.d;
         for (int i = threadIdx.x; i < p.d; i += blockDim.x) qs[i] = (double)qf[i];
     }
@@ -916,8 +907,8 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
         if (merge > surv_bytes) surv_bytes = (merge + 7) & ~(size_t)7;
     }
     double* sc = reinterpret_cast<double*>(smem_raw + sizeof(FinalizeShared) + surv_bytes);
-    long long* id = reinterpret_cast<long long*>(sc + POOL_KPMAX);
-    u64* ok = reinterpret_cast<u64*>(id + POOL_KPMAX);  // qs (filled at kernel start) follows
+    long long* id = reinterpret_cast<long long*>(sc + pool_rescore_slots(f));
+    u64* ok = reinterpret_cast<u64*>(id + pool_rescore_slots(f));  // qs (filled at kernel start) follows
     if (p.cta_clock && t == 0) {
         unsigned long long* x = p.cta_clock + 2 * gridDim.x;
         x[0] = globaltimer_ns();  // this (the last) CTA holds its ticket
@@ -1091,40 +1082,100 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
     }
     fin_stamp(f, 2);  // the KP best ranked
     const float twoE = s_twoE;
-    if (f.shadow_emax == nullptr) {
+    if (!I8 || f.shadow_emax == nullptr) {  // (only the int8 copy is searched under the bound)
         finalize_rank_emit<(ScanOcc<T, 1, NV>::value >= 4 ? 2 : 4)>(f, p.q0, A, sh, sc, id, ok, qs, reinterpret_cast<unsigned char*>(surv));
     } else {
         // rule 2: C = every pool key >= key_lowered(s~_(k)), read again from the pool (the survivors above were cut at the
-        // plain KP-th best).  Every key C needs is in the pool: rule 1 never dropped one.
+        // plain KP-th best).  Every key C needs is in the pool: rule 1 never dropped one.  A member's fp32 row is sent to
+        // L2 by the thread that finds it, so that all of C's rows are on their way before the re-score starts.  (A window of
+        // more than POOL_CMAX keys is gathered again by pool_wide_rounds, which walks the pool in the same order: the rows
+        // prefetched here are those its first round re-scores.)
         const u64 kth = A[f.k - 1];
         __syncthreads();  // A lives in surv: read before C is gathered there
         const u64 cut = kth ? key_lowered(kth, twoE) : 1ull;  // fewer than k keys: all of them
         u64* cand = surv;
         if (t == 0) s_ns = 0;
         __syncthreads();
-        for (unsigned i = t; i < m; i += nt) {
-            const u64 key = __ldcg(S + i);
-            if (key != 0ull && key >= cut) {
-                const int pos = atomicAdd(&s_ns, 1);
-                if (pos < POOL_KPMAX) cand[pos] = key;
+        constexpr int GU = 8;  // pool keys per thread in flight
+        for (unsigned b0 = 0; b0 < m; b0 += GU * nt) {
+            u64 kg[GU];
+#pragma unroll
+            for (int u = 0; u < GU; u++) {
+                const unsigned i = b0 + t + u * nt;
+                kg[u] = i < m ? __ldcg(S + i) : 0ull;
+            }
+#pragma unroll
+            for (int u = 0; u < GU; u++) {
+                if (kg[u] != 0ull && kg[u] >= cut) {
+                    const int pos = atomicAdd(&s_ns, 1);
+                    if (pos < POOL_CMAX) {
+                        cand[pos] = kg[u];
+                        prefetch_row_l2(f, kg[u]);
+                    }
+                }
             }
         }
         __syncthreads();
+        fin_stamp(f, 5);  // C gathered
         int nc = s_ns;
         if (t == 0 && f.wide) {
             f.wide[1] = (unsigned)nc;
             if (nc > POOL_KPMAX) atomicAdd(f.wide, 1u);
         }
-        if (nc > POOL_KPMAX) nc = pool_wide_rounds(f, S, m, cut, cand, surv + POOL_KPMAX, sc, id, ok, qs, &s_ns);
-        const int lines = (f.d * 4 + 127) / 128;  // the fp32 master rows of C on their way to L2
-        for (int i = t; i < nc * lines; i += nt) {
-            const char* row = reinterpret_cast<const char*>(f.xb) + (size_t)key_row(cand[i / lines]) * f.d * 4 + (size_t)(i % lines) * 128;
-            asm volatile("prefetch.global.L2 [%0];" ::"l"(row));
-        }
+        if (nc > POOL_CMAX) nc = pool_wide_rounds(f, S, m, cut, cand, surv + POOL_CMAX, sc, id, ok, qs, &s_ns);
         for (int i = nc + t; i < KP; i += nt) cand[i] = 0ull;  // at least KP slots, empty ones as padding
         __syncthreads();
+        // every member of C re-scored exactly once, then ranked from these scores
+        const int nk = nc > KP ? nc : KP;
+        pool_rescore(f, cand, nk, sc, id, ok, qs);
+        __syncthreads();
+        fin_stamp(f, 6);  // C re-scored
+        // Only members with a canonical score >= b = fl_down(s~_(k) - E (1 + 2^-10)) are ranked.  The k best-by-scan rows are
+        // in C with exact scores >= s~_(k) - E.  A canonical score is within (d / 32 + 5) 2^-53 |x| |q| of the exact one (fp64
+        // sums of exact products), and E >= 2^-22 (|q - q^| + |q^|) N >= 2^-22 |q| N, so that is below 2^-25 E at d <= 1024
+        // (the argument needs 2^-10 E): at least k members reach b, and every member below b ranks below all of them.
+        // Ranking by counting is quadratic in the members ranked.
+        int nr = nk;
+        if (kth != 0ull && twoE <= FLT_MAX) {
+            const double b = (double)__fsub_rd(key_score(kth), __fmul_ru(twoE, 0.5f * (1.f + 0x1p-10f)));
+            constexpr int PT = POOL_CMAX / 256;  // slots per thread (blockDim.x = 256)
+            u64 ck[PT], co[PT];
+            double cs[PT];
+            long long ci[PT];
+            bool keep[PT];
+#pragma unroll
+            for (int u = 0; u < PT; u++) {
+                const int c = t + u * nt;
+                keep[u] = c < nk && id[c] >= 0 && sc[c] >= b;
+                if (keep[u]) {
+                    ck[u] = cand[c];
+                    cs[u] = sc[c];
+                    ci[u] = id[c];
+                    co[u] = ok[c];
+                }
+            }
+            if (t == 0) s_ns = 0;
+            __syncthreads();
+#pragma unroll
+            for (int u = 0; u < PT; u++)
+                if (keep[u]) {  // ranks by counting do not depend on the order
+                    const int pos = atomicAdd(&s_ns, 1);
+                    cand[pos] = ck[u];
+                    sc[pos] = cs[u];
+                    id[pos] = ci[u];
+                    ok[pos] = co[u];
+                }
+            __syncthreads();
+            nr = s_ns > KP ? s_ns : KP;
+            for (int i = s_ns + t; i < nr; i += nt) {  // empty padding up to KP slots
+                cand[i] = 0ull;
+                id[i] = -1;
+                ok[i] = 0ull;
+            }
+            __syncthreads();
+        }
         finalize_rank_emit<(ScanOcc<T, 1, NV>::value >= 4 ? 2 : 4)>(f, p.q0, cand, sh, sc, id, ok, qs, reinterpret_cast<unsigned char*>(surv),
-                                                                     nc > KP ? nc : KP, twoE * 0.5f, cut);
+                                                                     nr, twoE * 0.5f, cut, true);
     }
     if (p.cta_clock && t == 0) p.cta_clock[2 * gridDim.x + 1] = globaltimer_ns();
 }

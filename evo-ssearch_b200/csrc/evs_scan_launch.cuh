@@ -53,9 +53,9 @@ static ScanParams scan_params(const ScanArgs& a, const ScanPlan* plan) {
 }
 
 // dynamic shared memory of the pool kernel: the warps' buffers or the finalise area, whichever is larger (the pool kernel
-// re-scores up to POOL_KPMAX candidates at a time)
+// re-scores up to pool_rescore_slots candidates at a time)
 static size_t pool_smem_bytes(const ScanPlan* plan, const FinalizeParams& f) {
-    const size_t fs = pool_finalize_smem_bytes(64, f.d, f.x.world * f.k) + 3 * (size_t)(POOL_KPMAX - 64) * 8;
+    const size_t fs = pool_finalize_smem_bytes(64, f.d, f.x.world * f.k) + 3 * (size_t)(pool_rescore_slots(f) - 64) * 8;
     const size_t bufs = (size_t)(plan->threads / 32) * 128 * 8;
     return fs > bufs ? fs : bufs;
 }

@@ -132,9 +132,9 @@ class IndexFlatIP:
         return r.value, u.value
 
     def shadow_stats(self):
-        """``(wide_searches, emax, last_candidates)``: single-query searches of the int8 scan copy that re-scored more
-        candidates than one round holds, the largest ``|x - s c|_2`` of a row of the copy (-1 without a copy), and how many
-        candidates the last such search re-scored exactly."""
+        """``(wide_searches, emax, last_candidates)``: single-query searches of the int8 scan copy whose window held more
+        than 256 candidates, the largest ``|x - s c|_2`` of a row of the copy (-1 without a copy), and how many
+        candidates (the window C) the last search of the copy re-scored exactly."""
         w, e, c = ctypes.c_int64(0), ctypes.c_float(0), ctypes.c_int64(0)
         check(lib().evs_index_shadow_stats(self._h, ctypes.byref(w), ctypes.byref(e), ctypes.byref(c)))
         return w.value, e.value, c.value

@@ -201,9 +201,9 @@ EVS_API int evs_index_last_margins(evs_index* idx, int64_t nq, float* margins_ho
 /* counters of this handle: queries finalised again from the device-side exact re-run, and results that stayed
  * uncertified (more than k' - k rows within the scan error of rank k: ties at fp32 resolution) */
 EVS_API int evs_index_guard_stats(evs_index* idx, int64_t* reruns, int64_t* uncertified);
-/* the bf16 scan copy: single-query searches that re-scored more candidates than one round holds (bursts of near-ties
- * around rank k: slower, never wrong), the largest |x - bf16(x)|_2 of a row (-1 when the index has no copy), and the number
- * of candidates the last such search re-scored exactly */
+/* the int8 scan copy: single-query searches whose window held more than 256 candidates (rows re-scored exactly; at 10M rows
+ * most searches), the largest |x - s c|_2 of a row (-1 when the index has no copy), and the number of candidates (the window
+ * C) the last search of the copy re-scored exactly */
 EVS_API int evs_index_shadow_stats(evs_index* idx, int64_t* wide_searches, float* emax, int64_t* last_candidates);
 /* large-k searches (k > EVS_MAX_K) on this handle, and the number of candidates the last one re-scored exactly (the largest
  * over its queries): rows whose fp32 scan score lies within twice the scan's error bound of the k-th best scan score */

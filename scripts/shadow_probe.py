@@ -82,10 +82,20 @@ def probe(n, d, k, shadow, queries, iters, seed=5):
 def scan_clock_pass(idx, qt, k, scan_bytes, searches=16):
     """Medians over `searches` searches of the loop time (first CTA start to the last CTA's loop end), the loop's rate over
     the bytes it streams, and the tail: last loop end -> the last CTA holds its ticket -> pool read -> the best KP ranked
-    -> re-scored -> results written (evs_scan.cuh: scan_pool_kernel)."""
+    -> re-scored (the final ranking starts) -> results written (evs_scan.cuh: scan_pool_kernel).  Searches of the int8
+    copy also split "ranked -> written" at the finalise stamps 5-7 (finalize stamps 2 -> 5 -> 6 -> 3 -> 7 -> 4):
+      ranked_to_c_gathered_us      the window C read from the pool (its rows sent to L2 as they join);
+      c_gathered_to_c_rescored_us  C re-scored once (with the re-score rounds first when C holds more than 1024 keys).
+                                   Before C was re-scored in one pass: the rounds of 256 only;
+      c_rescored_to_rank_start_us  the ranked members restricted to canonical scores >= b.  Before: the final re-score of
+                                   the kept k and the last round's keys;
+      rank_start_to_c_ranked_us    ranks by counting, results stored;
+      c_ranked_to_written_us       padding, the guard."""
     evs.set_option("scan_clock", 1)
     rec = {"loop_us": [], "end_spread_us": [], "loop_end_to_ticket_us": [], "ticket_to_pool_read_us": [],
            "pool_read_to_ranked_us": [], "ranked_to_rescored_us": [], "rescored_to_written_us": [], "kernel_us": []}
+    window = {"ranked_to_c_gathered_us": [], "c_gathered_to_c_rescored_us": [], "c_rescored_to_rank_start_us": [],
+              "rank_start_to_c_ranked_us": [], "c_ranked_to_written_us": []}
     try:
         for i in range(searches):
             idx.search(qt[i:i + 1], k)
@@ -97,8 +107,15 @@ def scan_clock_pass(idx, qt, k, scan_bytes, searches=16):
                             ("ranked_to_rescored_us", fs[3] - fs[2]), ("rescored_to_written_us", fs[4] - fs[3]),
                             ("kernel_us", fs[4] - t0)):
                 rec[name].append(v / 1e3)
+            if fs[5] and fs[6]:  # the int8 copy's window stamps
+                for name, v in (("ranked_to_c_gathered_us", fs[5] - fs[2]), ("c_gathered_to_c_rescored_us", fs[6] - fs[5]),
+                                ("c_rescored_to_rank_start_us", fs[3] - fs[6]), ("rank_start_to_c_ranked_us", fs[7] - fs[3]),
+                                ("c_ranked_to_written_us", fs[4] - fs[7])):
+                    window[name].append(v / 1e3)
     finally:
         evs.set_option("scan_clock", 0)
+    if window["ranked_to_c_gathered_us"]:
+        rec.update(window)
     out = {name: round(float(np.median(v)), 2) for name, v in rec.items()}
     out["loop_tb_s"] = round(scan_bytes / (out["loop_us"] * 1e-6) / 1e12, 3)
     return {"scan_clock": out}
