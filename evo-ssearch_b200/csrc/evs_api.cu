@@ -1384,19 +1384,13 @@ extern "C" int evs_merge_partials_dev(int device, int nparts, int64_t nq, int64_
     if (nparts <= 0 || nq < 0 || k <= 0) return fail(EVS_EINVAL, "bad nparts/nq/k");
     if (nq == 0) return EVS_OK;
     if (!scores_dev || !ids_dev || !D_dev || !I_dev) return fail(EVS_EINVAL, "NULL buffer");
-    if (k > EVS_MAX_K) {  // large k: up to 8 parts, merged without a shared-memory copy
+    if (k <= EVS_MAX_K) {  // the entries of a query are staged in shared memory
+        if ((size_t)nparts * k * 24 > 200 * 1024) return fail(EVS_ELIMIT, "nparts*k too large for one merge");
+    } else {  // large k: up to 8 parts, ranked in global memory
         const ScanTuning tune = tune_snapshot();
         if (k > tune.max_k) return fail(EVS_ELIMIT, "k = %lld exceeds the option max_k = %d", (long long)k, tune.max_k);
         if (nparts > 8) return fail(EVS_ELIMIT, "a merge for k > %d takes at most 8 parts (got %d)", EVS_MAX_K, nparts);
-        int rc = use_device(device);
-        if (rc) return rc;
-        if (part_stride == 0) part_stride = nq * k;
-        if (part_stride < nq * k) return fail(EVS_EINVAL, "part_stride smaller than nq*k");
-        CU(launch_merge_partials_large(nparts, nq, (int)k, scores_dev, reinterpret_cast<const long long*>(ids_dev), part_stride,
-                                       D_dev, reinterpret_cast<long long*>(I_dev), (cudaStream_t)stream));
-        return EVS_OK;
     }
-    if ((size_t)nparts * k * 24 > 200 * 1024) return fail(EVS_ELIMIT, "nparts*k too large for one merge");
     int rc = use_device(device);
     if (rc) return rc;
     if (part_stride == 0) part_stride = nq * k;
@@ -1713,9 +1707,7 @@ static int search_exchange_enqueue_locked(evs_index* idx, evs_exchange* ex, int6
                                               : search_dev_common(idx, nq, q_dev, k, out, st, tune, pi);
     cudaError_t e = cudaSuccess;
     if (!rc && staged) e = launch_publish_partials(x, nq, (int)k, ex->stage_scores, reinterpret_cast<const long long*>(ex->stage_ids), st);
-    if (!rc && e == cudaSuccess && !one_launch)
-        e = k > EVS_MAX_K ? launch_merge_exchange_large(x, nq, (int)k, D_dev, reinterpret_cast<long long*>(I_dev), st)
-                          : launch_merge_exchange(x, nq, (int)k, D_dev, reinterpret_cast<long long*>(I_dev), st);
+    if (!rc && e == cudaSuccess && !one_launch) e = launch_merge_exchange(x, nq, (int)k, D_dev, reinterpret_cast<long long*>(I_dev), st);
     if (!rc && e != cudaSuccess) rc = fail(EVS_ECUDA, "exchange launch failed: %s", cudaGetErrorString(e));
     ex->seq = x.seq;  // stay in step with the peers whatever happened
     if (rc) {

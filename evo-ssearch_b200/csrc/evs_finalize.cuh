@@ -9,6 +9,7 @@
 //        index.search(q.reshape(1,-1), k) (/root/reference/oldapp.py:2005, :2112).
 #pragma once
 #include <float.h>
+#include <limits.h>
 
 #include <type_traits>
 
@@ -32,6 +33,79 @@ __device__ __forceinline__ u64 score_rank_key(double s) { return f64_to_ordered(
 __device__ __forceinline__ int better_i(u64 oa, long long ia, u64 ob, long long ib) {
     return (int)(oa > ob) | ((int)(oa == ob) & (int)(ia < ib));
 }
+
+// ---- merge of sorted shard partials (one query; merge_partials_kernel, exchange_merge) ----
+// Every part holds the shard's k best sorted by (score desc, id asc), padding (id < 0) at the end.  `at(part, j)` returns
+// entry j of a part (key = score_rank_key(score); any value for padding), so one body serves the entries staged in shared
+// memory, the [part][nq][k] partials in global memory and the flagged exchange entries.
+struct PartEntry {
+    double score;
+    u64 key;
+    long long id;
+};
+// Rank in the merged order of entry (part, r), whose rank key and id are (key, id): r plus, for every other part, the
+// number of its entries that beat it -- a binary search in which padding never beats (it sits at the end).  Asked with
+// key 0 and id LLONG_MAX, a padding entry ranks behind every real one.
+template <class At>
+__device__ __forceinline__ int merge_rank(const At& at, int nparts, int k, int part, int r, u64 key, long long id) {
+    int rank = r;
+    for (int pp = 0; pp < nparts; pp++) {
+        if (pp == part) continue;
+        int lo = 0, hi = k;  // first position in part pp that does not beat (part, r)
+        while (lo < hi) {
+            const int mid = (lo + hi) >> 1;
+            const PartEntry o = at(pp, mid);
+            if (o.id >= 0 && better_i(o.key, o.id, key, id)) lo = mid + 1;
+            else hi = mid;
+        }
+        rank += lo;
+    }
+    return rank;
+}
+// The merge of one query by one CTA: every real entry is written to its rank in D[0..k) / I[0..k) (the query's row) and
+// counted in *nvalid (a shared int, 0 before), then the slots [nvalid, k) are padded.  Called by all threads of the CTA.
+template <class At>
+__device__ __forceinline__ void merge_query(const At& at, int nparts, int k, float* __restrict__ D, long long* __restrict__ I,
+                                            int* nvalid) {
+    for (int e = threadIdx.x; e < nparts * k; e += blockDim.x) {
+        const int part = e / k, r = e - part * k;
+        const PartEntry t = at(part, r);
+        if (t.id < 0) continue;
+        atomicAdd(nvalid, 1);
+        const int rank = merge_rank(at, nparts, k, part, r, t.key, t.id);
+        if (rank < k) {
+            D[rank] = (float)at(part, r).score;
+            I[rank] = t.id;
+        }
+    }
+    __syncthreads();
+    for (int r = *nvalid + threadIdx.x; r < k; r += blockDim.x) {
+        D[r] = -FLT_MAX;
+        I[r] = -1;
+    }
+}
+// The entries of `nparts` parts staged in shared memory: score[m] | id[m] | key[m], m = nparts * k (24 bytes an entry).
+struct StagedParts {
+    double* sc;
+    long long* id;
+    u64* key;
+    int k;
+    __device__ StagedParts(unsigned char* smem, int nparts, int k_) : k(k_) {
+        const int m = nparts * k;
+        sc = reinterpret_cast<double*>(smem);
+        id = reinterpret_cast<long long*>(sc + m);
+        key = reinterpret_cast<u64*>(id + m);
+    }
+    __device__ void put(int e, double s, long long i) const {
+        sc[e] = s;
+        id[e] = i;
+        key[e] = score_rank_key(s);
+    }
+    __device__ PartEntry operator()(int part, int j) const {
+        const int e = part * k + j;
+        return {sc[e], key[e], id[e]};
+    }
+};
 // exact fp32 -> fp64 widening with integer ops for normal numbers (F2F.F64.F32 issues at 1/8 rate)
 __device__ __forceinline__ double widen_f32(float f) {
     const uint32_t u = __float_as_uint(f);
@@ -243,89 +317,78 @@ __device__ __forceinline__ void exchange_store_entry(const Exchange& x, size_t e
     }
 }
 
-// Merge after the peer-store exchange: poll the world*k entries of query `qi` in the LOCAL gather buffer until each carries
-// the flag of search x.seq, then rank them into (D, I).  A rank that never arrives (~10 s watchdog) or that reported failure
-// (poisoned flag) makes the result padding and sets *x.status (host-mapped): stale entries are never merged.
-// Called by all threads of the CTA; smem_raw holds world*k*24 bytes (+ 8); `fail` / `nvalid` are shared ints set to 0 before.
-__device__ __forceinline__ void exchange_merge(const Exchange& x, long long qi, long long nq, int k, float* __restrict__ D,
-                                               long long* __restrict__ I, unsigned char* smem_raw, int* fail, int* nvalid) {
-    (void)nq;
-    const int m = x.world * k;
-    double* sc = reinterpret_cast<double*>(smem_raw);
-    long long* id = reinterpret_cast<long long*>(sc + m);
-    u64* ok = reinterpret_cast<u64*>(id + m);
-    const unsigned char* local = x.peer[x.rank];
+// entry (part, r) of query qi in the LOCAL gather buffer, and its payload
+__device__ __forceinline__ const unsigned char* exchange_entry(const Exchange& x, long long qi, int k, int part, int r) {
+    return x.peer[x.rank] + ((size_t)x.parity * x.world + part) * x.slot_bytes + ((size_t)qi * k + r) * kExchangeEntryBytes;
+}
+__device__ __forceinline__ PartEntry exchange_decode(uint4 a, uint4 b) {
+    const double s = __longlong_as_double((long long)(((unsigned long long)a.z << 32) | a.x));
+    return {s, score_rank_key(s), (long long)(((unsigned long long)b.z << 32) | b.x)};
+}
+// Poll entry (part, r) of query qi until it carries the flag of search x.seq and return its payload in *v.  False when the
+// merge must not happen: that rank reported failure (poisoned flag; *fail raised to 2), it never arrived (~10 s watchdog;
+// *fail raised to 1), or another thread of the CTA already gave up.  `fail` is a shared int of the CTA, 0 before.
+__device__ __forceinline__ bool exchange_wait_entry(const Exchange& x, long long qi, int k, int part, int r, int* fail, PartEntry* v) {
+    const unsigned char* ent = exchange_entry(x, qi, k, part, r);
     const uint32_t want = exchange_flag(x.seq);
-    for (int e = threadIdx.x; e < m; e += blockDim.x) {
-        const int part = e / k, r = e % k;
-        const unsigned char* ent = local + ((size_t)x.parity * x.world + part) * x.slot_bytes + ((size_t)qi * k + r) * kExchangeEntryBytes;
-        const long long t0 = clock64();
-        uint4 a, b;
-        for (;;) {
-            a = ld_volatile_v4(ent);
-            b = ld_volatile_v4(ent + 16);
-            if (a.y == want && a.w == want && b.y == want && b.w == want) break;
-            if (a.y == (want | kExchangePoison) || b.y == (want | kExchangePoison)) {  // that rank failed this search
-                atomicMax(fail, 2);
-                break;
-            }
-            if (*reinterpret_cast<volatile int*>(fail)) break;                // another thread already gave up
-            if (clock64() - t0 > 20000000000ll) {                             // ~10 s: a rank never arrived
-                atomicMax(fail, 1);
-                break;
-            }
-            __nanosleep(20);
+    const long long t0 = clock64();
+    for (;;) {
+        const uint4 a = ld_volatile_v4(ent), b = ld_volatile_v4(ent + 16);
+        if (a.y == want && a.w == want && b.y == want && b.w == want) {
+            *v = exchange_decode(a, b);
+            return true;
         }
-        const double sv = __longlong_as_double((long long)(((unsigned long long)a.z << 32) | a.x));
-        const long long iv = (long long)(((unsigned long long)b.z << 32) | b.x);
-        sc[e] = sv;
-        id[e] = iv;
-        ok[e] = iv >= 0 ? score_rank_key(sv) : 0ull;
+        if (a.y == (want | kExchangePoison) || b.y == (want | kExchangePoison)) {
+            atomicMax(fail, 2);
+            return false;
+        }
+        if (*reinterpret_cast<volatile int*>(fail)) return false;
+        if (clock64() - t0 > 20000000000ll) {
+            atomicMax(fail, 1);
+            return false;
+        }
+        __nanosleep(20);
+    }
+}
+// The result of a merge that did not get every rank's partial: padding in the query's row D[0..k) / I[0..k), and the
+// failure code in *x.status (host-mapped).  Never a merge of what sits in the slots: it may be an older search's partial.
+__device__ __forceinline__ void exchange_fail_result(const Exchange& x, int k, int fail, float* __restrict__ D, long long* __restrict__ I) {
+    for (int r = threadIdx.x; r < k; r += blockDim.x) {
+        D[r] = -FLT_MAX;
+        I[r] = -1;
+    }
+    if (threadIdx.x == 0 && x.status) {
+        *reinterpret_cast<volatile int*>(x.status) = fail;
+        __threadfence_system();
+    }
+}
+
+// Merge after the peer-store exchange: wait for the world*k entries of query `qi` in the local gather buffer, then rank them
+// into (D, I) with merge_query.  STAGED: the entries are copied to smem_raw (world*k*24 bytes) as they arrive, which
+// k <= EVS_MAX_K always fits; otherwise they are ranked where they lie.  Called by all threads of the CTA; `fail` / `nvalid`
+// are shared ints set to 0 before.
+template <bool STAGED>
+__device__ __forceinline__ void exchange_merge(const Exchange& x, long long qi, int k, float* __restrict__ D, long long* __restrict__ I,
+                                               unsigned char* smem_raw, int* fail, int* nvalid) {
+    const int m = x.world * k;
+    const StagedParts staged(smem_raw, x.world, k);
+    for (int e = threadIdx.x; e < m; e += blockDim.x) {
+        PartEntry v;
+        if (exchange_wait_entry(x, qi, k, e / k, e % k, fail, &v) && STAGED) staged.put(e, v.score, v.id);
     }
     __syncthreads();
-    if (*fail) {  // CTA-uniform: report, never merge what sits in the slots (it may be an older search's partial)
-        for (int r = threadIdx.x; r < k; r += blockDim.x) {
-            D[(size_t)qi * k + r] = -FLT_MAX;
-            I[(size_t)qi * k + r] = -1;
-        }
-        if (threadIdx.x == 0 && x.status) {
-            *reinterpret_cast<volatile int*>(x.status) = *fail;
-            __threadfence_system();
-        }
+    D += (size_t)qi * k;
+    I += (size_t)qi * k;
+    if (*fail) {  // CTA-uniform
+        exchange_fail_result(x, k, *fail, D, I);
         return;
     }
-    // every part is sorted by (score desc, id asc) with its padding at the end: the rank of an entry is its own position plus,
-    // for every other part, the number of entries there that beat it -- a binary search per part (7 x 6 steps at 8 ranks
-    // instead of 384 comparisons)
-    for (int e = threadIdx.x; e < m; e += blockDim.x) {
-        if (id[e] < 0) continue;
-        atomicAdd(nvalid, 1);
-        const int part = e / k;
-        const long long it = id[e];
-        const u64 ot = ok[e];
-        int rank = e - part * k;
-        for (int pp = 0; pp < x.world; pp++) {
-            if (pp == part) continue;
-            const int base = pp * k;
-            int lo = 0, hi = k;  // first position in part pp that does NOT beat e
-            while (lo < hi) {
-                const int mid = (lo + hi) >> 1;
-                const bool beats = id[base + mid] >= 0 && better_i(ok[base + mid], id[base + mid], ot, it);
-                if (beats) lo = mid + 1;
-                else hi = mid;
-            }
-            rank += lo;
-        }
-        if (rank < k) {
-            D[(size_t)qi * k + rank] = (float)sc[e];
-            I[(size_t)qi * k + rank] = it;
-        }
-    }
-    __syncthreads();
-    for (int r = *nvalid + threadIdx.x; r < k; r += blockDim.x) {
-        D[(size_t)qi * k + r] = -FLT_MAX;
-        I[(size_t)qi * k + r] = -1;
-    }
+    const auto in_place = [&](int part, int j) {
+        const unsigned char* ent = exchange_entry(x, qi, k, part, j);
+        return exchange_decode(ld_volatile_v4(ent), ld_volatile_v4(ent + 16));
+    };
+    if (STAGED) merge_query(staged, x.world, k, D, I, nvalid);
+    else merge_query(in_place, x.world, k, D, I, nvalid);
 }
 
 // Second half of the finalise, shared by every candidate source (per-CTA lists: finalize_query; the survivor pool of the
@@ -449,8 +512,7 @@ __device__ __forceinline__ void finalize_rank_emit(const FinalizeParams& p, long
         if (p.x.merge_D != nullptr) {
             // single-query search fused into the scan kernel: the same CTA waits for the peers' partials and merges
             __syncthreads();
-            exchange_merge(p.x, p.x.q_off + qi, p.x.nq_total, p.k, p.x.merge_D, p.x.merge_I, scratch,
-                           &sh->fail, &sh->nvalid);
+            exchange_merge<true>(p.x, p.x.q_off + qi, p.k, p.x.merge_D, p.x.merge_I, scratch, &sh->fail, &sh->nvalid);
         }
     }
 }

@@ -320,8 +320,5 @@ struct LargeKArgs {
 size_t large_k_state_bytes(int qpp);  // hist + st of a pass (zeroed before it)
 cudaError_t launch_large_k_scan(const LargeKArgs& a, cudaStream_t st);
 cudaError_t launch_large_k_rest(const LargeKArgs& a, int sm_count, cudaStream_t st);
-cudaError_t launch_merge_partials_large(int nparts, long long nq, int k, const double* scores, const long long* ids,
-                                        long long part_stride, float* D, long long* I, cudaStream_t st);
-cudaError_t launch_merge_exchange_large(const Exchange& x, long long nq, int k, float* D, long long* I, cudaStream_t st);
 
 }  // namespace evs

@@ -3,7 +3,9 @@
 //   scan launchers       score + fused top-k' selection               (evs_scan.cuh)
 //   finalize_kernel      merge the per-CTA lists of one query, re-score the k' candidates in the
 //                        canonical fp64 order, rank, emit (D,I) or a shard partial
-//   merge_partials_kernel  G-way merge of shard partials after the NCCL all-gather
+//   merge_partials_kernel  G-way merge of shard partials after the NCCL all-gather, every k
+//   merge_exchange_kernel  the same merge after the peer-store exchange, behind its wait protocol, every k (both rank
+//                        with merge_rank, evs_finalize.cuh)
 //   l2_normalize_kernel  oldapp.py:35/43/51, 128-bit coalesced, in place
 //   f32_to_bf16_kernel   the one-time database layout kernel
 //   synth_fill_kernel    counter-based synthetic embeddings (bit-identical to oracle/orc_synth_fill)
@@ -74,13 +76,13 @@ __global__ void publish_poison_kernel(Exchange x, long long count) {
 
 // =============================================================================================
 // merge after the peer-store exchange: poll the entries of this search in the LOCAL gather buffer until every
-// shard's have arrived, then rank the world*k partials of each query.  grid = nq, block = 256.
+// shard's have arrived, then rank the world*k partials of each query (exchange_merge).  grid = nq, block = 256 for
+// k <= EVS_MAX_K (entries staged in shared memory), 1024 above (ranked in the gather buffer).
 // Every rank runs this kernel on its own GPU; the entries are written by the other GPUs' finalise / publish kernels.
 // A rank that never arrives (~10 s watchdog) or that reported failure (poisoned flag) makes the whole result
 // padding (-FLT_MAX, -1) and sets *x.status (host-mapped): stale slots are never merged.
 // =============================================================================================
-__global__ void __launch_bounds__(256) merge_exchange_kernel(Exchange x, long long nq, int k, float* __restrict__ D,
-                                                            long long* __restrict__ I) {
+__global__ void __launch_bounds__(1024) merge_exchange_kernel(Exchange x, int k, float* __restrict__ D, long long* __restrict__ I) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ int s_nvalid, s_fail;
     if (threadIdx.x == 0) {
@@ -90,11 +92,16 @@ __global__ void __launch_bounds__(256) merge_exchange_kernel(Exchange x, long lo
     asm volatile("griddepcontrol.wait;" ::: "memory");  // launched programmatically behind this rank's finalise / publish kernel
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     __syncthreads();
-    exchange_merge(x, blockIdx.x, nq, k, D, I, smem_raw, &s_fail, &s_nvalid);
+    if (k <= EVS_MAX_K) exchange_merge<true>(x, blockIdx.x, k, D, I, smem_raw, &s_fail, &s_nvalid);
+    else exchange_merge<false>(x, blockIdx.x, k, D, I, smem_raw, &s_fail, &s_nvalid);
 }
 
 // =============================================================================================
-// merge of shard partials: scores/ids laid out [part][nq][k]; grid = nq, block = 256
+// merge of shard partials: scores/ids laid out [part][nq][k].  k <= EVS_MAX_K: grid = nq, the query's nparts*k entries
+// staged in shared memory and merged by merge_query.  Larger k (nparts*k*24 bytes outgrow shared memory): grid = (entry
+// blocks, query stride), one thread per entry ranked straight from global memory by merge_rank; with the query spread over
+// CTAs nothing counts the real entries, so the padding entries of part 0 rank themselves behind all of them and fill the
+// slots [nvalid, k) (a later part's padding ranks behind part 0's k entries).  block = 256.
 // =============================================================================================
 __global__ void __launch_bounds__(256) merge_partials_kernel(int nparts, long long nq, int k,
                                                             const double* __restrict__ scores,
@@ -102,39 +109,38 @@ __global__ void __launch_bounds__(256) merge_partials_kernel(int nparts, long lo
                                                             float* __restrict__ D, long long* __restrict__ I) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int m = nparts * k;
-    double* sc = reinterpret_cast<double*>(smem_raw);
-    long long* id = reinterpret_cast<long long*>(sc + m);
-    u64* ok = reinterpret_cast<u64*>(id + m);  // integer rank keys (see score_rank_key)
-    __shared__ int s_nvalid;
-    const long long qi = blockIdx.x;
-    if (threadIdx.x == 0) s_nvalid = 0;
-    for (int e = threadIdx.x; e < m; e += blockDim.x) {
-        int part = e / k, r = e % k;
-        size_t src = (size_t)part * part_stride + (size_t)qi * k + r;
-        const double sv = scores[src];
-        const long long iv = ids[src];
-        sc[e] = sv;
-        id[e] = iv;
-        ok[e] = iv >= 0 ? score_rank_key(sv) : 0ull;
-    }
-    __syncthreads();
-    for (int e = threadIdx.x; e < m; e += blockDim.x) {
-        if (id[e] < 0) continue;
-        atomicAdd(&s_nvalid, 1);
-        const double st = sc[e];
-        const long long it = id[e];
-        const u64 ot = ok[e];
-        int rank = 0;
-        for (int j = 0; j < m; j++) rank += better_i(ok[j], id[j], ot, it) & (int)(id[j] >= 0);
-        if (rank < k) {
-            D[(size_t)qi * k + rank] = (float)st;
-            I[(size_t)qi * k + rank] = it;
+    if (k <= EVS_MAX_K) {
+        __shared__ int s_nvalid;
+        const long long qi = blockIdx.x;
+        const StagedParts staged(smem_raw, nparts, k);
+        if (threadIdx.x == 0) s_nvalid = 0;
+        for (int e = threadIdx.x; e < m; e += blockDim.x) {
+            const size_t src = (size_t)(e / k) * part_stride + (size_t)qi * k + e % k;
+            staged.put(e, scores[src], ids[src]);
         }
+        __syncthreads();
+        merge_query(staged, nparts, k, D + (size_t)qi * k, I + (size_t)qi * k, &s_nvalid);
+        return;
     }
-    __syncthreads();
-    for (int r = s_nvalid + threadIdx.x; r < k; r += blockDim.x) {
-        D[(size_t)qi * k + r] = -FLT_MAX;
-        I[(size_t)qi * k + r] = -1;
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= m) return;
+    const int part = e / k, r = e - part * k;
+    // not unrolled: the unrolled loop's trip count costs a 64-bit division call and a spill
+#pragma unroll 1
+    for (long long qi = blockIdx.y; qi < nq; qi += gridDim.y) {
+        const auto in_place = [&](int pp, int j) {
+            const size_t o = (size_t)pp * part_stride + (size_t)qi * k + j;
+            const double s = scores[o];
+            return PartEntry{s, score_rank_key(s), ids[o]};
+        };
+        const PartEntry t = in_place(part, r);
+        const bool pad = t.id < 0;
+        if (pad && part > 0) continue;
+        const int rank = merge_rank(in_place, nparts, k, part, r, pad ? 0ull : t.key, pad ? LLONG_MAX : t.id);
+        if (rank < k) {
+            D[(size_t)qi * k + rank] = pad ? -FLT_MAX : (float)t.score;
+            I[(size_t)qi * k + rank] = pad ? -1 : t.id;
+        }
     }
 }
 
@@ -599,11 +605,17 @@ cudaError_t launch_synth_fill(float* out, long long n, int d, unsigned long long
 cudaError_t launch_merge_partials(int nparts, long long nq, int k, const double* scores, const long long* ids,
                                   long long part_stride, float* D, long long* I, cudaStream_t st) {
     if (nq <= 0) return cudaSuccess;
-    size_t smem = (size_t)nparts * k * 24;
-    if (smem > 200 * 1024) return cudaErrorInvalidValue;
-    if (smem > 48 * 1024)
-        cudaFuncSetAttribute(merge_partials_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    merge_partials_kernel<<<(unsigned)nq, 256, smem, st>>>(nparts, nq, k, scores, ids, part_stride, D, I);
+    if (k <= EVS_MAX_K) {
+        const size_t smem = (size_t)nparts * k * 24;
+        if (smem > 200 * 1024) return cudaErrorInvalidValue;
+        if (smem > 48 * 1024)
+            cudaFuncSetAttribute(merge_partials_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        merge_partials_kernel<<<(unsigned)nq, 256, smem, st>>>(nparts, nq, k, scores, ids, part_stride, D, I);
+    } else {
+        const unsigned gx = (unsigned)((nparts * k + 255) / 256);
+        const unsigned gy = (unsigned)(nq < 65535 ? nq : 65535);
+        merge_partials_kernel<<<dim3(gx, gy), 256, 0, st>>>(nparts, nq, k, scores, ids, part_stride, D, I);
+    }
     EVS_LAUNCH_CHECK();
     return cudaSuccess;
 }
@@ -629,11 +641,10 @@ cudaError_t launch_publish_poison(const Exchange& x, cudaStream_t st) {
 
 cudaError_t launch_merge_exchange(const Exchange& x, long long nq, int k, float* D, long long* I, cudaStream_t st) {
     if (nq <= 0) return cudaSuccess;
-    size_t smem = (size_t)x.world * k * 24;
-    if (smem > 200 * 1024) return cudaErrorInvalidValue;
-    if (smem > 48 * 1024)
-        cudaFuncSetAttribute(merge_exchange_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    cudaError_t le = launch_pdl(merge_exchange_kernel, dim3((unsigned)nq), dim3(256), smem, st, x, nq, k, D, I);
+    if (x.world < 1 || x.world > 8) return cudaErrorInvalidValue;
+    const bool staged = k <= EVS_MAX_K;
+    const size_t smem = staged ? (size_t)x.world * k * 24 : 0;  // at most 8 * 112 * 24 bytes: no opt-in needed
+    cudaError_t le = launch_pdl(merge_exchange_kernel, dim3((unsigned)nq), dim3(staged ? 256 : 1024), smem, st, x, k, D, I);
     g_kernel_launches.fetch_add(1);
     if (le != cudaSuccess) return le;
     return cudaGetLastError();

@@ -510,166 +510,4 @@ cudaError_t launch_large_k_rest(const LargeKArgs& a, int sm_count, cudaStream_t 
     return cudaGetLastError();
 }
 
-// ---------------------------------------------------------------------------------------------
-// merges of sorted shard partials for large k: the rank of an entry is its position in its own part plus, for every other
-// part, the number of entries there that beat it -- a binary search per part, read from global memory (nparts * k * 24
-// bytes do not fit shared memory at k = 2048)
-// ---------------------------------------------------------------------------------------------
-// partials [part][nq][k] (evs_merge_partials_dev); grid = (entry blocks, query stride), nparts <= 8
-__global__ void __launch_bounds__(256) merge_partials_large_kernel(int nparts, long long nq, int k, const double* __restrict__ scores,
-                                                                  const long long* __restrict__ ids, long long part_stride,
-                                                                  float* __restrict__ D, long long* __restrict__ I) {
-    const int e = blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= nparts * k) return;
-    const int part = e / k, r = e % k;
-    for (long long qi = blockIdx.y; qi < nq; qi += gridDim.y) {
-        auto at = [&](int p, int j) { return (size_t)p * part_stride + (size_t)qi * k + j; };
-        int valid[8];
-        int total = 0;
-        for (int p = 0; p < nparts; p++) {  // padding (id < 0) sits at the end of every part
-            int lo = 0, hi = k;
-            while (lo < hi) {
-                const int mid = (lo + hi) >> 1;
-                if (ids[at(p, mid)] >= 0) lo = mid + 1;
-                else hi = mid;
-            }
-            valid[p] = lo;
-            total += lo;
-        }
-        if (e < k && e >= total) {
-            D[(size_t)qi * k + e] = -FLT_MAX;
-            I[(size_t)qi * k + e] = -1;
-        }
-        if (r >= valid[part]) continue;
-        const double sv = scores[at(part, r)];
-        const long long it = ids[at(part, r)];
-        const u64 ot = score_rank_key(sv);
-        int rank = r;
-        for (int p = 0; p < nparts; p++) {
-            if (p == part) continue;
-            int lo = 0, hi = valid[p];
-            while (lo < hi) {
-                const int mid = (lo + hi) >> 1;
-                if (better_i(score_rank_key(scores[at(p, mid)]), ids[at(p, mid)], ot, it)) lo = mid + 1;
-                else hi = mid;
-            }
-            rank += lo;
-        }
-        if (rank < k) {
-            D[(size_t)qi * k + rank] = (float)sv;
-            I[(size_t)qi * k + rank] = it;
-        }
-    }
-}
-
-cudaError_t launch_merge_partials_large(int nparts, long long nq, int k, const double* scores, const long long* ids,
-                                        long long part_stride, float* D, long long* I, cudaStream_t st) {
-    if (nq <= 0) return cudaSuccess;
-    if (nparts < 1 || nparts > 8) return cudaErrorInvalidValue;
-    const unsigned gx = (unsigned)((nparts * k + 255) / 256);
-    const unsigned gy = (unsigned)(nq < 65535 ? nq : 65535);
-    merge_partials_large_kernel<<<dim3(gx, gy), 256, 0, st>>>(nparts, nq, k, scores, ids, part_stride, D, I);
-    EVS_LAUNCH_CHECK();
-    return cudaSuccess;
-}
-
-// the peer-store exchange (evs_internal.h: Exchange) for large k: poll every entry of query blockIdx.x in the local gather
-// buffer, then rank them as above.  A rank that never arrives or reported failure makes the result padding, as in
-// exchange_merge.  grid = nq, block = 1024.
-__device__ __forceinline__ const unsigned char* lk_entry(const Exchange& x, long long qi, int k, int part, int r) {
-    return x.peer[x.rank] + ((size_t)x.parity * x.world + part) * x.slot_bytes + ((size_t)qi * k + r) * kExchangeEntryBytes;
-}
-__device__ __forceinline__ void lk_read_entry(const unsigned char* ent, double* s, long long* id) {
-    const uint4 a = ld_volatile_v4(ent), b = ld_volatile_v4(ent + 16);
-    *s = __longlong_as_double((long long)(((unsigned long long)a.z << 32) | a.x));
-    *id = (long long)(((unsigned long long)b.z << 32) | b.x);
-}
-
-__global__ void __launch_bounds__(1024) merge_exchange_large_kernel(Exchange x, long long nq, int k, float* __restrict__ D,
-                                                                   long long* __restrict__ I) {
-    __shared__ int s_fail, s_valid[8];
-    const long long qi = blockIdx.x;
-    const int t = threadIdx.x, m = x.world * k;
-    if (t == 0) s_fail = 0;
-    if (t < 8) s_valid[t] = k;
-    lk_wait();
-    __syncthreads();
-    const uint32_t want = exchange_flag(x.seq);
-    for (int e = t; e < m; e += blockDim.x) {
-        const int part = e / k, r = e % k;
-        const unsigned char* ent = lk_entry(x, qi, k, part, r);
-        const long long t0 = clock64();
-        uint4 a, b;
-        for (;;) {
-            a = ld_volatile_v4(ent);
-            b = ld_volatile_v4(ent + 16);
-            if (a.y == want && a.w == want && b.y == want && b.w == want) break;
-            if (a.y == (want | kExchangePoison) || b.y == (want | kExchangePoison)) {  // that rank failed this search
-                atomicMax(&s_fail, 2);
-                break;
-            }
-            if (*reinterpret_cast<volatile int*>(&s_fail)) break;  // another thread already gave up
-            if (clock64() - t0 > 20000000000ll) {                   // ~10 s: a rank never arrived
-                atomicMax(&s_fail, 1);
-                break;
-            }
-            __nanosleep(20);
-        }
-        if ((long long)(((unsigned long long)b.z << 32) | b.x) < 0) atomicMin(&s_valid[part], r);
-    }
-    __syncthreads();
-    if (s_fail) {  // CTA-uniform: report, never merge what sits in the slots
-        for (int r = t; r < k; r += blockDim.x) {
-            D[(size_t)qi * k + r] = -FLT_MAX;
-            I[(size_t)qi * k + r] = -1;
-        }
-        if (t == 0 && x.status) {
-            *reinterpret_cast<volatile int*>(x.status) = s_fail;
-            __threadfence_system();
-        }
-        return;
-    }
-    int total = 0;
-    for (int p = 0; p < x.world; p++) total += s_valid[p];
-    for (int r = total + t; r < k; r += blockDim.x) {
-        D[(size_t)qi * k + r] = -FLT_MAX;
-        I[(size_t)qi * k + r] = -1;
-    }
-    for (int e = t; e < m; e += blockDim.x) {
-        const int part = e / k, r = e % k;
-        if (r >= s_valid[part]) continue;
-        double sv;
-        long long it;
-        lk_read_entry(lk_entry(x, qi, k, part, r), &sv, &it);
-        const u64 ot = score_rank_key(sv);
-        int rank = r;
-        for (int p = 0; p < x.world; p++) {
-            if (p == part) continue;
-            int lo = 0, hi = s_valid[p];
-            while (lo < hi) {
-                const int mid = (lo + hi) >> 1;
-                double ps;
-                long long pid;
-                lk_read_entry(lk_entry(x, qi, k, p, mid), &ps, &pid);
-                if (better_i(score_rank_key(ps), pid, ot, it)) lo = mid + 1;
-                else hi = mid;
-            }
-            rank += lo;
-        }
-        if (rank < k) {
-            D[(size_t)qi * k + rank] = (float)sv;
-            I[(size_t)qi * k + rank] = it;
-        }
-    }
-}
-
-cudaError_t launch_merge_exchange_large(const Exchange& x, long long nq, int k, float* D, long long* I, cudaStream_t st) {
-    if (nq <= 0) return cudaSuccess;
-    if (x.world < 1 || x.world > 8) return cudaErrorInvalidValue;
-    cudaError_t le = launch_pdl(merge_exchange_large_kernel, dim3((unsigned)nq), dim3(1024), 0, st, x, nq, k, D, I);
-    g_kernel_launches.fetch_add(1);
-    if (le != cudaSuccess) return le;
-    return cudaGetLastError();
-}
-
 }  // namespace evs
