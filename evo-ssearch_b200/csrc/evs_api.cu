@@ -1260,8 +1260,8 @@ static int search_enqueue_locked(evs_index* idx, int64_t nq, const float* q_dev,
                 a.ticket = idx->words + W_TICKET;
                 if (tune.pool_select && kp == 64) {
                     // under the lowered thresholds of the int8 scan a near-tie burst may send any number of keys to the pool:
-                    // room for one per row (each row's key enters the pool at most once)
-                    const size_t need = scan_pool_words(plan) + (shadow ? (size_t)idx->ntotal : 0);
+                    // room for one per row (each row's key enters the pool at most once), then the window pass's list
+                    const size_t need = scan_pool_words(plan) + (shadow ? (size_t)idx->ntotal + scan_pool_window_words() : 0);
                     if (idx->pool_cap < need) {  // (re)allocated zeroed; every search's last CTA leaves it zeroed
                         if (idx->pool) CU(cudaFree(idx->pool));
                         idx->pool = nullptr;
@@ -1288,7 +1288,7 @@ static int search_enqueue_locked(evs_index* idx, int64_t nq, const float* q_dev,
                     a.chunk_groups = tune.scan_chunk_groups > 0 ? tune.scan_chunk_groups : 2;
                 }
                 if (tune.scan_clock) {
-                    if ((rc = ensure_dev(&idx->cta_clock, &idx->cta_clock_cap, (size_t)plan.grid * 2 + 16))) return rc;
+                    if ((rc = ensure_dev(&idx->cta_clock, &idx->cta_clock_cap, (size_t)plan.grid * 2 + 24))) return rc;
                     idx->cta_clock_n = plan.grid;
                     a.cta_clock = idx->cta_clock;
                     f.dbg = idx->cta_clock + (size_t)plan.grid * 2 + 8;
@@ -1915,8 +1915,10 @@ extern "C" int evs_index_scan_clocks(evs_index* idx, uint64_t* out_host, int64_t
     if (cap_ctas < idx->cta_clock_n) return fail(EVS_EINVAL, "buffer holds %lld CTAs, need %d", (long long)cap_ctas, idx->cta_clock_n);
     if (idx->have_last_stream) CU(cudaStreamSynchronize(idx->last_stream));
     CU(cudaMemcpy(out_host, idx->cta_clock, (size_t)idx->cta_clock_n * 16, cudaMemcpyDeviceToHost));
-    if (cap_ctas >= idx->cta_clock_n + 8)  // then the last CTA's own stamps (8) and the phases of its finalise (8)
-        CU(cudaMemcpy(out_host + 2 * (size_t)idx->cta_clock_n, idx->cta_clock + 2 * (size_t)idx->cta_clock_n, 128, cudaMemcpyDeviceToHost));
+    // then the last CTA's own stamps (8) and the phases of its finalise: 8 with room for n + 8 CTAs, 16 with room for n + 12
+    if (cap_ctas >= idx->cta_clock_n + 8)
+        CU(cudaMemcpy(out_host + 2 * (size_t)idx->cta_clock_n, idx->cta_clock + 2 * (size_t)idx->cta_clock_n,
+                      cap_ctas >= idx->cta_clock_n + 12 ? 192 : 128, cudaMemcpyDeviceToHost));
     return EVS_OK;
 }
 

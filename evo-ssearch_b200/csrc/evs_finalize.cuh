@@ -296,6 +296,10 @@ __device__ __forceinline__ void fin_stamp(const FinalizeParams& p, int slot) {
         p.dbg[slot] = t;
     }
 }
+// a count beside the stamps (slots 11-13: the int8 window pass)
+__device__ __forceinline__ void fin_note(const FinalizeParams& p, int slot, unsigned long long v) {
+    if (p.dbg != nullptr && threadIdx.x == 0) p.dbg[slot] = v;
+}
 
 // ---- exchange entries (evs_internal.h: Exchange): payload and flag in the same 16-byte stores ----
 __device__ __forceinline__ uint32_t exchange_flag(unsigned long long seq) { return (uint32_t)(seq & 0x7FFFFFFFull); }

@@ -253,6 +253,7 @@ int max_queries_per_pass(int d, int is_bf16);
 cudaError_t launch_scan(const ScanArgs& a, ScanPlan* plan, cudaStream_t st);
 size_t scan_pool_key_slots(size_t pool_words);  // key slots behind the header of a pool of that many words
 size_t scan_pool_words(const ScanPlan& plan);  // u64 words of the pool a fused single-query launch of this plan needs (zeroed once)
+size_t scan_pool_window_words();  // u64 words of the int8 window pass's list W, behind the pool's room for one key per row
 cudaError_t launch_finalize(const FinalizeParams& p, long long nq, cudaStream_t st);
 size_t finalize_smem_bytes_host(int L, int kp, int d);
 cudaError_t launch_publish_partials(const Exchange& x, long long nq, int k, const double* scores, const long long* ids,

@@ -749,6 +749,7 @@ cudaError_t plan_scan(long long n, int d, int elem, int kp, int nq_pass, int sm_
 
 size_t scan_pool_key_slots(size_t pool_words) { return pool_words > (size_t)POOL_HDR ? pool_words - (size_t)POOL_HDR : 0; }
 size_t scan_pool_words(const ScanPlan& plan) { return (size_t)POOL_HDR + (size_t)plan.grid * (plan.threads / 32) * 128; }
+size_t scan_pool_window_words() { return 3 * (size_t)POOL_CMAX; }
 
 cudaError_t launch_scan(const ScanArgs& a, ScanPlan* plan, cudaStream_t st) {
     if (a.n <= 0) return cudaErrorInvalidValue;

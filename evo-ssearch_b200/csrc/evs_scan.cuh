@@ -470,6 +470,21 @@ constexpr int POOL_SURV = 2048;         // survivors the last CTA holds in share
 constexpr int POOL_KPMAX = 256;         // re-score slots of the fp32 / bf16 scans' finalise area; an int8 window of more candidates
                                         // is counted as wide (evs_index_shadow_stats)
 constexpr int POOL_CMAX = 1024;         // candidates of the int8 copy's window the last CTA re-scores in one pass
+// The int8 copy's window pass (scan_pool_kernel, DESIGN.md section 2 rule 2): the CTAs holding the POOL_HELPERS tickets
+// before the last one stay and re-score the pool's window W with the last CTA, slices of POOL_SLICE keys at a time.
+// Its header words share the ticket's line (free there in both pool kernels) and are zero between searches; the list W
+// (key, canonical score bits, rank key per entry, POOL_CMAX entries) lies behind the survivor pool's room
+// (scan_pool_window_words).
+constexpr int POOL_HELPERS = 63;
+constexpr int POOL_SLICE = 256;         // = blockDim.x: one key per thread
+constexpr int POOL_WGO = POOL_TICKET + 1;     // the pass opened: m + 1 (keys in the pool) | the high word of cutW << 32
+constexpr int POOL_WCLAIM = POOL_TICKET + 2;  // slices claimed
+constexpr int POOL_WDONE = POOL_TICKET + 3;   // slices finished
+constexpr int POOL_WN = POOL_TICKET + 4;      // entries reserved in W
+constexpr int POOL_WOVER = POOL_TICKET + 5;   // 1: W overflowed
+constexpr int POOL_WLEFT = POOL_TICKET + 6;   // helpers that have left
+static_assert(POOL_WLEFT < POOL_HDR, "window header outside the pool header");
+static_assert(2 * POOL_CMAX <= POOL_SURV, "the last CTA ranks W's top entries behind W in the survivor buffer");
 // re-score slots (sc / id / ok) of the pool kernel's finalise area
 __host__ __device__ inline int pool_rescore_slots(const FinalizeParams& f) { return f.shadow_emax != nullptr ? POOL_CMAX : POOL_KPMAX; }
 __host__ __device__ inline size_t pool_finalize_smem_bytes(int kp, int d, int world_k) {
@@ -584,6 +599,103 @@ __device__ __forceinline__ void pool_publish(u64* G, u64 key, u64 ga, u64 gb) {
     const u64 va = __shfl_sync(0xffffffffu, ga, slot & 31), vb = __shfl_sync(0xffffffffu, gb, slot & 31);
     const u64 cur = slot < 32 ? va : vb;
     if (key != 0ull && key > cur) atomicMax(reinterpret_cast<unsigned long long*>(G + (size_t)slot * POOL_GSTRIDE), (unsigned long long)key);
+}
+
+// (polls read relaxed and fence once after the wait: an acquire load invalidates the SM's L1 on every poll)
+__device__ __forceinline__ unsigned ld_relaxed_gpu_u32(const unsigned* p) {
+    unsigned v;
+    asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ u64 ld_relaxed_gpu_u64(const u64* p) {
+    u64 v;
+    asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ void st_relaxed_gpu_u64(u64* p, u64 v) {
+    asm volatile("st.relaxed.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
+}
+// thread 0 waits until *p >= want (the words it waits on are raised by CTAs that are running), then fences: what the
+// raisers stored before their fence and increment is visible after it
+__device__ __forceinline__ void pool_wait_count(const unsigned* p, unsigned want) {
+    unsigned ns = 32;
+    while (ld_relaxed_gpu_u32(p) < want) {
+        __nanosleep(ns);
+        ns = ns < 256 ? 2 * ns : ns;
+    }
+    __threadfence();
+}
+
+// The window pass of the int8 copy: claim slices of POOL_SLICE pool keys until none are left, gather the keys >= cutW of
+// consecutive claims until they fill one re-score round (8 warps x 4 rows), re-score them (canon_rescore: the same bits in
+// every CTA) and append (key, score, rank key) to W; the slices gathered count as done once their entries are visible.
+// (Only ~12 keys per slice pass cutW: a round per slice made a participant that finds every slice left alone -- no helper
+// joined -- 4x slower than the pool read.)  When W overflows, the claimant takes every slice left at once and the last CTA
+// falls back to the pool read.  Called by all threads of a participant; cand / sc / id / ok: POOL_SLICE + 32 slots of its
+// finalise area; *s_n = 0 before.  Returns the slices this CTA took.
+__device__ __forceinline__ unsigned pool_window_pass(const FinalizeParams& f, u64* pool, u64* W, const u64* S, unsigned m, u64 cutW,
+                                                     u64* cand, double* sc, long long* id, u64* ok, const double* qs, int* s_n,
+                                                     unsigned* s_sl) {
+    constexpr int ROUND = 32;  // rows of one canon_rescore<4> round of 8 warps
+    unsigned* claim = reinterpret_cast<unsigned*>(pool + POOL_WCLAIM);
+    unsigned* done = reinterpret_cast<unsigned*>(pool + POOL_WDONE);
+    unsigned* wn = reinterpret_cast<unsigned*>(pool + POOL_WN);
+    unsigned* over = reinterpret_cast<unsigned*>(pool + POOL_WOVER);
+    const int t = threadIdx.x;
+    const unsigned nslices = (m + POOL_SLICE - 1) / POOL_SLICE;
+    unsigned taken = 0, pend = 0;  // CTA-uniform: slices claimed, of them not yet counted done
+    for (;;) {
+        if (t == 0) {
+            unsigned sl = atomicAdd(claim, 1u);
+            if (sl < nslices && __ldcg(over)) {  // W overflowed: close the pass (every slice is counted once, by its claimant)
+                const unsigned rest = atomicAdd(claim, nslices);
+                atomicAdd(done, 1u + (rest < nslices ? nslices - rest : 0u));
+                sl = nslices;
+            }
+            *s_sl = sl;
+        }
+        __syncthreads();
+        const unsigned sl = *s_sl;
+        const bool last = sl >= nslices;  // CTA-uniform
+        if (!last) {
+            taken++;
+            pend++;
+            const unsigned i = sl * POOL_SLICE + t;
+            const u64 key = i < m ? __ldcg(S + i) : 0ull;
+            if (key != 0ull && key >= cutW) cand[atomicAdd(s_n, 1)] = key;
+        }
+        __syncthreads();
+        const int n = *s_n;
+        if (n >= ROUND || (last && n > 0)) {
+            pool_rescore(f, cand, n, sc, id, ok, qs);
+            __syncthreads();
+            if (t == 0) *s_sl = atomicAdd(wn, (unsigned)n);
+            __syncthreads();
+            const unsigned b = *s_sl;
+            if (b + n <= POOL_CMAX) {
+                for (int c = t; c < n; c += blockDim.x) {
+                    W[3 * (size_t)(b + c)] = cand[c];
+                    W[3 * (size_t)(b + c) + 1] = (u64)__double_as_longlong(sc[c]);
+                    W[3 * (size_t)(b + c) + 2] = ok[c];
+                }
+            } else if (t == 0) {
+                atomicExch(over, 1u);
+            }
+            __threadfence();
+            __syncthreads();
+            if (t == 0) {
+                atomicAdd(done, pend);
+                *s_n = 0;
+            }
+            pend = 0;
+        } else if (last && pend > 0) {  // (no key of the gathered slices passed cutW)
+            if (t == 0) atomicAdd(done, pend);
+            pend = 0;
+        }
+        if (last) break;
+        __syncthreads();  // *s_sl / *s_n read before the next claim
+    }
+    return taken;
 }
 
 template <typename T, int NV>
@@ -892,11 +1004,16 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
 
     __threadfence();  // this thread's pool stores / slot updates are visible device-wide before the CTA takes its ticket
     __syncthreads();
-    if (threadIdx.x == 0) s_last = atomicAdd(ticket, 1u) == gridDim.x - 1 ? 1 : 0;
+    if (threadIdx.x == 0) {
+        const unsigned tk = atomicAdd(ticket, 1u);
+        s_last = tk == gridDim.x - 1 ? 1 : 0;
+        if constexpr (I8) {
+            if (bounded && tk + 1u + (unsigned)POOL_HELPERS >= gridDim.x && !s_last) s_last = 2;  // a helper of the window pass
+        }
+    }
     __syncthreads();
     if (!s_last) return;  // CTA-uniform
 
-    // ---------------- the last CTA: every other CTA's survivors are in S ----------------
     __threadfence();
     const int t = threadIdx.x, nt = blockDim.x;
     FinalizeShared* sh = reinterpret_cast<FinalizeShared*>(smem_raw);
@@ -909,6 +1026,36 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
     double* sc = reinterpret_cast<double*>(smem_raw + sizeof(FinalizeShared) + surv_bytes);
     long long* id = reinterpret_cast<long long*>(sc + pool_rescore_slots(f));
     u64* ok = reinterpret_cast<u64*>(id + pool_rescore_slots(f));  // qs (filled at kernel start) follows
+    const float twoE = s_twoE;
+    // the window pass's list W, behind the survivor pool's room (one key per row under the bound)
+    u64* const W = I8 ? S + (size_t)gridDim.x * nwarps * CAPW + (size_t)p.n : nullptr;
+    if constexpr (I8) {
+        if (s_last == 2) {
+            // ---------------- a helper: wait for the last CTA to open the window pass, then take slices of it ----------------
+            if (t == 0) {
+                const unsigned long long t0 = globaltimer_ns();
+                unsigned ns = 32;
+                u64 go;
+                // the last CTA is running or about to (every CTA of the grid has started before a following kernel can take
+                // a slot) and only has its loop's tail left; the watchdog only guards against a stalled machine
+                while ((go = ld_relaxed_gpu_u64(pool + POOL_WGO)) == 0ull && globaltimer_ns() - t0 < 10000000ull) {
+                    __nanosleep(ns);
+                    ns = ns < 256 ? 2 * ns : ns;
+                }
+                __threadfence();  // the pool's keys were stored before the tickets, the go word after the last one
+                s_wtau[0] = go;
+                s_ns = 0;
+            }
+            __syncthreads();
+            const u64 go = s_wtau[0];
+            if (go) pool_window_pass(f, pool, W, S, (unsigned)go - 1u, go & 0xFFFFFFFF00000000ull, surv, sc, id, ok, qs, &s_ns, &s_base);
+            __syncthreads();
+            if (t == 0) atomicAdd(reinterpret_cast<unsigned*>(pool + POOL_WLEFT), 1u);  // the last CTA may reset the header now
+            return;
+        }
+    }
+
+    // ---------------- the last CTA: every other CTA's survivors are in S ----------------
     if (p.cta_clock && t == 0) {
         unsigned long long* x = p.cta_clock + 2 * gridDim.x;
         x[0] = globaltimer_ns();  // this (the last) CTA holds its ticket
@@ -916,6 +1063,186 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
         x[3] = t_app;
         x[4] = t_loop;            // ... had left its scan loop
     }
+    // Rule 2 restricted to the members that can reach the top k, then the ranking and output (finalize_rank_emit).
+    // cand / sc / id / ok [0, nk): C re-scored (plus, from W, members below cut, which are skipped), nk >= KP; kth = s~_(k).
+    // Only members with a canonical score >= b = fl_down(s~_(k) - E (1 + 2^-10)) are ranked.  The k best-by-scan rows are
+    // in C with exact scores >= s~_(k) - E.  A canonical score is within (d / 32 + 5) 2^-53 |x| |q| of the exact one (fp64
+    // sums of exact products), and E >= 2^-22 (|q - q^| + |q^|) N >= 2^-22 |q| N, so that is below 2^-25 E at d <= 1024
+    // (the argument needs 2^-10 E): at least k members reach b, and every member below b ranks below all of them.
+    // Ranking by counting is quadratic in the members ranked.
+    auto rank_window = [&](u64* cand, int nk, u64 kth, u64 cut) {
+        int nr = nk;
+        if (kth != 0ull && twoE <= FLT_MAX) {
+            const double b = (double)__fsub_rd(key_score(kth), __fmul_ru(twoE, 0.5f * (1.f + 0x1p-10f)));
+            constexpr int PT = POOL_CMAX / 256;  // slots per thread (blockDim.x = 256)
+            u64 ck[PT], co[PT];
+            double cs[PT];
+            long long ci[PT];
+            bool keep[PT];
+#pragma unroll
+            for (int u = 0; u < PT; u++) {
+                const int c = t + u * nt;
+                keep[u] = c < nk && id[c] >= 0 && cand[c] >= cut && sc[c] >= b;
+                if (keep[u]) {
+                    ck[u] = cand[c];
+                    cs[u] = sc[c];
+                    ci[u] = id[c];
+                    co[u] = ok[c];
+                }
+            }
+            if (t == 0) s_ns = 0;
+            __syncthreads();
+#pragma unroll
+            for (int u = 0; u < PT; u++)
+                if (keep[u]) {  // ranks by counting do not depend on the order
+                    const int pos = atomicAdd(&s_ns, 1);
+                    cand[pos] = ck[u];
+                    sc[pos] = cs[u];
+                    id[pos] = ci[u];
+                    ok[pos] = co[u];
+                }
+            __syncthreads();
+            nr = s_ns > KP ? s_ns : KP;
+            for (int i = s_ns + t; i < nr; i += nt) {  // empty padding up to KP slots
+                cand[i] = 0ull;
+                id[i] = -1;
+                ok[i] = 0ull;
+            }
+            __syncthreads();
+        }
+        finalize_rank_emit<(ScanOcc<T, 1, NV>::value >= 4 ? 2 : 4)>(f, p.q0, cand, sh, sc, id, ok, qs, reinterpret_cast<unsigned char*>(surv),
+                                                                     nr, twoE * 0.5f, cut, true);
+    };
+    bool ranked = false;  // CTA-uniform: the window was ranked from W
+    if constexpr (I8) {
+        if (bounded) {
+            // ---------------- the window pass: open it, take slices like the helpers, then rank from W ----------------
+            if (warp == 0) {
+                u64 ga, gb;
+                const u64 tg = pool_tau(G, lane, ga, gb);  // the final tau_g
+                // t_k = the k-th largest slot maximum: k different rows reach it, so s~_(k) >= t_k >= tau_g (slot maxima of
+                // different slots are different rows' keys; 0 when fewer than k slots are taken).  On unordered data t_k
+                // lies near the 90th best key at k = 48, tau_g near the 300th: W = every pool key >= key_lowered(t_k) is
+                // a few tens of keys more than C, not a few hundred.  (Not unrolled: this tail runs once per search from
+                // code the scan has evicted from L2, and the unrolled rank -- ~400 instructions -- took 18 us to fetch.)
+                int ra = 0, rb = 0;
+#pragma unroll 1
+                for (int j = 0; j < 32; j++) {
+                    const u64 a = __shfl_sync(0xffffffffu, ga, j), b = __shfl_sync(0xffffffffu, gb, j);
+                    ra += (a > ga) + (b > ga);
+                    rb += (a > gb) + (b > gb);
+                }
+                const unsigned fa = __ballot_sync(0xffffffffu, ra == f.k - 1), fb = __ballot_sync(0xffffffffu, rb == f.k - 1);
+                const u64 tk = fa ? __shfl_sync(0xffffffffu, ga, __ffs(fa) - 1) : (fb ? __shfl_sync(0xffffffffu, gb, __ffs(fb) - 1) : tg);
+                if (lane == 0) {
+                    s_tau = tg;
+                    const unsigned m = __ldcg(count);
+                    s_base = m;
+                    // one word: this CTA fenced after its ticket, so the pool's keys are visible to a helper that sees it
+                    // (key_lowered's low word is 0; its value 1, every key, becomes 0, the same set of nonzero keys)
+                    st_relaxed_gpu_u64(pool + POOL_WGO, (key_lowered(tk, twoE) & 0xFFFFFFFF00000000ull) | ((u64)m + 1ull));
+                    fin_note(f, 13, m);
+                    s_wtau[1] = tk;
+                }
+            }
+            if (t == 0) {
+                sh->nsurv = 0;
+                sh->nvalid = 0;
+                sh->maxerr = 0u;
+                sh->ndeep = 0;
+                sh->T0 = 0ull;
+                sh->qnorm2 = 0.0;
+                sh->fail = 0;
+                sh->uncert = 0;
+                s_ns = 0;
+            }
+            __syncthreads();
+            fin_stamp(f, 8);  // window opened
+            const u64 tg = s_tau;
+            const unsigned m = s_base;
+            __syncthreads();  // (s_base is the pass's scratch)
+            u64* cand = surv;
+            u64& s_kth = s_wtau[0];  // (free after the loop)
+            const unsigned nslices = (m + POOL_SLICE - 1) / POOL_SLICE;
+            const unsigned own = pool_window_pass(f, pool, W, S, m, key_lowered(s_wtau[1], twoE) & 0xFFFFFFFF00000000ull, surv, sc, id, ok, qs,
+                                                  &s_ns, &s_base);
+            if (t == 0) {
+                pool_wait_count(reinterpret_cast<const unsigned*>(pool + POOL_WDONE), nslices);  // only running CTAs hold slices
+                s_base = __ldcg(reinterpret_cast<const unsigned*>(pool + POOL_WOVER)) ? 0xFFFFFFFFu
+                                                                                       : __ldcg(reinterpret_cast<const unsigned*>(pool + POOL_WN));
+                s_kth = 0ull;
+                s_ns = 0;
+            }
+            __syncthreads();
+            fin_stamp(f, 9);  // slices done
+            const int nw = (int)s_base;
+            fin_note(f, 11, (unsigned)nw);  // (0xffffffff: W overflowed)
+            fin_note(f, 12, nslices - own);
+            __syncthreads();
+            if (nw >= f.k) {  // CTA-uniform (-1: overflow)
+                // W = every pool key >= cutW, re-scored.  s~_(k) = its k-th largest key (keys are unique: one has rank k - 1)
+                constexpr int PT = POOL_CMAX / 256;
+                u64 wk[PT];
+#pragma unroll
+                for (int u = 0; u < PT; u++) {
+                    const int c = t + u * nt;
+                    wk[u] = 0ull;
+                    if (c < nw) {
+                        wk[u] = __ldcg(W + 3 * (size_t)c);
+                        cand[c] = wk[u];
+                        sc[c] = __longlong_as_double((long long)__ldcg(W + 3 * (size_t)c + 1));
+                        ok[c] = __ldcg(W + 3 * (size_t)c + 2);
+                        id[c] = (long long)key_row(wk[u]);
+                    } else if (c < KP) {
+                        cand[c] = 0ull;
+                        sc[c] = -DBL_MAX;
+                        ok[c] = 0ull;
+                        id[c] = -1;
+                    }
+                }
+                // s~_(k) >= t_k: only the entries >= t_k (~90 of ~490 at 10M rows) can rank k-th, and every entry above one of
+                // them is one of them, so they are ranked among themselves
+                const u64 tk = s_wtau[1];
+                u64* top = surv + POOL_CMAX;  // behind cand (surv holds POOL_SURV + KP >= 2 POOL_CMAX slots)
+#pragma unroll
+                for (int u = 0; u < PT; u++)
+                    if (wk[u] != 0ull && wk[u] >= tk) top[atomicAdd(&s_ns, 1)] = wk[u];
+                __syncthreads();
+                const int ntop = s_ns;
+                for (int c = t; c < ntop; c += nt) {
+                    const u64 key = top[c];
+                    int r = 0;
+                    for (int j = 0; j < ntop; j++) r += top[j] > key ? 1 : 0;
+                    if (r == f.k - 1) s_kth = key;
+                }
+                __syncthreads();
+                const u64 kth = s_kth;
+                // the pool read would have ranked the keys >= tau_g: the same s~_(k) only if k of them are (else: the pool read)
+                if (kth >= tg) {  // CTA-uniform
+                    ranked = true;
+                    const u64 cut = key_lowered(kth, twoE);
+                    int nc = 0;
+#pragma unroll
+                    for (int u = 0; u < PT; u++) nc += __syncthreads_count(wk[u] != 0ull && wk[u] >= cut);
+                    if (t == 0 && f.wide) {
+                        f.wide[1] = (unsigned)nc;
+                        if (nc > POOL_KPMAX) atomicAdd(f.wide, 1u);
+                    }
+                    // reset the pool for the next search of this handle (its CTAs touch it only after this kernel has completed)
+                    if (t < POOL_SLOTS) G[(size_t)t * POOL_GSTRIDE] = 0ull;
+                    if (t == 0) {
+                        *count = 0u;
+                        *ticket = 0u;
+                        if (p.next_chunk) *p.next_chunk = 0u;
+                    }
+                    fin_stamp(f, 10);  // W ranked: s~_(k) and C known
+                    rank_window(cand, nw > KP ? nw : KP, kth, cut);
+                }
+            }
+            if (!ranked) fin_note(f, 10, 0ull);  // the pool read below
+        }
+    }
+    if (!ranked) {
     // one round of loads: the survivor count, the slot maxima and -- speculatively -- the first keys of the pool
     const unsigned m = __ldcg(count);
     u64 spec[POOL_SURV / 2 / 256];
@@ -1081,7 +1408,6 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
         A = surv;
     }
     fin_stamp(f, 2);  // the KP best ranked
-    const float twoE = s_twoE;
     if (!I8 || f.shadow_emax == nullptr) {  // (only the int8 copy is searched under the bound)
         finalize_rank_emit<(ScanOcc<T, 1, NV>::value >= 4 ? 2 : 4)>(f, p.q0, A, sh, sc, id, ok, qs, reinterpret_cast<unsigned char*>(surv));
     } else {
@@ -1130,52 +1456,19 @@ __global__ void __launch_bounds__(256, ScanOcc<T, 1, NV>::value) scan_pool_kerne
         pool_rescore(f, cand, nk, sc, id, ok, qs);
         __syncthreads();
         fin_stamp(f, 6);  // C re-scored
-        // Only members with a canonical score >= b = fl_down(s~_(k) - E (1 + 2^-10)) are ranked.  The k best-by-scan rows are
-        // in C with exact scores >= s~_(k) - E.  A canonical score is within (d / 32 + 5) 2^-53 |x| |q| of the exact one (fp64
-        // sums of exact products), and E >= 2^-22 (|q - q^| + |q^|) N >= 2^-22 |q| N, so that is below 2^-25 E at d <= 1024
-        // (the argument needs 2^-10 E): at least k members reach b, and every member below b ranks below all of them.
-        // Ranking by counting is quadratic in the members ranked.
-        int nr = nk;
-        if (kth != 0ull && twoE <= FLT_MAX) {
-            const double b = (double)__fsub_rd(key_score(kth), __fmul_ru(twoE, 0.5f * (1.f + 0x1p-10f)));
-            constexpr int PT = POOL_CMAX / 256;  // slots per thread (blockDim.x = 256)
-            u64 ck[PT], co[PT];
-            double cs[PT];
-            long long ci[PT];
-            bool keep[PT];
-#pragma unroll
-            for (int u = 0; u < PT; u++) {
-                const int c = t + u * nt;
-                keep[u] = c < nk && id[c] >= 0 && sc[c] >= b;
-                if (keep[u]) {
-                    ck[u] = cand[c];
-                    cs[u] = sc[c];
-                    ci[u] = id[c];
-                    co[u] = ok[c];
-                }
+        rank_window(cand, nk, kth, cut);
+    }
+    }
+    if constexpr (I8) {
+        if (bounded) {
+            // the window header is read by the helpers until they leave: reset it once all of them have (they all hold
+            // tickets, so they are running)
+            if (t == 0) {
+                const unsigned nh = gridDim.x - 1 < (unsigned)POOL_HELPERS ? gridDim.x - 1 : (unsigned)POOL_HELPERS;
+                pool_wait_count(reinterpret_cast<const unsigned*>(pool + POOL_WLEFT), nh);
+                for (int w = POOL_WGO; w <= POOL_WLEFT; w++) pool[w] = 0ull;
             }
-            if (t == 0) s_ns = 0;
-            __syncthreads();
-#pragma unroll
-            for (int u = 0; u < PT; u++)
-                if (keep[u]) {  // ranks by counting do not depend on the order
-                    const int pos = atomicAdd(&s_ns, 1);
-                    cand[pos] = ck[u];
-                    sc[pos] = cs[u];
-                    id[pos] = ci[u];
-                    ok[pos] = co[u];
-                }
-            __syncthreads();
-            nr = s_ns > KP ? s_ns : KP;
-            for (int i = s_ns + t; i < nr; i += nt) {  // empty padding up to KP slots
-                cand[i] = 0ull;
-                id[i] = -1;
-                ok[i] = 0ull;
-            }
-            __syncthreads();
         }
-        finalize_rank_emit<(ScanOcc<T, 1, NV>::value >= 4 ? 2 : 4)>(f, p.q0, cand, sh, sc, id, ok, qs, reinterpret_cast<unsigned char*>(surv),
-                                                                     nr, twoE * 0.5f, cut, true);
     }
     if (p.cta_clock && t == 0) p.cta_clock[2 * gridDim.x + 1] = globaltimer_ns();
 }

@@ -151,13 +151,14 @@ class IndexFlatIP:
         the last fused single-query scan."""
         n = ctypes.c_int64(0)
         check(lib().evs_index_scan_clocks(self._h, None, 0, ctypes.byref(n)))
-        out = np.zeros((n.value + 8, 2), np.uint64)
+        out = np.zeros((n.value + 12, 2), np.uint64)
         if n.value:
-            check(lib().evs_index_scan_clocks(self._h, out.ctypes.data_as(ctypes.c_void_p), n.value + 8, ctypes.byref(n)))
+            check(lib().evs_index_scan_clocks(self._h, out.ctypes.data_as(ctypes.c_void_p), n.value + 12, ctypes.byref(n)))
         # the last CTA: [ticket taken, finalise (+ merge) done, buffers sorted, list merged + stored, scan loop left] and the
-        # finalise's phases [head blocks loaded, survivors, ranked, re-scored, results written]
+        # finalise's phases [head blocks loaded, survivors, ranked, re-scored, results written, ...] (16 slots; slots 8-13:
+        # the int8 window pass, evs_scan.cuh)
         self.last_cta_stamps = out[n.value:n.value + 4].reshape(-1)
-        self.finalize_stamps = out[n.value + 4:n.value + 8].reshape(-1)
+        self.finalize_stamps = out[n.value + 4:n.value + 12].reshape(-1)
         return out[:n.value]
 
     def reset(self) -> None:

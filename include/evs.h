@@ -296,7 +296,9 @@ EVS_API int evs_index_time_scan(evs_index* idx, int64_t nq, const float* q_dev, 
 EVS_API int evs_index_scan_profile(evs_index* idx, int64_t* count, double* total_ms);
 /* With option "scan_clock" = 1 every fused single-query scan records, per CTA, the %globaltimer at its start and at the
  * end of its scan loop: out_host = uint64 [nctas][2] of the last such search (ns); a call with out_host = NULL only returns
- * the count.  Diagnostics for the tail of the streaming scan. */
+ * the count.  With cap_ctas >= nctas + 8 the rows behind the CTAs receive 8 uint64 stamps of the last CTA and the first 8
+ * phase stamps of its finalise; with cap_ctas >= nctas + 12 all 16 finalise slots (slots 8-13: the int8 window pass,
+ * evs_scan.cuh).  Diagnostics for the tail of the streaming scan. */
 EVS_API int evs_index_scan_clocks(evs_index* idx, uint64_t* out_host, int64_t cap_ctas, int64_t* nctas);
 /* Diagnostics for the tensor-core scans (tcgen05): raw scan scores of every row against nq queries,
  * out_dev = float32 [ntotal][pitch]; the pitch (queries padded per block) is returned in *npad, and a call

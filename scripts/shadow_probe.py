@@ -90,12 +90,21 @@ def scan_clock_pass(idx, qt, k, scan_bytes, searches=16):
       c_rescored_to_rank_start_us  the ranked members restricted to canonical scores >= b.  Before: the final re-score of
                                    the kept k and the last round's keys;
       rank_start_to_c_ranked_us    ranks by counting, results stored;
-      c_ranked_to_written_us       padding, the guard."""
+      c_ranked_to_written_us       padding, the guard.
+    Since the window pass (finalise stamps 8-10, counts in slots 11-13), searches ranked from W report instead:
+      ticket_to_window_open_us     tau_g and the pool count read, m and cutW published to the helpers;
+      window_open_to_slices_done_us  the pool re-scored in slices above cutW by the last CTA and the helpers, W complete;
+      slices_done_to_w_ranked_us   W read, s~_(k) ranked, |C| counted;
+      w_ranked_to_written_us       the restricted ranking of C, results stored;
+      ticket_to_written_us         (every search) the whole tail;
+    with |W|, the pool's size m and the slices the helpers took (medians), and how many searches fell back to the pool read."""
     evs.set_option("scan_clock", 1)
-    rec = {"loop_us": [], "end_spread_us": [], "loop_end_to_ticket_us": [], "ticket_to_pool_read_us": [],
-           "pool_read_to_ranked_us": [], "ranked_to_rescored_us": [], "rescored_to_written_us": [], "kernel_us": []}
+    rec = {"loop_us": [], "end_spread_us": [], "loop_end_to_ticket_us": [], "ticket_to_written_us": [], "kernel_us": []}
     window = {"ranked_to_c_gathered_us": [], "c_gathered_to_c_rescored_us": [], "c_rescored_to_rank_start_us": [],
               "rank_start_to_c_ranked_us": [], "c_ranked_to_written_us": []}
+    wpass = {"ticket_to_window_open_us": [], "window_open_to_slices_done_us": [], "slices_done_to_w_ranked_us": [],
+             "w_ranked_to_written_us": [], "w_entries": [], "pool_keys": [], "helper_slices": []}
+    fallbacks = 0
     try:
         for i in range(searches):
             idx.search(qt[i:i + 1], k)
@@ -103,10 +112,20 @@ def scan_clock_pass(idx, qt, k, scan_bytes, searches=16):
             st, fs = idx.last_cta_stamps.astype(np.int64), idx.finalize_stamps.astype(np.int64)
             t0, end = c[:, 0].min(), c[:, 1].max()
             for name, v in (("loop_us", end - t0), ("end_spread_us", end - c[:, 1].min()), ("loop_end_to_ticket_us", st[0] - end),
-                            ("ticket_to_pool_read_us", fs[0] - st[0]), ("pool_read_to_ranked_us", fs[2] - fs[0]),
-                            ("ranked_to_rescored_us", fs[3] - fs[2]), ("rescored_to_written_us", fs[4] - fs[3]),
-                            ("kernel_us", fs[4] - t0)):
+                            ("ticket_to_written_us", fs[4] - st[0]), ("kernel_us", fs[4] - t0)):
                 rec[name].append(v / 1e3)
+            if len(fs) > 13 and fs[8] and fs[10]:  # ranked from the window pass's W (stamps 0-2, 5, 6 are an older search's)
+                for name, v in (("ticket_to_window_open_us", fs[8] - st[0]), ("window_open_to_slices_done_us", fs[9] - fs[8]),
+                                ("slices_done_to_w_ranked_us", fs[10] - fs[9]), ("w_ranked_to_written_us", fs[4] - fs[10])):
+                    wpass[name].append(v / 1e3)
+                wpass["w_entries"].append(fs[11])
+                wpass["helper_slices"].append(fs[12])
+                wpass["pool_keys"].append(fs[13])
+                continue
+            fallbacks += len(fs) > 13 and fs[8] != 0
+            for name, v in (("ticket_to_pool_read_us", fs[0] - st[0]), ("pool_read_to_ranked_us", fs[2] - fs[0]),
+                            ("ranked_to_rescored_us", fs[3] - fs[2]), ("rescored_to_written_us", fs[4] - fs[3])):
+                rec.setdefault(name, []).append(v / 1e3)
             if fs[5] and fs[6]:  # the int8 copy's window stamps
                 for name, v in (("ranked_to_c_gathered_us", fs[5] - fs[2]), ("c_gathered_to_c_rescored_us", fs[6] - fs[5]),
                                 ("c_rescored_to_rank_start_us", fs[3] - fs[6]), ("rank_start_to_c_ranked_us", fs[7] - fs[3]),
@@ -116,7 +135,12 @@ def scan_clock_pass(idx, qt, k, scan_bytes, searches=16):
         evs.set_option("scan_clock", 0)
     if window["ranked_to_c_gathered_us"]:
         rec.update(window)
+    if wpass["w_entries"]:
+        rec.update(wpass)
     out = {name: round(float(np.median(v)), 2) for name, v in rec.items()}
+    if wpass["w_entries"] or fallbacks:
+        out["window_pass_searches"] = len(wpass["w_entries"])
+        out["pool_read_fallbacks"] = int(fallbacks)
     out["loop_tb_s"] = round(scan_bytes / (out["loop_us"] * 1e-6) / 1e12, 3)
     return {"scan_clock": out}
 
