@@ -68,6 +68,7 @@ SIGNATURES = {
     "evs_index_guard_stats": (_i, [_vp, _pi64, _pi64]),
     "evs_index_shadow_stats": (_i, [_vp, _pi64, _pf, _pi64]),
     "evs_index_large_k_stats": (_i, [_vp, _pi64, _pi64]),
+    "evs_index_coalesce_stats": (_i, [_vp, _pi64, _pi64, _pi64]),
     "evs_index_read_rows": (_i, [_c.c_char_p, _i, _i, _i64, _i64, _c.POINTER(_vp), _pi64]),
     "evs_index_file_info": (_i, [_c.c_char_p, _pi, _pi64]),
     "evs_index_scan_clocks": (_i, [_vp, _vp, _i64, _pi64]),

@@ -11,6 +11,8 @@
 #include <unistd.h>
 
 #include <atomic>
+#include <condition_variable>
+#include <deque>
 #include <mutex>
 #include <new>
 #include <string>
@@ -70,6 +72,8 @@ enum { W_TICKET = 0, W_NEXT_CHUNK = 1, W_GUARD_COUNT0 = 2, W_GUARD_COUNT1 = 3, W
        W_EMAX = 13 /* float: largest |x - s c|_2 of a row of the int8 copy */, W_WIDE = 14 /* single-query searches of the int8
        copy whose window held more than 256 candidates */, W_LASTC = 15 /* candidates the last of them re-scored */, W_WORDS = 16 };
 
+struct CoalesceWaiter;  // a single-query caller of evs_index_search waiting for its group (see there)
+
 struct evs_index {
     int d = 0, device = 0, storage = EVS_STORE_F32;
     int64_t ntotal = 0, capacity = 0, id_base = 0;
@@ -120,6 +124,13 @@ struct evs_index {
     // stats word; allocated by the first such search
     unsigned char* lk_ws = nullptr; size_t lk_ws_cap = 0;
     int64_t lk_searches = 0;
+    int64_t i8_batch_passes = 0;      // passes of the int8 batch route (plan_path), any entry point
+    // concurrent single-query callers of evs_index_search (group commit; see there)
+    std::mutex cq_mu;
+    std::condition_variable cq_cv;
+    std::deque<CoalesceWaiter*> cq;  // queued callers, first = next leader
+    bool cq_busy = false;             // a single-query host search runs (alone or as the leader of a group)
+    int64_t co_groups = 0, co_queries = 0;  // groups of two or more callers and the queries they held (under mu)
     unsigned* lk_stats = nullptr;     // into lk_ws: largest |C| of the last large-k search
 };
 
@@ -655,6 +666,7 @@ struct PathInfo {
     float err_trunc = 0.f; // single tf32: the truncation part of the bound, relative to (|q| max|x| + |worst retained score|)
     bool fused = false;  // PATH_GEMV, one query: the scan's last CTA finalises (and, in exchange mode, merges): ONE launch
     bool shadow = false; // ... with the pool kernel over the int8 copy under the bound W_EMAX (exact: evs_scan.cuh)
+    bool i8 = false;     // PATH_LARGE_K over the int8 copy: batches of 2..kI8BatchMaxNQ queries, k <= EVS_MAX_K
 };
 
 // scan error models, relative to |q| * |x| (DESIGN.md section 2).  fp32 GEMV: 4 partial chains of d/128 FMAs per lane, 3 + 5
@@ -693,10 +705,31 @@ static bool shadow_applies(const evs_index* idx, int64_t nq, int kp, const ScanT
            plan.threads == 256;
 }
 
+// Batches of 2..kI8BatchMaxNQ queries (k <= EVS_MAX_K) scan the int8 copy once per pass of LK_I8_NQ queries, keep
+// every row's scan key and re-score exactly every row within 2E of the k-th (evs_large_k.cu: the large-k selection with the
+// int8 bound), under the conditions of shadow_applies other than nq == 1.  Exact by construction for fp32 and bf16 storage.
+// One pass of up to LK_I8_NQ = 4 queries costs less than the tf32 scan of the fp32 rows (k = 48, x 512: 1.27-1.78 ms against
+// 2.91 at 10M rows, 0.20-0.22 against 0.41 at 1.25M, 0.091-0.094 against 0.14 at 300k; profiles/i8_batch_probe.jsonl); two
+// passes (5-8 queries) cost as much or more (2.90-3.28 ms at 10M; profiles/i8_batch_probe_pass4.jsonl), so larger batches
+// keep the tensor-core scan (scripts/i8_batch_probe.py; one B200, 1000 W).
+static const int kI8BatchMaxNQ = LK_I8_NQ;
+static bool i8_batch_applies(const evs_index* idx, int64_t nq, int64_t k, const ScanTuning& tune) {
+    if (nq < 2 || nq > kI8BatchMaxNQ || k > EVS_MAX_K || idx->xi8 == nullptr) return false;
+    if (idx->storage != EVS_STORE_BF16_F32 && !tune.scan_shadow) return false;
+    return idx->special_host == 0 && idx->emax_host <= FLT_MAX && idx->max_norm_host <= FLT_MAX && idx->d % 256 == 0 &&
+           idx->d <= 1024 && idx->ntotal > tune.small_max_rows && idx->ntotal >= tune.shadow_min_rows &&
+           idx->ntotal < ((int64_t)1 << 32) - 32 && i8_batch_grid(idx->d / 256, idx->sm_count) > 0;
+}
+
 static PathInfo plan_path(const evs_index* idx, int64_t nq, int64_t k, const ScanTuning& tune, bool allow_tc) {
     PathInfo pi;
     if (k > EVS_MAX_K) {  // whatever nq, storage or tensor-core routing say: the fp32 rows, exact by construction
         pi.kind = PATH_LARGE_K;
+        return pi;
+    }
+    if (i8_batch_applies(idx, nq, k, tune)) {
+        pi.kind = PATH_LARGE_K;
+        pi.i8 = true;
         return pi;
     }
     const bool bf16 = idx->storage == EVS_STORE_BF16_F32;
@@ -1134,14 +1167,22 @@ static int search_tc_sync_locked(evs_index* idx, int64_t nq, const float* q_dev,
 // k > EVS_MAX_K (evs_large_k.cu): passes of max_queries_per_pass(d) queries over the fp32 rows, each a score scan that keeps
 // every row's scan key, a radix select of the k-th key, the window cut at 2E below it, a grid-wide canonical re-score of the
 // window and the ranking.  Exact by construction (DESIGN.md section 2): nothing is certified afterwards or re-run.
+// With i8 (plan_path: batches of 2..kI8BatchMaxNQ queries) the score scan reads the int8 copy and E is its bound.
 static int search_large_k_locked(evs_index* idx, int64_t nq, const float* q_dev, int64_t k, const SearchOut& out, cudaStream_t st,
-                                 const ScanTuning& tune, bool scan_only, int profile) {
+                                 const ScanTuning& tune, bool scan_only, int profile, bool i8) {
     if (out.x) return fail(EVS_ECUDA, "internal: a large-k search writes its partial to staging, not to the exchange slots");
-    const int qpp = max_queries_per_pass(idx->d, 0);
+    const int qpp = i8 ? LK_I8_NQ : max_queries_per_pass(idx->d, 0);
     ScanTuning gt = tune;
     gt.scan_variant = 1;  // the direct-load grid (the ring variant keeps lists, not keys)
     ScanPlan plan;
-    CU(plan_scan(idx->ntotal, idx->d, SCAN_F32, 64, qpp, idx->sm_count, gt, &plan));
+    if (i8) {
+        plan.variant = 1;
+        plan.nv = idx->d / 256;
+        plan.grid = i8_batch_grid(plan.nv, idx->sm_count);
+        if (plan.grid < 1) return fail(EVS_ECUDA, "int8 batch scan: no resident CTA");
+    } else {
+        CU(plan_scan(idx->ntotal, idx->d, SCAN_F32, 64, qpp, idx->sm_count, gt, &plan));
+    }
     const size_t npad = ((size_t)idx->ntotal + 31) & ~(size_t)31;
     const size_t arrays = (size_t)qpp * npad * 16;  // S, C (u32) and R (u64)
     const size_t state = large_k_state_bytes(qpp);
@@ -1149,11 +1190,13 @@ static int search_large_k_locked(evs_index* idx, int64_t nq, const float* q_dev,
     if (rc) return rc;
     unsigned char* ws = idx->lk_ws;
     idx->lk_stats = reinterpret_cast<unsigned*>(ws + arrays + state);
+    // the int8 batches report their largest |C| where the single-query searches of the copy do (W_LASTC)
+    unsigned* stats = i8 ? idx->words + W_LASTC : idx->lk_stats;
     if (!scan_only) {
         if ((rc = ensure_dev(&idx->margins_dev, &idx->margins_cap, (size_t)nq))) return rc;
         idx->last_nq = nq;
-        idx->lk_searches++;
-        CU(cudaMemsetAsync(idx->lk_stats, 0, sizeof(unsigned), st));
+        if (!i8) idx->lk_searches++;
+        CU(cudaMemsetAsync(stats, 0, sizeof(unsigned), st));
     }
     LargeKArgs a;
     a.xb = idx->xb32;
@@ -1172,8 +1215,13 @@ static int search_large_k_locked(evs_index* idx, int64_t nq, const float* q_dev,
     a.R = reinterpret_cast<unsigned long long*>(a.C + (size_t)qpp * npad);
     a.hist = reinterpret_cast<unsigned*>(ws + arrays);
     a.st = reinterpret_cast<LargeKQuery*>(a.hist + (size_t)3 * qpp * LK_BINS);
-    a.stats = idx->lk_stats;
+    a.stats = stats;
     a.id_base = idx->id_base;
+    if (i8) {
+        a.xi8 = idx->xi8;
+        a.xs8 = idx->xs8;
+        a.emax = reinterpret_cast<const float*>(idx->words + W_EMAX);
+    }
     for (int64_t p0 = 0; p0 < nq; p0 += qpp) {
         a.nq_pass = (int)((nq - p0) < qpp ? (nq - p0) : qpp);
         a.xq = q_dev + (size_t)p0 * idx->d;
@@ -1188,6 +1236,7 @@ static int search_large_k_locked(evs_index* idx, int64_t nq, const float* q_dev,
         CU(launch_large_k_scan(a, st));
         if ((rc = prof.end(st))) return rc;
         if (!scan_only) CU(launch_large_k_rest(a, idx->sm_count, st));
+        if (i8) idx->i8_batch_passes++;
     }
     return EVS_OK;
 }
@@ -1199,7 +1248,7 @@ static int search_enqueue_locked(evs_index* idx, int64_t nq, const float* q_dev,
         std::lock_guard<std::mutex> lk(g_tune_mu);
         profile = g_profile_scans && !scan_only;
     }
-    if (pi.kind == PATH_LARGE_K) return search_large_k_locked(idx, nq, q_dev, k, out, st, tune, scan_only, profile);
+    if (pi.kind == PATH_LARGE_K) return search_large_k_locked(idx, nq, q_dev, k, out, st, tune, scan_only, profile, pi.i8);
     if (pi.kind == PATH_TC_HEAP || pi.kind == PATH_TC_SYNC) {
         idx->bar_used = false;
         int rc = pi.kind == PATH_TC_HEAP ? search_tc_heap_locked(idx, nq, q_dev, k, out, st, tune, pi, scan_only, profile)
@@ -1456,12 +1505,10 @@ static int host_fetch_locked(evs_index* idx, int64_t nq, int64_t k, float* D_hos
     return EVS_OK;
 }
 
-extern "C" int evs_index_search(evs_index* idx, int64_t nq, const float* q_host, int64_t k, float* D_host, int64_t* I_host) {
-    const ScanTuning tune = tune_snapshot();
-    int rc = check_search_args(idx, nq, q_host, k, D_host, I_host, tune);
-    if (rc || nq == 0) return rc;
-    std::lock_guard<std::mutex> lk(idx->mu);
-    if ((rc = use_device(idx->device))) return rc;
+static int search_host_locked(evs_index* idx, int64_t nq, const float* q_host, int64_t k, float* D_host, int64_t* I_host,
+                              const ScanTuning& tune) {
+    int rc = use_device(idx->device);
+    if (rc) return rc;
     if ((rc = host_stage_locked(idx, nq, k))) return rc;
     cudaStream_t st = idx->stream;
     if ((rc = ws_acquire(idx, st))) return rc;
@@ -1539,6 +1586,159 @@ extern "C" int evs_index_search(evs_index* idx, int64_t nq, const float* q_host,
         rc = host_fetch_locked(idx, nq, k, D_host, I_host, st);
     }
     if (rc) cudaStreamSynchronize(st);  // the pinned query buffer may still be in flight: it is reused by the next call
+    return rc;
+}
+
+// ---- coalescing of concurrent single-query callers (group commit) ----
+// A single-query caller (k <= EVS_MAX_K) that finds no such search running on the handle runs alone, exactly as above.  One
+// that arrives while one runs queues itself; when the running search returns, the first queued caller leads the next group:
+// it takes up to kCoalesceCap queued callers and, where group_runs_as_one, searches them as ONE search of nq = m queries
+// and k = the largest k, handing each its prefix (the top k under (canonical desc, id asc) is a prefix of the top k_max);
+// otherwise it searches them one by one.  The others wait for their results; leadership then passes to the next queued
+// caller, so no thread serves other callers' requests for long.
+struct CoalesceWaiter {
+    const float* q;
+    int64_t k;
+    float* D;
+    int64_t* I;
+    int rc = 0;
+    bool done = false, lead = false;
+    char err[512] = "";
+};
+
+// A group runs as one search only on shards where the int8 batch route applies (an int8 copy, at least shadow_min_rows
+// rows): groups of up to kI8BatchMaxNQ take that route, larger fp32 groups the tensor-core scan (2.9 ms for 16 queries at
+// 10M x 512 against 0.75 ms per lone search; scripts/i8_batch_probe.py).  On smaller shards it does not pay: at 10 000 rows
+// (the small-shard kernel, ~30 us end to end) groups of 2-4 through the batch GEMV search ran at 0.78x the lone rate
+// (scripts/coalesce_probe.py, profiles/coalesce_probe_every_size.jsonl), so those callers are searched one by one.
+// The answer is the lone answer for fp32 storage (every path is exact); for bf16 storage only where both read the int8
+// copy (groups of up to kI8BatchMaxNQ, k <= 48) -- its other paths are the uncertified recall mode.
+static const int kCoalesceCap = 16;
+static bool group_runs_as_one(const evs_index* idx, int64_t m, int64_t kmax, const ScanTuning& tune) {
+    if (!i8_batch_applies(idx, 2, kmax, tune)) return false;
+    if (idx->storage != EVS_STORE_BF16_F32) return true;
+    return m <= kI8BatchMaxNQ && kmax <= 48 && shadow_applies(idx, 1, pick_kp(kmax), tune);
+}
+
+// idx->mu is held.  The group's queries go through the pinned staging buffer, its results come back in one copy.
+static int search_group_locked(evs_index* idx, CoalesceWaiter* const* g, int m, const ScanTuning& tune) {
+    int64_t kmax = 0;
+    for (int j = 0; j < m; j++) kmax = g[j]->k > kmax ? g[j]->k : kmax;
+    int rc = use_device(idx->device);
+    if (rc) return rc;
+    if ((rc = host_stage_locked(idx, m, kmax))) return rc;
+    cudaStream_t st = idx->stream;
+    if ((rc = ws_acquire(idx, st))) return rc;
+    const size_t d = (size_t)idx->d;
+    for (int j = 0; j < m; j++) memcpy(idx->q_pin + j * d, g[j]->q, d * sizeof(float));
+    CU(cudaMemcpyAsync(idx->q_dev, idx->q_pin, (size_t)m * d * sizeof(float), cudaMemcpyHostToDevice, st));
+    SearchOut out;
+    out.D = idx->D_dev;
+    out.I = idx->I_dev;
+    rc = search_dev_common(idx, m, idx->q_dev, kmax, out, st, tune, plan_path(idx, m, kmax, tune, true));
+    if (!rc) {
+        const size_t n = (size_t)m * kmax;
+        const cudaError_t e = cudaMemcpyAsync(idx->I_pin, idx->I_dev, n * (sizeof(int64_t) + sizeof(float)), cudaMemcpyDeviceToHost, st);
+        if (e != cudaSuccess) rc = fail(EVS_ECUDA, "%s", cudaGetErrorString(e));
+    }
+    if (!rc) {
+        const cudaError_t e = cudaStreamSynchronize(st);
+        if (e != cudaSuccess) rc = fail(EVS_ECUDA, "search failed: %s", cudaGetErrorString(e));
+    }
+    if (rc) {
+        cudaStreamSynchronize(st);  // the pinned query buffer may still be in flight
+        return rc;
+    }
+    for (int j = 0; j < m; j++) {
+        memcpy(g[j]->D, idx->D_pin + (size_t)j * kmax, (size_t)g[j]->k * sizeof(float));
+        memcpy(g[j]->I, idx->I_pin + (size_t)j * kmax, (size_t)g[j]->k * sizeof(int64_t));
+    }
+    idx->co_groups++;
+    idx->co_queries += m;
+    return EVS_OK;
+}
+
+// the leader `self`, already off the queue: takes up to kCoalesceCap - 1 more callers, searches them, wakes them
+static int lead_group(evs_index* idx, CoalesceWaiter* self, const ScanTuning& tune) {
+    CoalesceWaiter* g[kCoalesceCap];
+    int m = 0;
+    g[m++] = self;
+    {
+        std::lock_guard<std::mutex> lq(idx->cq_mu);
+        while (m < kCoalesceCap && !idx->cq.empty()) {
+            g[m++] = idx->cq.front();
+            idx->cq.pop_front();
+        }
+    }
+    {
+        std::lock_guard<std::mutex> lk(idx->mu);
+        // bf16 storage: sub-groups of at most kI8BatchMaxNQ (the int8 route); fp32: the whole group
+        const int step = idx->storage == EVS_STORE_BF16_F32 ? kI8BatchMaxNQ : m;
+        for (int j0 = 0; j0 < m; j0 += step) {
+            const int n = m - j0 < step ? m - j0 : step;
+            int64_t kmax = 0;
+            for (int j = j0; j < j0 + n; j++) kmax = g[j]->k > kmax ? g[j]->k : kmax;
+            if (n >= 2 && group_runs_as_one(idx, n, kmax, tune)) {
+                const int rc = search_group_locked(idx, g + j0, n, tune);
+                for (int j = j0; j < j0 + n; j++) {
+                    g[j]->rc = rc;
+                    if (rc) snprintf(g[j]->err, sizeof(g[j]->err), "%s", t_err);
+                }
+            } else {
+                for (int j = j0; j < j0 + n; j++) {
+                    g[j]->rc = search_host_locked(idx, 1, g[j]->q, g[j]->k, g[j]->D, g[j]->I, tune);
+                    if (g[j]->rc) snprintf(g[j]->err, sizeof(g[j]->err), "%s", t_err);
+                }
+            }
+        }
+    }
+    {
+        std::lock_guard<std::mutex> lq(idx->cq_mu);
+        for (int j = 1; j < m; j++) g[j]->done = true;
+    }
+    idx->cq_cv.notify_all();
+    return self->rc ? fail(self->rc, "%s", self->err) : EVS_OK;
+}
+
+extern "C" int evs_index_search(evs_index* idx, int64_t nq, const float* q_host, int64_t k, float* D_host, int64_t* I_host) {
+    const ScanTuning tune = tune_snapshot();
+    int rc = check_search_args(idx, nq, q_host, k, D_host, I_host, tune);
+    if (rc || nq == 0) return rc;
+    if (nq != 1 || k > EVS_MAX_K) {
+        std::lock_guard<std::mutex> lk(idx->mu);
+        return search_host_locked(idx, nq, q_host, k, D_host, I_host, tune);
+    }
+    CoalesceWaiter w;
+    w.q = q_host;
+    w.k = k;
+    w.D = D_host;
+    w.I = I_host;
+    {
+        std::unique_lock<std::mutex> lq(idx->cq_mu);
+        if (idx->cq_busy) {
+            idx->cq.push_back(&w);
+            idx->cq_cv.wait(lq, [&] { return w.done || w.lead; });
+            if (w.done) return w.rc ? fail(w.rc, "%s", w.err) : EVS_OK;
+        } else {
+            idx->cq_busy = true;
+        }
+    }
+    if (w.lead) {
+        rc = lead_group(idx, &w, tune);
+    } else {
+        std::lock_guard<std::mutex> lk(idx->mu);
+        rc = search_host_locked(idx, nq, q_host, k, D_host, I_host, tune);
+    }
+    {  // hand the handle to the next queued caller, or leave it idle
+        std::lock_guard<std::mutex> lq(idx->cq_mu);
+        if (idx->cq.empty()) {
+            idx->cq_busy = false;
+        } else {
+            idx->cq.front()->lead = true;
+            idx->cq.pop_front();
+        }
+    }
+    idx->cq_cv.notify_all();
     return rc;
 }
 
@@ -1893,6 +2093,15 @@ extern "C" int evs_index_large_k_stats(evs_index* idx, int64_t* searches, int64_
     if (idx->lk_stats) CU(cudaMemcpy(&c, idx->lk_stats, sizeof(c), cudaMemcpyDeviceToHost));
     if (searches) *searches = idx->lk_searches;
     if (last_candidates) *last_candidates = (int64_t)c;
+    return EVS_OK;
+}
+
+extern "C" int evs_index_coalesce_stats(evs_index* idx, int64_t* groups, int64_t* grouped_queries, int64_t* i8_batch_passes) {
+    if (!idx) return fail(EVS_EINVAL, "idx is NULL");
+    std::lock_guard<std::mutex> lk(idx->mu);
+    if (groups) *groups = idx->co_groups;
+    if (grouped_queries) *grouped_queries = idx->co_queries;
+    if (i8_batch_passes) *i8_batch_passes = idx->i8_batch_passes;
     return EVS_OK;
 }
 

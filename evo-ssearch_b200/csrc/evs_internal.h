@@ -305,6 +305,9 @@ struct LargeKArgs {
     int all_rows = 0;           // ... it does: every row is a candidate
     float err_coef = 0.f;       // scan error relative to |q| max|x| (gemv_err_coef)
     const float* max_norm = nullptr;
+    const signed char* xi8 = nullptr;  // non-null: the score scan reads the int8 copy (codes [n][d], scales xs8 [n]) and E is
+    const float* xs8 = nullptr;        //   its bound (i8_scan_bound, e_max at *emax); nv = d / 256; the re-score reads xb
+    const float* emax = nullptr;
     unsigned* S = nullptr;      // [nq_pass][npad] order-preserving scan keys
     unsigned* C = nullptr;      // [nq_pass][npad] candidate rows
     unsigned long long* R = nullptr;  // [nq_pass][npad] canonical rank keys of the candidates (0: NaN)
@@ -319,6 +322,10 @@ struct LargeKArgs {
     float* margins = nullptr;   // [nq_pass]
 };
 size_t large_k_state_bytes(int qpp);  // hist + st of a pass (zeroed before it)
+// queries per pass of the int8 score scan (lk_score_i8_kernel): 8 ran at half the read rate, limited by IDP.4A
+// (scripts/i8_batch_probe.py, profiles/i8_batch_probe_pass8.jsonl)
+constexpr int LK_I8_NQ = 4;
+int i8_batch_grid(int nv, int sm_count);  // its CTAs, nv = d / 256: as many as are resident at once (0: none)
 cudaError_t launch_large_k_scan(const LargeKArgs& a, cudaStream_t st);
 cudaError_t launch_large_k_rest(const LargeKArgs& a, int sm_count, cudaStream_t st);
 

@@ -16,7 +16,11 @@
 //                           or -- larger C (ties, special data) -- a radix select of the k-th (score, row) pair first.
 // Exact by construction: the k rows with the best scan scores all have exact scores >= s_(k) - E, so the exact k-th score
 // is >= s_(k) - E and every row of the exact top k has a scan score >= s_(k) - 2E.
+// Batches of 2..4 queries with k <= EVS_MAX_K over an int8 copy take the same kernels with lk_score_i8_kernel as step 1 and
+// the copy's bound as E (plan_path in evs_api.cu).
 #include <float.h>
+
+#include <atomic>
 
 #include "evs_internal.h"
 #include "evs_scan.cuh"
@@ -131,6 +135,98 @@ __global__ void __launch_bounds__(256) lk_score_generic_kernel(LargeKArgs a) {
     lk_flush_hist(h, a.hist + (size_t)qi * LK_BINS, LK_BINS);
 }
 
+// The int8 copy, NQ = LK_I8_NQ queries per pass (batches of 2..4 queries, k <= EVS_MAX_K; DESIGN.md section 2): the
+// arithmetic of scan_pool_kernel<int8_t> -- the same query codes and split 16-bit IDP.4A chains, the exact integer I, the
+// same wide-d fp64 combine and s~ = fl(fl(I) fl(s_q s_r)) -- so that its bound E holds for every key.  A group of R rows
+// yields R * NQ (* 2 for wide d) lane sums, 32 in all: one halving reduction leaves lane l with value l, so every lane
+// (every other lane for wide d) ends holding one (row, query) score.
+template <int NQ, int NV>
+struct I8Batch {
+    static constexpr int W = NV <= 2 ? 1 : 2;  // values per (row, query): the int32 sum, or the h and l chains
+    static constexpr int R = 32 / (NQ * W);    // rows per group
+    static_assert(R >= 1 && R * NQ * W == 32, "one value per lane after the reduction");
+    static constexpr int OCC = 2;              // CTAs of 256 threads per SM (128 registers)
+};
+
+template <int NQ, int NV>
+__global__ void __launch_bounds__(256, I8Batch<NQ, NV>::OCC) lk_score_i8_kernel(LargeKArgs a) {
+    extern __shared__ unsigned lk_i8_hist[];  // [NQ][LK_BINS]
+    typedef I8Lane<NV> L;
+    typedef I8Batch<NQ, NV> B;
+    constexpr int R = B::R, W = B::W;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
+    for (int i = threadIdx.x; i < NQ * LK_BINS; i += blockDim.x) lk_i8_hist[i] = 0u;
+    lk_wait();
+    __syncthreads();
+    // queries past the pass's last repeat it: their keys are never stored
+    QueryRegs<int8_t, 1, NV> q[NQ];
+#pragma unroll
+    for (int qi = 0; qi < NQ; qi++) q[qi].load(a.xq, qi < a.nq_pass ? qi : a.nq_pass - 1, a.d, lane);
+    const int pair = lane / W, my_r = pair / NQ, my_q = pair % NQ;
+    const bool rep = (lane % W) == 0;
+    float my_sq = q[0].sq;
+#pragma unroll
+    for (int qi = 1; qi < NQ; qi++) my_sq = my_q == qi ? q[qi].sq : my_sq;
+    const int8_t* codes = reinterpret_cast<const int8_t*>(a.xi8);
+    struct Group {
+        unsigned w[R][L::WORDS];
+        float sr;  // the scale of row my_r
+    };
+    auto load = [&](Group& b, long long g) {
+        const long long r0 = g * R;
+        b.sr = __ldg(a.xs8 + (r0 + my_r < a.n ? r0 + my_r : a.n - 1));
+#pragma unroll
+        for (int r = 0; r < R; r++) {
+            const long long row = r0 + r < a.n ? r0 + r : a.n - 1;  // clamp: tail rows are re-read, not stored
+            L::load(codes + (size_t)row * a.d, lane, b.w[r]);
+        }
+    };
+    auto score = [&](const Group& b, long long g) {
+        int v[32];
+#pragma unroll
+        for (int r = 0; r < R; r++)
+#pragma unroll
+            for (int qi = 0; qi < NQ; qi++) {
+                int ih = 0, il = 0;
+#pragma unroll
+                for (int w = 0; w < L::WORDS; w++) {
+                    ih = __dp4a((int)b.w[r][w], q[qi].h[w], ih);
+                    il = __dp4a((int)b.w[r][w], q[qi].l[w], il);
+                }
+                if constexpr (W == 1) v[r * NQ + qi] = ih * 256 + il;
+                else {
+                    v[2 * (r * NQ + qi)] = ih;
+                    v[2 * (r * NQ + qi) + 1] = il;
+                }
+            }
+        i8_warp_sum<32>(v, lane);
+        float fi;
+        if constexpr (W == 1) fi = __int2float_rn(v[0]);
+        else {  // even lanes hold the h sum, odd lanes the l sum of the same (row, query)
+            const int o = __shfl_xor_sync(0xffffffffu, v[0], 1);
+            fi = __double2float_rn(fma((double)(rep ? v[0] : o), 256.0, (double)(rep ? o : v[0])));
+        }
+        const float s = __fmul_rn(fi, __fmul_rn(my_sq, b.sr));
+        const long long row = g * R + my_r;
+        if (rep && row < a.n && my_q < a.nq_pass) {
+            const unsigned key = score_to_ordered(s);
+            a.S[(size_t)my_q * a.npad + row] = key;
+            atomicAdd(&lk_i8_hist[my_q * LK_BINS + (key >> 21)], 1u);
+        }
+    };
+    const long long ngroups = (a.n + R - 1) / R;
+    const long long total_warps = (long long)gridDim.x * nwarps;
+    long long g = (long long)blockIdx.x * nwarps + warp;
+    // one group in registers per warp: the other warps of the SM keep the loads in flight (two resident CTAs)
+    for (; g < ngroups; g += total_warps) {
+        Group A;
+        load(A, g);
+        score(A, g);
+    }
+    __syncthreads();
+    for (int qi = 0; qi < a.nq_pass && qi < NQ; qi++) lk_flush_hist(lk_i8_hist + qi * LK_BINS, a.hist + (size_t)qi * LK_BINS, LK_BINS);
+}
+
 // ---------------------------------------------------------------------------------------------
 // 2. threshold: radix select of the k-th largest scan key
 // ---------------------------------------------------------------------------------------------
@@ -169,12 +265,63 @@ __device__ __forceinline__ void lk_find_digit(const unsigned* h, unsigned krem, 
     __syncthreads();
 }
 
-// one CTA of 1024 threads per query; level 0 also derives E from |q| and max|x|
+// E of query qi over the fp32 rows: gemv_err_coef(d) |q| max|x|, |q| and max|x| inflated for their own roundings (max_norm is
+// an fp32 sum of squares: within d 2^-24 of the truth), plus an absolute term for products that underflow in fp32.  All
+// threads of the CTA; every thread returns E.
+__device__ __noinline__ float lk_f32_bound(const LargeKArgs& a, int qi, double* s_q2) {
+    const int t = threadIdx.x;
+    double q2 = 0.0;
+    for (int i = t; i < a.d; i += blockDim.x) {
+        const double v = (double)a.xq[(size_t)qi * a.d + i];
+        q2 = fma(v, v, q2);
+    }
+#pragma unroll
+    for (int off = 16; off >= 1; off >>= 1) q2 += __shfl_xor_sync(0xffffffffu, q2, off);
+    if ((t & 31) == 0) s_q2[t >> 5] = q2;
+    __syncthreads();
+    q2 = 0.0;
+    for (int w = 0; w < 32; w++) q2 += s_q2[w];
+    const double qn = sqrt(q2) * (1.0 + 0x1p-20), nx = (double)__ldg(a.max_norm) * (1.0 + 0x1p-7);
+    double e = (double)a.err_coef * qn * nx * (1.0 + 0x1p-20) + 0x1p-120;
+    if (!(qn * nx <= 0x1p126)) e = INFINITY;  // fp32 partial sums might overflow: every row is a candidate
+    return __double2float_ru(e);
+}
+// ... over the int8 copy: i8_scan_bound of |q - q^| and |q^|, from the query codes every warp of the score scan derived
+__device__ __noinline__ float lk_i8_bound(const LargeKArgs& a, int qi, double* s_dq2, double* s_qh2) {
+    const int t = threadIdx.x;
+    const float* q = a.xq + (size_t)qi * a.d;
+    const float sq = i8_query_scale(q, a.d, t & 31);
+    double dq2 = 0.0, qh2 = 0.0;
+    for (int i = t; i < a.d; i += blockDim.x) {
+        const double qh = (double)sq * (double)i8_query_code(q[i], sq);  // exact: 24 x 16 bits
+        dq2 = fma((double)q[i] - qh, (double)q[i] - qh, dq2);
+        qh2 = fma(qh, qh, qh2);
+    }
+#pragma unroll
+    for (int off = 16; off >= 1; off >>= 1) {
+        dq2 += __shfl_xor_sync(0xffffffffu, dq2, off);
+        qh2 += __shfl_xor_sync(0xffffffffu, qh2, off);
+    }
+    if ((t & 31) == 0) {
+        s_dq2[t >> 5] = dq2;
+        s_qh2[t >> 5] = qh2;
+    }
+    __syncthreads();
+    dq2 = 0.0;
+    qh2 = 0.0;
+    for (int w = 0; w < 32; w++) {
+        dq2 += s_dq2[w];
+        qh2 += s_qh2[w];
+    }
+    return i8_scan_bound(dq2, qh2, __ldg(a.max_norm), __ldg(a.emax));
+}
+
+// one CTA of 1024 threads per query; level 0 also derives E (lk_f32_bound, or lk_i8_bound for the int8 copy)
 __global__ void __launch_bounds__(1024) lk_select_kernel(LargeKArgs a, int level) {
     __shared__ unsigned s_warp[32];
     __shared__ int s_digit;
     __shared__ unsigned s_above;
-    __shared__ double s_q2[32];
+    __shared__ double s_q2[32], s_qh2[32];
     const int qi = blockIdx.x, t = threadIdx.x;
     lk_wait();
     LargeKQuery* st = a.st + qi;
@@ -185,28 +332,7 @@ __global__ void __launch_bounds__(1024) lk_select_kernel(LargeKArgs a, int level
         krem = __ldcg(&st->krem);
     }
     if (t == 0) s_digit = -1;
-    float E = 0.f;
-    if (level == 0) {
-        double q2 = 0.0;
-        for (int i = t; i < a.d; i += blockDim.x) {
-            const double v = (double)a.xq[(size_t)qi * a.d + i];
-            q2 = fma(v, v, q2);
-        }
-#pragma unroll
-        for (int off = 16; off >= 1; off >>= 1) q2 += __shfl_xor_sync(0xffffffffu, q2, off);
-        if ((t & 31) == 0) s_q2[t >> 5] = q2;
-        __syncthreads();
-        q2 = 0.0;
-        for (int w = 0; w < 32; w++) q2 += s_q2[w];
-        // |q| and max|x| inflated for their own roundings (max_norm is an fp32 sum of squares: within d 2^-24 of the truth),
-        // plus an absolute term for products that underflow in fp32
-        const double qn = sqrt(q2) * (1.0 + 0x1p-20), nx = (double)__ldg(a.max_norm) * (1.0 + 0x1p-7);
-        double e = (double)a.err_coef * qn * nx * (1.0 + 0x1p-20) + 0x1p-120;
-        if (!(qn * nx <= 0x1p126)) e = INFINITY;  // fp32 partial sums might overflow: every row is a candidate
-        E = __double2float_ru(e);
-    } else {
-        E = __ldcg(&st->E);
-    }
+    const float E = level > 0 ? __ldcg(&st->E) : a.xi8 ? lk_i8_bound(a, qi, s_q2, s_qh2) : lk_f32_bound(a, qi, s_q2);
     __syncthreads();
     const bool all = a.all_rows || !(2.f * E <= FLT_MAX);
     if (!all) lk_find_digit(a.hist + ((size_t)level * a.nq_pass + qi) * LK_BINS, krem, s_warp, &s_digit, &s_above);
@@ -458,7 +584,60 @@ static cudaError_t launch_score_nq(const LargeKArgs& a, cudaStream_t st) {
     }
 }
 
+template <int NV>
+static cudaError_t i8_kernel_setup(int sm_count, int* grid) {
+    static std::atomic<int> occ_dev[16];  // per instantiation and device: CTAs per SM once the attribute is set (0: not yet)
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return e;
+    int occ = occ_dev[dev & 15].load();
+    if (occ == 0) {
+        const size_t smem = (size_t)LK_I8_NQ * LK_BINS * sizeof(unsigned);
+        e = cudaFuncSetAttribute(lk_score_i8_kernel<LK_I8_NQ, NV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, lk_score_i8_kernel<LK_I8_NQ, NV>, 256, smem);
+        if (e != cudaSuccess) return e;
+        if (occ < 1) return cudaErrorInvalidConfiguration;
+        occ_dev[dev & 15].store(occ);
+    }
+    *grid = sm_count * occ;
+    return cudaSuccess;
+}
+int i8_batch_grid(int nv, int sm_count) {
+    int grid = 0;
+    cudaError_t e;
+    switch (nv) {
+        case 1: e = i8_kernel_setup<1>(sm_count, &grid); break;
+        case 2: e = i8_kernel_setup<2>(sm_count, &grid); break;
+        case 3: e = i8_kernel_setup<3>(sm_count, &grid); break;
+        case 4: e = i8_kernel_setup<4>(sm_count, &grid); break;
+        default: e = cudaErrorInvalidValue;
+    }
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return 0;
+    }
+    return grid;
+}
+static cudaError_t launch_score_i8(const LargeKArgs& a, cudaStream_t st) {
+    const size_t smem = (size_t)LK_I8_NQ * LK_BINS * sizeof(unsigned);
+    const dim3 grid((unsigned)a.grid), block(256);
+    switch (a.nv) {
+        case 1: return launch_pdl(lk_score_i8_kernel<LK_I8_NQ, 1>, grid, block, smem, st, a);
+        case 2: return launch_pdl(lk_score_i8_kernel<LK_I8_NQ, 2>, grid, block, smem, st, a);
+        case 3: return launch_pdl(lk_score_i8_kernel<LK_I8_NQ, 3>, grid, block, smem, st, a);
+        case 4: return launch_pdl(lk_score_i8_kernel<LK_I8_NQ, 4>, grid, block, smem, st, a);
+        default: return cudaErrorInvalidValue;
+    }
+}
+
 cudaError_t launch_large_k_scan(const LargeKArgs& a, cudaStream_t st) {
+    if (a.xi8) {  // up to LK_I8_NQ queries, a.grid from i8_batch_grid
+        if (a.n <= 0 || a.nq_pass < 1 || a.nq_pass > LK_I8_NQ || a.grid < 1) return cudaErrorInvalidValue;
+        const cudaError_t e = launch_score_i8(a, st);
+        g_kernel_launches.fetch_add(1);
+        if (e != cudaSuccess) return e;
+        return cudaGetLastError();
+    }
     if (a.n <= 0 || a.nq_pass < 1 || a.nq_pass > 4) return cudaErrorInvalidValue;
     cudaError_t e;
     switch (a.nv) {

@@ -167,7 +167,7 @@ __device__ __forceinline__ float i8_query_scale(const float* __restrict__ q, int
 }
 template <int NQ, int NV>
 struct QueryRegs<int8_t, NQ, NV> {
-    static_assert(NQ == 1, "the int8 copy is scanned for single queries only");
+    static_assert(NQ == 1, "one query per object (the multi-query score scan of evs_large_k.cu holds an array of them)");
     int h[2 * NV], l[2 * NV];  // packed signed bytes of the query codes that pair with word w of the lane's row data
     float sq;
     __device__ __forceinline__ void load(const float* __restrict__ xq, int q0, int d, int lane) {
@@ -514,12 +514,17 @@ __host__ __device__ inline size_t small_query_smem_offset(int kp, int d, int wor
 //           < s~_(k) - E, below each of the k best-by-scan rows, so the top k of C is the exact answer.
 // With shadow_emax == null the lowered threshold IS the threshold (twoE = 0): the fp32 / bf16 scans as before.
 // ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ float shadow_bound_i8(const FinalizeParams& f, double dq2, double qh2) {
+// dq2 = |q - q^|^2 and qh2 = |q^|^2 summed in fp64 (any order), max_norm = N before its inflation, emax = e_max; shared by
+// the single-query pool kernel and the multi-query score scan of evs_large_k.cu
+__device__ __forceinline__ float i8_scan_bound(double dq2, double qh2, float max_norm, float emax) {
     const double dq = sqrt(dq2) * (1.0 + 0x1p-20), qh = sqrt(qh2) * (1.0 + 0x1p-20);  // |q - q^|, |q^|
-    const double nx = (double)__ldg(f.max_norm) * (1.0 + 0x1p-7);
-    const double em = (double)__ldg(f.shadow_emax);
+    const double nx = (double)max_norm * (1.0 + 0x1p-7);
+    const double em = (double)emax;
     const double e = (dq * nx + qh * em + 0x1p-22 * qh * (nx + em)) * (1.0 + 0x1p-20) + 0x1p-117;
     return __double2float_ru(e);  // inf when it does not fit: every key is kept below
+}
+__device__ __forceinline__ float shadow_bound_i8(const FinalizeParams& f, double dq2, double qh2) {
+    return i8_scan_bound(dq2, qh2, __ldg(f.max_norm), __ldg(f.shadow_emax));
 }
 // the smallest key of score score(t) - 2E (rounded down); 1 (every key) without a finite bound
 __device__ __forceinline__ u64 key_lowered(u64 t, float twoE) {

@@ -146,6 +146,14 @@ class IndexFlatIP:
         check(lib().evs_index_large_k_stats(self._h, ctypes.byref(s), ctypes.byref(c)))
         return s.value, c.value
 
+    def coalesce_stats(self):
+        """``(groups, grouped_queries, i8_batch_passes)``: groups of two or more concurrent single-query ``search`` calls
+        served as one search and the queries they held (a caller that found the index idle moves neither), and the passes
+        of the exact batch search of the int8 copy (batches of 2..4 queries, any entry point)."""
+        g, q, p = ctypes.c_int64(0), ctypes.c_int64(0), ctypes.c_int64(0)
+        check(lib().evs_index_coalesce_stats(self._h, ctypes.byref(g), ctypes.byref(q), ctypes.byref(p)))
+        return g.value, q.value, p.value
+
     def scan_clocks(self) -> np.ndarray:
         """Diagnostics (option ``scan_clock``): ``uint64[nctas, 2]`` start / end-of-scan-loop times (ns) of the CTAs of
         the last fused single-query scan."""

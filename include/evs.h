@@ -16,7 +16,15 @@
  *   - the index handle owns all device memory it allocates; the caller owns every buffer it passes.
  *     add() copies, so the caller may free its array immediately (oldapp.py:86-88 does).
  *   - search on one handle may be entered from several threads (the Flask dev server is threaded,
- *     oldapp.py:2258); calls on the same handle are serialised internally.
+ *     oldapp.py:2258); calls on the same handle are serialised internally.  Single-query
+ *     evs_index_search calls (k <= EVS_MAX_K) that arrive while another one runs are queued and served
+ *     together, up to 16 at a time, as ONE search of the largest k, each receiving its own prefix
+ *     (group commit: no timer, and a caller that finds the handle idle runs alone at once).  Groups
+ *     form on shards with an int8 copy of at least option shadow_min_rows rows, where one search of
+ *     m queries costs less than m lone ones; there every answer is the answer of the same call made
+ *     alone (fp32 storage; bf16 storage in groups of up to 4 with k <= 48, which read the int8 copy
+ *     either way), so results never depend on concurrency.  Elsewhere queued callers are searched
+ *     one by one.  See evs_index_coalesce_stats.
  *   - there is NO CPU fallback: without a CUDA device every compute entry point fails with
  *     EVS_ENODEV.
  *
@@ -133,9 +141,13 @@ EVS_API int evs_index_get_rows(const evs_index* idx, int64_t row0, int64_t n, fl
  *                          mapped completion word instead of draining the stream).
  *
  * Exactness of fp32-storage indexes (every entry point: host, device, partial, exchange):
- *   1 query        fp32 CUDA-core GEMV scan;
- *   2..32 queries  single-tf32 tensor-core scan with the top-k' kept on chip (option "x3": batches of up to 16 queries take
- *                  the 3xTF32 split scan instead -- fp32-class scan error, ~1e-6 on unit vectors);
+ *   1 query        fp32 CUDA-core GEMV scan (or the int8 copy, exact by construction: option "scan_shadow");
+ *   2..4 queries   over shards with an int8 copy, above small_max_rows and of at least shadow_min_rows rows, d a multiple
+ *                  of 256 up to 1024: one pass over the int8 copy, every row's scan key kept, every row
+ *                  within 2E of the k-th re-scored exactly (E the copy's proven bound): exact by construction, for bf16
+ *                  storage too, and last_margins = canonical k-th score - (best excluded scan score + E);
+ *   2..32 queries  otherwise: single-tf32 tensor-core scan with the top-k' kept on chip (option "x3": batches of up to 16
+ *                  queries take the 3xTF32 split scan instead -- fp32-class scan error, ~1e-6 on unit vectors);
  *   more           single-tf32 tensor-core scan, candidates k' = 64/128 selected through sampled thresholds.
  *   Every result is then ranked by the canonical fp64 re-score of its candidates, and the finalise step CERTIFIES it: the
  *   k-th canonical score must clear the worst retained scan score by more than the error bound of the scan that selected
@@ -208,6 +220,10 @@ EVS_API int evs_index_shadow_stats(evs_index* idx, int64_t* wide_searches, float
 /* large-k searches (k > EVS_MAX_K) on this handle, and the number of candidates the last one re-scored exactly (the largest
  * over its queries): rows whose fp32 scan score lies within twice the scan's error bound of the k-th best scan score */
 EVS_API int evs_index_large_k_stats(evs_index* idx, int64_t* searches, int64_t* last_candidates);
+/* coalescing of concurrent single-query evs_index_search calls on this handle: groups of two or more callers served as one
+ * search, and the queries they held (a caller that ran alone moves neither); and the passes of the int8 batch search
+ * (2..4 queries, any entry point; its largest window |C| is the last_candidates of evs_index_shadow_stats) */
+EVS_API int evs_index_coalesce_stats(evs_index* idx, int64_t* groups, int64_t* grouped_queries, int64_t* i8_batch_passes);
 
 /* ---- persistence: <folder>/.clip_index/index.faiss -------------------------------------------
  * evs_index_write       <- faiss.write_index(index, path)           oldapp.py:98
